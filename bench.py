@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- AES-GCM enc+tag throughput of the B200 engine (BASELINE.json metric).
 
-  python bench.py [--gpus N --steps K --warmup W] [--impl reference]
+  python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one fused GCTR+GHASH pass (encrypt + tag) over one synthetic stream resident in HBM.
 N=1: BASELINE config 2, AES-256, one 2^30-byte stream, 16 B AAD.
@@ -37,6 +37,8 @@ UNIT = "GB/s"
 SHARD_BYTES = 1 << 30
 AAD_BYTES = 16
 PARITY_BYTES_PER_RANK = 64 << 20
+DUMP_WINDOW = 4096      # bytes per sampled ciphertext window (--dump-outputs)
+DUMP_WINDOWS = 2048     # windows over all ranks: 8 MiB of ciphertext, 32 MiB as float32
 
 
 def stream_inputs():
@@ -428,6 +430,23 @@ def batched_split(eng, torch, dist, dev, rank, world, iters=5, weak=False):
     return res
 
 
+def dump_outputs(out_dir, rank, world, d_ct, d_tag):
+    """Writes what the last timed step handed its caller, so that two builds can be compared output
+    for output: the 16-byte tag (tag.npy) and a fixed sample of this rank's ciphertext, DUMP_WINDOWS /
+    world windows of DUMP_WINDOW bytes at window indices drawn by default_rng(3), one row per window
+    in stream order (ciphertext_sample.npy, or ciphertext_sample_rank<r>.npy when N > 1).  Bytes are
+    stored as float32."""
+    import torch
+    n_win = d_ct.numel() // DUMP_WINDOW
+    pick = np.sort(np.random.default_rng(3).choice(n_win, min(n_win, DUMP_WINDOWS // world), replace=False))
+    windows = d_ct[:n_win * DUMP_WINDOW].view(n_win, DUMP_WINDOW).index_select(0, torch.from_numpy(pick).to(d_ct.device))
+    os.makedirs(out_dir, exist_ok=True)
+    name = "ciphertext_sample.npy" if world == 1 else "ciphertext_sample_rank%d.npy" % rank
+    np.save(os.path.join(out_dir, name), windows.cpu().numpy().astype(np.float32))
+    if rank == 0:
+        np.save(os.path.join(out_dir, "tag.npy"), d_tag.cpu().numpy().astype(np.float32))
+
+
 def run_ours(args, rank, world, local_rank):
     import torch
     import aesgcm_b200
@@ -551,6 +570,8 @@ def run_ours(args, rank, world, local_rank):
     value = total * args.steps / (ms * 1e-3) / 1e9
     if px is not None:
         px.check()   # raises if any exchange failed closed
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rank, world, d_out, d_tag)   # before the strong-scaling steps reuse both
 
     # the work was real: the plaintext round-trips on this rank's shard (the tag was checked above)
     d_chk = torch.empty_like(d_in)
@@ -695,7 +716,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's tag and a fixed ciphertext sample as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs; the reference arm times a host-dependent sample")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -28,3 +28,33 @@ def test_reference_arm_other_ranks_exit_quietly():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1"],
                          capture_output=True, text=True, env=env, timeout=120)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+def test_steps_below_one_refused():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"],
+                         capture_output=True, text=True, timeout=120)
+    assert out.returncode == 2 and "--steps" in out.stderr
+
+
+def test_dump_outputs_files(tmp_path):
+    """--dump-outputs: the tag and seeded 4 KiB ciphertext windows, as float32, within 64 MB."""
+    import numpy as np
+    import torch
+    import bench
+    g = torch.Generator()
+    g.manual_seed(0)
+    ct = torch.randint(0, 256, (1 << 24,), dtype=torch.uint8, generator=g)
+    tag = torch.arange(16, dtype=torch.uint8)
+    bench.dump_outputs(str(tmp_path), 0, 1, ct, tag)
+    assert sorted(os.listdir(tmp_path)) == ["ciphertext_sample.npy", "tag.npy"]
+    assert np.load(tmp_path / "tag.npy").tolist() == list(range(16))
+    got = np.load(tmp_path / "ciphertext_sample.npy")
+    assert got.dtype == np.float32 and got.shape == (bench.DUMP_WINDOWS, bench.DUMP_WINDOW)
+    pick = np.sort(np.random.default_rng(3).choice(ct.numel() // bench.DUMP_WINDOW, bench.DUMP_WINDOWS, replace=False))
+    want = ct.numpy().reshape(-1, bench.DUMP_WINDOW)[pick]
+    assert np.array_equal(got, want)
+    assert sum(os.path.getsize(tmp_path / f) for f in os.listdir(tmp_path)) <= 64 << 20
+    # one file per rank when the stream is split, the tag once
+    bench.dump_outputs(str(tmp_path / "n2"), 1, 2, ct, tag)
+    assert os.listdir(tmp_path / "n2") == ["ciphertext_sample_rank1.npy"]
+    assert np.load(tmp_path / "n2" / "ciphertext_sample_rank1.npy").shape == (bench.DUMP_WINDOWS // 2, bench.DUMP_WINDOW)
