@@ -34,6 +34,23 @@ constexpr size_t SC_PARTS = 256;     // list of 16 B partials for finish (user p
 constexpr size_t SC_PARTS_MAX = 1024;
 constexpr size_t SC_BYTES = SC_PARTS + 16 * (SC_PARTS_MAX + 1);
 
+// device buffer grown on demand (grow()): the capacity only grows, and the contents are not preserved
+template <class T>
+struct GrownBuf {
+    T* p = nullptr;
+    size_t cap = 0;   // bytes
+};
+
+// A power of H cached on the device.  It is produced asynchronously by k_pow on whichever stream asked
+// first; a later consumer on a DIFFERENT stream (a user stream, the library's pipeline or side streams)
+// must not read it before that launch ran.
+struct PowCache {
+    uint32_t* d = nullptr;       // 4 BE words
+    uint64_t e = ~0ull;          // exponent it was computed for (~0 = none)
+    cudaEvent_t ev = nullptr;    // recorded after the producing launch
+    cudaStream_t st = nullptr;   // the producer's stream
+};
+
 }  // namespace
 
 struct agcm_ctx {
@@ -41,17 +58,13 @@ struct agcm_ctx {
     uint32_t* d_te0 = nullptr;
     KeyDev* d_key = nullptr;
     uint32_t* d_parts = nullptr;  // 2 x AG_MAX_CTA x 4 words: [0] CT partials, [1] AAD partials
-    uint32_t* d_seg_parts = nullptr;  // split batch layout: n_msgs x (split + 1) x 16 B, grown on demand
-    size_t seg_parts_bytes = 0;
+    GrownBuf<uint32_t> seg_parts;    // split batch layouts: segment partials and unit scratch
     uint8_t* d_scratch = nullptr;
     uint32_t* d_counters = nullptr;  // last-CTA tickets: [0] context scratch, [1+s] pipeline slot s
-    uint32_t* d_pow_n = nullptr;     // cached H^n (4 BE words) for the tag finish
-    uint64_t pow_n = ~0ull;          // exponent it was computed for (~0 = none)
-    uint32_t* d_pow_scale = nullptr; // cached H^blocks_after of the last shard call (4 BE words)
-    uint64_t pow_scale_e = ~0ull;
+    PowCache pow_n;                  // H^n for the tag finish
+    PowCache pow_scale;              // H^blocks_after of the last shard call
     uint32_t j0ctr = 1;              // counter field of J0 for the call in progress (1 for a 96-bit IV)
-    uint8_t* d_iv_stage = nullptr;   // padded long IV for the J0 derivation
-    size_t iv_stage_cap = 0;
+    GrownBuf<uint8_t> iv_stage;      // padded long IV for the J0 derivation
     // peer-memory exchange (multi-GPU)
     uint8_t** d_peer_bufs = nullptr; // device array of world pointers
     uint32_t* d_peer_status = nullptr;
@@ -62,9 +75,6 @@ struct agcm_ctx {
     cudaStream_t peer_side = nullptr;    // the finishes wait for the world's flags here, off the caller's stream
     cudaEvent_t peer_bulk_ev[AG_PEER_RING] = {};
     cudaEvent_t peer_fin_ev[AG_PEER_RING] = {};
-    // producer of the cached powers (a consumer on another stream waits for the event)
-    cudaEvent_t pow_n_ev = nullptr, pow_scale_ev = nullptr;
-    cudaStream_t pow_n_st = nullptr, pow_scale_st = nullptr;
     uint32_t h_rk[60];
     uint8_t h_H[16];
     uint8_t h_key_in[240];           // the key as it was loaded, to recognise a reload of the same key
@@ -87,15 +97,12 @@ struct agcm_ctx {
     uint8_t* d_stage_aux[kSlots] = {nullptr, nullptr, nullptr};  // iv / aad / tag / ok for batch chunks
     uint32_t* d_stage_parts[kSlots] = {nullptr, nullptr, nullptr};
     uint8_t* d_chunk_partials = nullptr;
-    uint8_t* d_aad_stage = nullptr;
-    size_t aad_stage_cap = 0;
+    GrownBuf<uint8_t> aad_stage;         // host-supplied AAD
     uint32_t* d_tile_ticket = nullptr;   // k_batch_tile / _warp / _cta: next unit (zeroed before each launch)
     bool no_ticket = false;              // set while the host batch pipeline runs chunks on several streams at once
-    uint32_t* d_sort = nullptr;          // length sort of an offset batch: 4096 bucket counters, then perm[n_msgs]
-    size_t sort_cap = 0;
+    GrownBuf<uint32_t> sort;             // length sort of an offset batch: 4096 bucket counters, then perm[n_msgs]
     void* tmap_encode = nullptr;         // cuTensorMapEncodeTiled, resolved through the runtime (no link-time libcuda)
-    uint8_t* d_verify = nullptr;     // whole ciphertext of a verify-then-release host decrypt, grown on demand
-    size_t verify_cap = 0;
+    GrownBuf<uint8_t> verify;            // whole ciphertext of a verify-then-release host decrypt
     bool pipeline_ready = false;
     size_t chunk_bytes = 32u << 20;
     size_t ramp_base = 1u << 20;         // first and last granule of the host pipeline (host_sched.h)
@@ -146,24 +153,42 @@ int timing_drain(agcm_ctx* c)
     return AGCM_OK;
 }
 
-// A cached power is produced asynchronously by k_pow on whichever stream asked first; a later
-// consumer on a DIFFERENT stream (a user stream, the library's pipeline or side streams) must not
-// read it before that launch ran.
-int pow_publish(agcm_ctx* c, cudaEvent_t* ev, cudaStream_t* owner, cudaStream_t st)
+template <class T>
+int grow(agcm_ctx* c, GrownBuf<T>& b, size_t need)
 {
-    if (!*ev) AG_CUDA(c, cudaEventCreateWithFlags(ev, cudaEventDisableTiming));
-    AG_CUDA(c, cudaEventRecord(*ev, st));
-    *owner = st;
+    if (need <= b.cap) return AGCM_OK;
+    AG_CUDA(c, cudaFree(b.p));
+    b.p = nullptr;
+    b.cap = 0;
+    AG_CUDA(c, cudaMalloc(&b.p, need));
+    b.cap = need;
     return AGCM_OK;
 }
 
-int pow_consume(agcm_ctx* c, cudaEvent_t ev, cudaStream_t owner, cudaStream_t st)
+// c->d_tile_ticket with its first `words` words zeroed on `st` (allocated on first use)
+int zeroed_ticket(agcm_ctx* c, size_t words, cudaStream_t st, uint32_t*& ticket)
 {
-    if (ev && owner != st) AG_CUDA(c, cudaStreamWaitEvent(st, ev, 0));
+    if (!c->d_tile_ticket) AG_CUDA(c, cudaMalloc(&c->d_tile_ticket, 4 * sizeof(uint32_t)));
+    AG_CUDA(c, cudaMemsetAsync(c->d_tile_ticket, 0, words * sizeof(uint32_t), st));
+    ticket = c->d_tile_ticket;
     return AGCM_OK;
 }
 
-// the caller's stream waits for every peer finish issued so far (they may still read d_pow_n)
+// H^e in `pc` for a consumer on `st`: waits for the cached value's producer, and runs k_pow on `st` for a new exponent
+int pow_get(agcm_ctx* c, PowCache& pc, uint64_t e, cudaStream_t st)
+{
+    if (pc.ev && pc.st != st) AG_CUDA(c, cudaStreamWaitEvent(st, pc.ev, 0));
+    if (pc.e == e) return AGCM_OK;
+    AG_CUDA(c, ag_launch_pow(c->d_key, e, pc.d, st));
+    c->launches++;
+    pc.e = e;
+    if (!pc.ev) AG_CUDA(c, cudaEventCreateWithFlags(&pc.ev, cudaEventDisableTiming));
+    AG_CUDA(c, cudaEventRecord(pc.ev, st));
+    pc.st = st;
+    return AGCM_OK;
+}
+
+// the caller's stream waits for every peer finish issued so far (they may still read pow_n)
 int peer_join_stream(agcm_ctx* c, cudaStream_t st)
 {
     if (c->peer_epoch && c->peer_fin_ev[0]) AG_CUDA(c, cudaStreamWaitEvent(st, c->peer_fin_ev[c->peer_epoch % AG_PEER_RING], 0));
@@ -173,32 +198,42 @@ int peer_join_stream(agcm_ctx* c, cudaStream_t st)
 // H^n for the tag finish, computed once per (key, n) on the caller's stream
 int ensure_pow(agcm_ctx* c, uint64_t n_blocks, cudaStream_t st)
 {
-    if (c->pow_n == n_blocks) return pow_consume(c, c->pow_n_ev, c->pow_n_st, st);
-    int rc = peer_join_stream(c, st);   // a deferred finish of an earlier message may still read the old power
-    if (rc) return rc;
-    rc = pow_consume(c, c->pow_n_ev, c->pow_n_st, st);   // ... and so may a consumer ordered after the old producer
-    if (rc) return rc;
-    AG_CUDA(c, ag_launch_pow(c->d_key, n_blocks, c->d_pow_n, st));
-    c->launches++;
-    c->pow_n = n_blocks;
-    return pow_publish(c, &c->pow_n_ev, &c->pow_n_st, st);
+    if (c->pow_n.e != n_blocks) {
+        int rc = peer_join_stream(c, st);   // a deferred finish of an earlier message may still read the old power
+        if (rc) return rc;
+    }
+    return pow_get(c, c->pow_n, n_blocks, st);   // ... and so may a consumer ordered after the old producer
 }
 
-// optional tag finish fused into the stream kernel (single-shard message, short AAD)
-struct FuseFinish {
-    const uint8_t* aad;
-    uint64_t aad_len, ct_len;
-    uint8_t* tag_calc;
-    const uint8_t* tag_expected;
-    uint8_t* ok;
-};
+// Fields all three forms of the tag finish share.  On decrypt the computed tag goes to scratch, never to the caller.
+FinishParams finish_params(const agcm_ctx* c, int decrypt, const uint8_t iv[12], const uint8_t* d_aad, uint64_t aad_len,
+                           uint64_t ct_len, uint8_t* d_tag, uint8_t* d_ok, const uint32_t* hn)
+{
+    FinishParams f;
+    memset(&f, 0, sizeof(f));
+    memcpy(f.rk, c->h_rk, sizeof(f.rk));
+    f.nr = (uint32_t)c->nr;
+    iv_words(iv, f.iv);
+    f.j0w = __builtin_bswap32(c->j0ctr);
+    f.key = c->d_key;
+    f.te0 = c->d_te0;
+    f.aad = d_aad;
+    f.aad_len = aad_len;
+    f.ct_len = ct_len;
+    f.tag_calc = decrypt ? c->d_scratch + SC_TAGCALC : d_tag;
+    f.tag_expected = decrypt ? d_tag : nullptr;
+    f.ok = decrypt ? d_ok : nullptr;
+    f.hn = hn;
+    return f;
+}
 
 // GHASH partial of `n_bytes` at d_in (optionally also CTR) -> 16 B at d_partial16,
 // scaled by H^blocks_after; the fold of the per-CTA partials runs in the last CTA of
 // the same launch.  parts_raw: per-CTA scratch (AG_MAX_CTA x 4 words); counter: its ticket.
+// ff: the tag finish fused into the same launch (single-shard message, short AAD).
 int run_stream(agcm_ctx* c, int mode, const uint8_t iv[12], uint64_t first_block, const uint8_t* d_in, uint8_t* d_out,
                uint64_t n_bytes, uint64_t blocks_after, uint32_t* parts_raw, uint8_t* d_partial16, cudaStream_t st,
-               uint32_t* counter, const FuseFinish* ff = nullptr, uint32_t peer_epoch = 0, const uint8_t* gate = nullptr)
+               uint32_t* counter, const FinishParams* ff = nullptr, uint32_t peer_epoch = 0, const uint8_t* gate = nullptr)
 {
     if (n_bytes == 0) {
         if (d_partial16) AG_CUDA(c, cudaMemsetAsync(d_partial16, 0, 16, st));
@@ -225,20 +260,10 @@ int run_stream(agcm_ctx* c, int mode, const uint8_t iv[12], uint64_t first_block
         // this stream instead of seven dependent products in the tail of every launch.  The
         // host-pipeline chunks (their own streams, a different exponent each) compute it in the tail.
         if (blocks_after && counter == c->d_counters && mode != AG_MODE_GHASH_ONLY) {
-            if (c->pow_scale_e != blocks_after) {
-                if (!c->d_pow_scale) AG_CUDA(c, cudaMalloc(&c->d_pow_scale, 16));
-                int rc = pow_consume(c, c->pow_scale_ev, c->pow_scale_st, st);
-                if (rc) return rc;
-                AG_CUDA(c, ag_launch_pow(c->d_key, blocks_after, c->d_pow_scale, st));
-                c->launches++;
-                c->pow_scale_e = blocks_after;
-                rc = pow_publish(c, &c->pow_scale_ev, &c->pow_scale_st, st);
-                if (rc) return rc;
-            } else {
-                int rc = pow_consume(c, c->pow_scale_ev, c->pow_scale_st, st);
-                if (rc) return rc;
-            }
-            p.scale_pow = c->d_pow_scale;
+            if (!c->pow_scale.d) AG_CUDA(c, cudaMalloc(&c->pow_scale.d, 16));
+            int rc = pow_get(c, c->pow_scale, blocks_after, st);
+            if (rc) return rc;
+            p.scale_pow = c->pow_scale.d;
         }
         p.out16 = d_partial16;
         if (ff) {
@@ -249,7 +274,7 @@ int run_stream(agcm_ctx* c, int mode, const uint8_t iv[12], uint64_t first_block
             p.tag_calc = ff->tag_calc;
             p.tag_expected = ff->tag_expected;
             p.ok = ff->ok;
-            p.hn = c->d_pow_n;
+            p.hn = ff->hn;
         }
         if (peer_epoch) {   // post the scaled partial to every rank (k_peer_finish does the rest)
             p.peer_bufs = c->d_peer_bufs;
@@ -307,52 +332,68 @@ int run_finish(agcm_ctx* c, int decrypt, const uint8_t iv[12], const uint8_t* d_
         np = n_parts + 1;
         aad_inline = nullptr;
     }
-    FinishParams f;
-    memcpy(f.rk, c->h_rk, sizeof(f.rk));
-    f.nr = (uint32_t)c->nr;
-    iv_words(iv, f.iv);
-    f.j0w = __builtin_bswap32(c->j0ctr);
-    f.key = c->d_key;
-    f.te0 = c->d_te0;
-    f.parts = parts;
-    f.n_parts = (uint32_t)np;
-    f.aad = aad_inline;
-    f.aad_len = aad_len;
-    f.ct_len = ct_len;
-    f.tag_calc = decrypt ? c->d_scratch + SC_TAGCALC : d_tag;
-    f.tag_expected = decrypt ? d_tag : nullptr;
-    f.ok = decrypt ? d_ok : nullptr;
-    f.hn = nullptr;
     if (aad_inline) {
         int rc = ensure_pow(c, n_ct_blocks, st);
         if (rc) return rc;
-        f.hn = c->d_pow_n;
     }
+    FinishParams f = finish_params(c, decrypt, iv, aad_inline, aad_len, ct_len, d_tag, d_ok, aad_inline ? c->pow_n.d : nullptr);
+    f.parts = parts;
+    f.n_parts = (uint32_t)np;
     AG_CUDA(c, ag_launch_finish(f, st));
     c->launches++;
-    return AGCM_OK;
-}
-
-// device staging buffer for host-supplied AAD, grown on demand
-int reserve_aad_stage(agcm_ctx* c, uint64_t aad_len)
-{
-    if (aad_len <= c->aad_stage_cap) return AGCM_OK;
-    cudaFree(c->d_aad_stage);
-    c->d_aad_stage = nullptr;
-    c->aad_stage_cap = 0;
-    AG_CUDA(c, cudaMalloc(&c->d_aad_stage, aad_len));
-    c->aad_stage_cap = aad_len;
     return AGCM_OK;
 }
 
 // J0 of an IV that is not 96 bits long (SP 800-38D 7.1 step 2): GHASH_H(IV || 0^(s+64) || [len(IV)]_64),
 // computed by the device (k_stream<GHASH_ONLY>) and read back; the message then runs with the
 // first 96 bits of J0 as its "IV" and J0's last 32 bits as the counter field.  Synchronises `st`.
-int derive_j0(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len, uint8_t j0[16], cudaStream_t st);
-
-int ensure_pipeline(agcm_ctx* c)
+int derive_j0(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len, uint8_t j0[16], cudaStream_t st)
 {
-    if (c->pipeline_ready) return AGCM_OK;
+    if (!h_iv || iv_len == 0 || iv_len > (1ull << 32)) return AGCM_E_BAD_LEN;
+    if (!c->key_set) return AGCM_E_NO_KEY;
+    const size_t padded = ((iv_len + 15) & ~(size_t)15) + 16;
+    std::vector<uint8_t> buf(padded, 0);
+    memcpy(buf.data(), h_iv, iv_len);
+    const uint64_t bits = (uint64_t)iv_len * 8;
+    for (int i = 0; i < 8; ++i) buf[padded - 1 - i] = (uint8_t)(bits >> (8 * i));
+    int rc = grow(c, c->iv_stage, padded < 4096 ? 4096 : padded);
+    if (rc) return rc;
+    AG_CUDA(c, cudaMemcpyAsync(c->iv_stage.p, buf.data(), padded, cudaMemcpyHostToDevice, st));
+    const uint8_t iv0[12] = {0};
+    rc = run_stream(c, AG_MODE_GHASH_ONLY, iv0, 0, c->iv_stage.p, nullptr, padded, 0, c->d_parts, c->d_scratch + SC_J0, st,
+                    c->d_counters);
+    if (rc) return rc;
+    AG_CUDA(c, cudaMemcpyAsync(j0, c->d_scratch + SC_J0, 16, cudaMemcpyDeviceToHost, st));
+    AG_CUDA(c, cudaStreamSynchronize(st));
+    return AGCM_OK;
+}
+
+// J0 of an IV of any length: IV || 0^31 || 1 for a 96-bit IV (no launch), else derive_j0 on `st`
+int resolve_j0(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len, uint8_t j0[16], cudaStream_t st)
+{
+    if (iv_len != 12) return derive_j0(c, h_iv, iv_len, j0, st);
+    memcpy(j0, h_iv, 12);
+    j0[12] = j0[13] = j0[14] = 0;
+    j0[15] = 1;
+    return AGCM_OK;
+}
+
+// The counter field of J0 replaces the constant 1 of the 96-bit case for the duration of a call.
+struct J0Scope {
+    agcm_ctx* c;
+    J0Scope(agcm_ctx* ctx, const uint8_t j0[16]) : c(ctx)
+    {
+        if (c && j0) c->j0ctr = ((uint32_t)j0[12] << 24) | ((uint32_t)j0[13] << 16) | ((uint32_t)j0[14] << 8) | (uint32_t)j0[15];
+    }
+    ~J0Scope() { if (c) c->j0ctr = 1; }
+};
+
+// First steps of a host-buffer call (they may allocate, so before anything is enqueued): the device, the pipeline
+// (created on first use) and room for `aad_len` bytes of AAD
+int host_begin(agcm_ctx* c, uint64_t aad_len)
+{
+    AG_CUDA(c, cudaSetDevice(c->device));
+    if (c->pipeline_ready) return grow(c, c->aad_stage, aad_len);
     if (const char* e = getenv("AGCM_CHUNK_MB")) {
         const long mb = atol(e);
         if (mb >= 1 && (size_t)mb <= (kChunkBytesMax >> 20)) c->chunk_bytes = (size_t)mb << 20;
@@ -369,6 +410,17 @@ int ensure_pipeline(agcm_ctx* c)
     }
     AG_CUDA(c, cudaMalloc(&c->d_chunk_partials, 16 * kMaxChunks));
     c->pipeline_ready = true;
+    return grow(c, c->aad_stage, aad_len);
+}
+
+// Last steps of a single-message host-buffer call: the ok byte (decrypt) or the tag out, then a wait for `st`.
+int host_end(agcm_ctx* c, int decrypt, uint8_t h_tag[16], int* h_ok, cudaStream_t st)
+{
+    uint8_t okb = 1;
+    if (decrypt) AG_CUDA(c, cudaMemcpyAsync(&okb, c->d_scratch + SC_OK, 1, cudaMemcpyDeviceToHost, st));
+    else AG_CUDA(c, cudaMemcpyAsync(h_tag, c->d_scratch + SC_TAG, 16, cudaMemcpyDeviceToHost, st));
+    AG_CUDA(c, cudaStreamSynchronize(st));
+    if (h_ok) *h_ok = okb ? 1 : 0;
     return AGCM_OK;
 }
 
@@ -388,7 +440,7 @@ int pick_lanes(const agcm_ctx* c, int lanes, uint64_t n_msgs, uint64_t avg_len, 
     const uint64_t total_lanes = (uint64_t)c->ncta * c->nt;
     const uint64_t blocks = (avg_len + 15) / 16 + 1;
     // From 32 KiB of work per message: one WARP per unit (k_batch_warp), units handed out by ticket,
-    // lane combine deferred to a second launch.  A unit is a message or one of S counter-range
+    // lane combine deferred to combine rounds of the same launch.  A unit is a message or one of S counter-range
     // segments of it; S keeps a unit near 64-256 rows of 32 blocks and gives every warp at least ~8
     // units to draw, so neither the per-unit overhead (a row or two) nor the tail matters.
     // (uniform batches say how many blocks a message really has, AAD included: bulk AAD counts in full here,
@@ -459,35 +511,6 @@ int pick_lanes(const agcm_ctx* c, int lanes, uint64_t n_msgs, uint64_t avg_len, 
 
 }  // namespace
 
-namespace {
-int derive_j0(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len, uint8_t j0[16], cudaStream_t st)
-{
-    if (!h_iv || iv_len == 0 || iv_len > (1ull << 32)) return AGCM_E_BAD_LEN;
-    if (!c->key_set) return AGCM_E_NO_KEY;
-    const size_t padded = ((iv_len + 15) & ~(size_t)15) + 16;
-    std::vector<uint8_t> buf(padded, 0);
-    memcpy(buf.data(), h_iv, iv_len);
-    const uint64_t bits = (uint64_t)iv_len * 8;
-    for (int i = 0; i < 8; ++i) buf[padded - 1 - i] = (uint8_t)(bits >> (8 * i));
-    if (padded > c->iv_stage_cap) {
-        AG_CUDA(c, cudaFree(c->d_iv_stage));
-        c->d_iv_stage = nullptr;
-        c->iv_stage_cap = 0;
-        const size_t cap = padded < 4096 ? 4096 : padded;
-        AG_CUDA(c, cudaMalloc(&c->d_iv_stage, cap));
-        c->iv_stage_cap = cap;
-    }
-    AG_CUDA(c, cudaMemcpyAsync(c->d_iv_stage, buf.data(), padded, cudaMemcpyHostToDevice, st));
-    const uint8_t iv0[12] = {0};
-    int rc = run_stream(c, AG_MODE_GHASH_ONLY, iv0, 0, c->d_iv_stage, nullptr, padded, 0, c->d_parts, c->d_scratch + SC_J0, st,
-                        c->d_counters);
-    if (rc) return rc;
-    AG_CUDA(c, cudaMemcpyAsync(j0, c->d_scratch + SC_J0, 16, cudaMemcpyDeviceToHost, st));
-    AG_CUDA(c, cudaStreamSynchronize(st));
-    return AGCM_OK;
-}
-}  // namespace
-
 #pragma GCC visibility push(default)
 extern "C" {
 
@@ -534,7 +557,7 @@ int agcm_ctx_create_ex(agcm_ctx** out, int device, int n_cta, int threads)
     if (e == cudaSuccess) e = cudaMemset(c->d_scratch, 0, SC_BYTES);
     if (e == cudaSuccess) e = cudaMalloc(&c->d_counters, sizeof(uint32_t) * (1 + kSlots));
     if (e == cudaSuccess) e = cudaMemset(c->d_counters, 0, sizeof(uint32_t) * (1 + kSlots));
-    if (e == cudaSuccess) e = cudaMalloc(&c->d_pow_n, 16);
+    if (e == cudaSuccess) e = cudaMalloc(&c->pow_n.d, 16);
     if (e == cudaSuccess) {
         uint8_t sbox[256];
         uint32_t te0[256];
@@ -571,19 +594,19 @@ void agcm_ctx_destroy(agcm_ctx* c)
     memset(c->h_H, 0, sizeof(c->h_H));
     memset(c->h_key_in, 0, sizeof(c->h_key_in));
     cudaFree(c->d_chunk_partials);
-    cudaFree(c->d_aad_stage);
-    cudaFree(c->d_verify);
+    cudaFree(c->aad_stage.p);
+    cudaFree(c->verify.p);
     cudaFree(c->d_tile_ticket);
-    cudaFree(c->d_sort);
+    cudaFree(c->sort.p);
     cudaFree(c->d_te0);
     cudaFree(c->d_key);
     cudaFree(c->d_parts);
-    cudaFree(c->d_seg_parts);
-    cudaFree(c->d_iv_stage);
+    cudaFree(c->seg_parts.p);
+    cudaFree(c->iv_stage.p);
     cudaFree(c->d_scratch);
     cudaFree(c->d_counters);
-    cudaFree(c->d_pow_n);
-    cudaFree(c->d_pow_scale);
+    cudaFree(c->pow_n.d);
+    cudaFree(c->pow_scale.d);
     cudaFree(c->d_peer_bufs);
     cudaFree(c->d_peer_status);
     if (c->h_peer_status) cudaFreeHost(c->h_peer_status);
@@ -592,8 +615,8 @@ void agcm_ctx_destroy(agcm_ctx* c)
         if (c->peer_bulk_ev[i]) cudaEventDestroy(c->peer_bulk_ev[i]);
         if (c->peer_fin_ev[i]) cudaEventDestroy(c->peer_fin_ev[i]);
     }
-    if (c->pow_n_ev) cudaEventDestroy(c->pow_n_ev);
-    if (c->pow_scale_ev) cudaEventDestroy(c->pow_scale_ev);
+    if (c->pow_n.ev) cudaEventDestroy(c->pow_n.ev);
+    if (c->pow_scale.ev) cudaEventDestroy(c->pow_scale.ev);
     delete c;
 }
 
@@ -673,8 +696,8 @@ int agcm_set_key(agcm_ctx* c, int mode, int pre_expanded, const uint8_t* h_key, 
         return AGCM_OK;
     AG_CUDA(c, cudaSetDevice(c->device));
     c->key_set = false;
-    c->pow_n = ~0ull;
-    c->pow_scale_e = ~0ull;
+    c->pow_n.e = ~0ull;
+    c->pow_scale.e = ~0ull;
     KeyIn in;
     memset(&in, 0, sizeof(in));
     memcpy(in.w, h_key, key_len);   // LE words == the byte string
@@ -759,13 +782,7 @@ int agcm_stream_crypt(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], const 
         if (!d_in || !d_out || (aad_len && !d_aad) || !d_tag || (decrypt && !d_ok)) return AGCM_E_BAD_ARG;
         if (((n_bytes + 15) >> 4) > kMaxBlocks) return AGCM_E_COUNTER_OVERFLOW;
         AG_CUDA(c, cudaSetDevice(c->device));
-        FuseFinish ff;
-        ff.aad = aad_len ? d_aad : nullptr;
-        ff.aad_len = aad_len;
-        ff.ct_len = n_bytes;
-        ff.tag_calc = decrypt ? c->d_scratch + SC_TAGCALC : d_tag;
-        ff.tag_expected = decrypt ? d_tag : nullptr;
-        ff.ok = decrypt ? d_ok : nullptr;
+        const FinishParams ff = finish_params(c, decrypt, h_iv12, aad_len ? d_aad : nullptr, aad_len, n_bytes, d_tag, d_ok, c->pow_n.d);
         if (aad_len) {
             int rc = ensure_pow(c, (n_bytes + 15) >> 4, (cudaStream_t)stream);
             if (rc) return rc;
@@ -785,12 +802,10 @@ int agcm_stream_crypt_iv(agcm_ctx* c, int decrypt, const uint8_t* h_iv, size_t i
     if (iv_len == 12) return agcm_stream_crypt(c, decrypt, h_iv, d_aad, aad_len, d_in, d_out, n_bytes, d_tag, d_ok, stream);
     AG_CUDA(c, cudaSetDevice(c->device));
     uint8_t j0[16];
-    int rc = derive_j0(c, h_iv, iv_len, j0, (cudaStream_t)stream);
+    int rc = resolve_j0(c, h_iv, iv_len, j0, (cudaStream_t)stream);
     if (rc) return rc;
-    c->j0ctr = ((uint32_t)j0[12] << 24) | ((uint32_t)j0[13] << 16) | ((uint32_t)j0[14] << 8) | (uint32_t)j0[15];
-    rc = agcm_stream_crypt(c, decrypt, j0, d_aad, aad_len, d_in, d_out, n_bytes, d_tag, d_ok, stream);
-    c->j0ctr = 1;
-    return rc;
+    J0Scope scope(c, j0);
+    return agcm_stream_crypt(c, decrypt, j0, d_aad, aad_len, d_in, d_out, n_bytes, d_tag, d_ok, stream);
 }
 
 int agcm_peer_setup(agcm_ctx* c, int rank, int world, const uint64_t* h_peer_ptrs)
@@ -878,19 +893,8 @@ static int peer_finish(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], const
     c->peer_epoch = epoch;
     PeerFinishParams pf;
     memset(&pf, 0, sizeof(pf));
-    memcpy(pf.f.rk, c->h_rk, sizeof(pf.f.rk));
-    pf.f.nr = (uint32_t)c->nr;
-    iv_words(h_iv12, pf.f.iv);
-    pf.f.j0w = __builtin_bswap32(c->j0ctr);
-    pf.f.key = c->d_key;
-    pf.f.te0 = c->d_te0;
-    pf.f.aad = aad_len ? d_aad : nullptr;
-    pf.f.aad_len = aad_len;
-    pf.f.ct_len = total_len;
-    pf.f.tag_calc = decrypt ? c->d_scratch + SC_TAGCALC : d_tag;
-    pf.f.tag_expected = decrypt ? d_tag : nullptr;
-    pf.f.ok = decrypt ? d_ok : nullptr;
-    pf.f.hn = aad_len ? c->d_pow_n : nullptr;
+    pf.f = finish_params(c, decrypt, h_iv12, aad_len ? d_aad : nullptr, aad_len, total_len, d_tag, d_ok,
+                         aad_len ? c->pow_n.d : nullptr);
     pf.peer_bufs = c->d_peer_bufs;
     pf.rank = (uint32_t)c->peer_rank;
     pf.world = (uint32_t)c->peer_world;
@@ -949,30 +953,12 @@ int agcm_stream_crypt_peer_async(agcm_ctx* c, int decrypt, const uint8_t h_iv12[
 }
 
 // ---- IVs of any length on the shard / peer / gctr entry points: the caller derives J0 once
-// (agcm_derive_j0) and passes it instead of the 12 IV bytes.  The counter field of J0 replaces
-// the constant 1 of the 96-bit case for the duration of the call.
-namespace {
-struct J0Scope {
-    agcm_ctx* c;
-    J0Scope(agcm_ctx* ctx, const uint8_t j0[16]) : c(ctx)
-    {
-        if (c && j0) c->j0ctr = ((uint32_t)j0[12] << 24) | ((uint32_t)j0[13] << 16) | ((uint32_t)j0[14] << 8) | (uint32_t)j0[15];
-    }
-    ~J0Scope() { if (c) c->j0ctr = 1; }
-};
-}  // namespace
-
+// (agcm_derive_j0) and passes it instead of the 12 IV bytes (J0Scope).
 int agcm_derive_j0(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len, uint8_t h_j0[16])
 {
     if (!c || !h_iv || !h_j0) return AGCM_E_BAD_ARG;
-    if (iv_len == 12) {
-        memcpy(h_j0, h_iv, 12);
-        h_j0[12] = h_j0[13] = h_j0[14] = 0;
-        h_j0[15] = 1;
-        return AGCM_OK;
-    }
-    AG_CUDA(c, cudaSetDevice(c->device));
-    return derive_j0(c, h_iv, iv_len, h_j0, nullptr);
+    if (iv_len != 12) AG_CUDA(c, cudaSetDevice(c->device));
+    return resolve_j0(c, h_iv, iv_len, h_j0, nullptr);   // the legacy stream: this call takes none
 }
 
 int agcm_gctr_j0(agcm_ctx* c, const uint8_t h_j0[16], uint64_t first_block, const uint8_t* d_in, uint8_t* d_out,
@@ -1019,7 +1005,7 @@ int agcm_stream_decrypt_verified(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len
     AG_CUDA(c, cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
     uint8_t j0[16];
-    int rc = agcm_derive_j0(c, h_iv, iv_len, j0);
+    int rc = resolve_j0(c, h_iv, iv_len, j0, st);   // on `st`: the caller's earlier work there may use the same scratch
     if (rc) return rc;
     J0Scope scope(c, j0);
     // pass 1: GHASH over the ciphertext only (about 4x the rate of the fused pass), then the tag check
@@ -1058,17 +1044,23 @@ int agcm_ghash(agcm_ctx* c, const uint8_t* d_in, uint64_t n_bytes, uint8_t* d_y1
 // scratch [4096-bucket histogram | 8 words of class bounds | perm[n_msgs]] and points p.perm at the order.
 static int len_sort(agcm_ctx* c, BatchParams& p, size_t n_msgs, cudaStream_t st)
 {
-    const size_t need_b = sizeof(uint32_t) * (4096 + 8 + n_msgs);
-    if (need_b > c->sort_cap) {
-        AG_CUDA(c, cudaFree(c->d_sort));
-        c->d_sort = nullptr;
-        c->sort_cap = 0;
-        AG_CUDA(c, cudaMalloc(&c->d_sort, need_b));
-        c->sort_cap = need_b;
-    }
-    AG_CUDA(c, ag_launch_len_sort(p, c->d_sort, c->d_sort + 4096, c->d_sort + 4096 + 8, st));
+    int rc = grow(c, c->sort, sizeof(uint32_t) * (4096 + 8 + n_msgs));
+    if (rc) return rc;
+    AG_CUDA(c, ag_launch_len_sort(p, c->sort.p, c->sort.p + 4096, c->sort.p + 4096 + 8, st));
     c->launches += 3;
-    p.perm = c->d_sort + 4096 + 8;
+    p.perm = c->sort.p + 4096 + 8;
+    return AGCM_OK;
+}
+
+// The argument check every shared-key batch kernel needs, then the context's key bound into p.
+static int batch_bind_key(agcm_ctx* c, int decrypt, BatchParams& p, size_t n_msgs)
+{
+    if (!p.iv || !p.tag || (decrypt && !p.ok)) return AGCM_E_BAD_ARG;
+    AG_CUDA(c, cudaSetDevice(c->device));
+    memcpy(p.rk, c->h_rk, sizeof(p.rk));
+    p.key = c->d_key;
+    p.te0 = c->d_te0;
+    p.n_msgs = n_msgs;
     return AGCM_OK;
 }
 
@@ -1077,16 +1069,12 @@ static int batch_common(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len, B
 {
     if (!c->key_set) return AGCM_E_NO_KEY;
     if (n_msgs == 0) return AGCM_OK;
-    if (!p.iv || !p.tag || (decrypt && !p.ok)) return AGCM_E_BAD_ARG;
+    int rc = batch_bind_key(c, decrypt, p, n_msgs);
+    if (rc) return rc;
     const bool ragged = p.in_off || p.aad_off || p.len_arr || p.aad_len_arr;   // messages of different lengths
     const uint64_t real_blocks = !ragged ? ((p.len + 15) >> 4) + (p.aad ? (p.aad_len + 15) >> 4 : 0) : 0;
     const int g = pick_lanes(c, lanes, n_msgs, avg_len, aligned16, real_blocks);
     if (g < 0) return AGCM_E_BAD_ARG;
-    AG_CUDA(c, cudaSetDevice(c->device));
-    memcpy(p.rk, c->h_rk, sizeof(p.rk));
-    p.key = c->d_key;
-    p.te0 = c->d_te0;
-    p.n_msgs = n_msgs;
     if (g > 4096) {
         // a warp per unit (k_batch_warp): balanced static partition for uniform batches, `split`
         // segments per message by ticket for offset batches
@@ -1113,15 +1101,9 @@ static int batch_common(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len, B
         const size_t zero_bytes = ((size_t)n_msgs * 20 + 255) & ~(size_t)255;
         const size_t desc_bytes = ((size_t)p.n_ids * 16 + 255) & ~(size_t)255;
         const size_t ej0_bytes = ((size_t)n_msgs * 16 + 255) & ~(size_t)255;
-        const size_t need = zero_bytes + desc_bytes + ej0_bytes + (size_t)p.n_ids * 512;
-        if (need > c->seg_parts_bytes) {
-            AG_CUDA(c, cudaFree(c->d_seg_parts));
-            c->d_seg_parts = nullptr;
-            c->seg_parts_bytes = 0;
-            AG_CUDA(c, cudaMalloc(&c->d_seg_parts, need));
-            c->seg_parts_bytes = need;
-        }
-        uint8_t* base = reinterpret_cast<uint8_t*>(c->d_seg_parts);
+        rc = grow(c, c->seg_parts, zero_bytes + desc_bytes + ej0_bytes + (size_t)p.n_ids * 512);
+        if (rc) return rc;
+        uint8_t* base = reinterpret_cast<uint8_t*>(c->seg_parts.p);
         p.msg_acc = reinterpret_cast<uint32_t*>(base);
         p.msg_cnt = reinterpret_cast<uint32_t*>(base + (size_t)n_msgs * 16);
         p.unit_desc = reinterpret_cast<uint64_t*>(base + zero_bytes);
@@ -1129,9 +1111,8 @@ static int batch_common(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len, B
         p.seg_acc = reinterpret_cast<uint4*>(base + zero_bytes + desc_bytes + ej0_bytes);
         AG_CUDA(c, cudaMemsetAsync(base, 0, zero_bytes, (cudaStream_t)stream));
         if (!uniform) {
-            if (!c->d_tile_ticket) AG_CUDA(c, cudaMalloc(&c->d_tile_ticket, 4 * sizeof(uint32_t)));
-            AG_CUDA(c, cudaMemsetAsync(c->d_tile_ticket, 0, sizeof(uint32_t), (cudaStream_t)stream));
-            p.ticket = c->d_tile_ticket;
+            rc = zeroed_ticket(c, 1, (cudaStream_t)stream, p.ticket);
+            if (rc) return rc;
         }
         AG_CUDA(c, ag_launch_batch_warp(p, c->nr, decrypt, ncta_w, (cudaStream_t)stream));
         c->launches++;
@@ -1141,21 +1122,14 @@ static int batch_common(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len, B
         p.split = g == 1024 ? 1u : (uint32_t)(g - 1024);
         const uint64_t n_units = (uint64_t)n_msgs * p.split;
         if (p.split > 1) {
-            const size_t need = (size_t)(n_units + n_msgs) * 16;
-            if (need > c->seg_parts_bytes) {
-                AG_CUDA(c, cudaFree(c->d_seg_parts));
-                c->d_seg_parts = nullptr;
-                c->seg_parts_bytes = 0;
-                AG_CUDA(c, cudaMalloc(&c->d_seg_parts, need));
-                c->seg_parts_bytes = need;
-            }
-            p.seg_parts = c->d_seg_parts;
+            rc = grow(c, c->seg_parts, (size_t)(n_units + n_msgs) * 16);
+            if (rc) return rc;
+            p.seg_parts = c->seg_parts.p;
         }
         const int ncta_m = (int)(n_units < (uint64_t)c->ncta ? n_units : (uint64_t)c->ncta);
         if (n_units > (uint64_t)ncta_m && n_units < 0xFFFFFFFFull && !c->no_ticket) {   // more units than CTAs: hand them out dynamically
-            if (!c->d_tile_ticket) AG_CUDA(c, cudaMalloc(&c->d_tile_ticket, 4 * sizeof(uint32_t)));
-            AG_CUDA(c, cudaMemsetAsync(c->d_tile_ticket, 0, sizeof(uint32_t), (cudaStream_t)stream));
-            p.ticket = c->d_tile_ticket;
+            rc = zeroed_ticket(c, 1, (cudaStream_t)stream, p.ticket);
+            if (rc) return rc;
         }
         AG_CUDA(c, ag_launch_batch_cta(p, c->nr, decrypt, ncta_m, c->nt, (cudaStream_t)stream));
         c->launches += p.split > 1 ? 2 : 1;
@@ -1172,24 +1146,25 @@ static int batch_common(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len, B
         // 16 KiB of work, 4 from 4 KiB, 1 below -- a heavy tail of long messages must not crawl through one lane.
         // The class sizes stay on the device (no host round trip): an empty class costs one idle launch.
         cudaStream_t st = (cudaStream_t)stream;
-        if (!c->d_tile_ticket) AG_CUDA(c, cudaMalloc(&c->d_tile_ticket, 4 * sizeof(uint32_t)));
-        AG_CUDA(c, cudaMemsetAsync(c->d_tile_ticket, 0, 4 * sizeof(uint32_t), st));
-        int rc_sort = len_sort(c, p, n_msgs, st);
-        if (rc_sort) return rc_sort;
-        uint32_t* ranges = c->d_sort + 4096;
+        uint32_t* tickets = nullptr;
+        rc = zeroed_ticket(c, 4, st, tickets);
+        if (rc) return rc;
+        rc = len_sort(c, p, n_msgs, st);
+        if (rc) return rc;
+        uint32_t* ranges = c->sort.p + 4096;
         if (lanes == 0 && !getenv("AGCM_NO_LEN_CLASSES")) {
             // short class: one lane per message with realigned wide accesses when records sit at odd addresses,
             // two lanes (32 contiguous bytes per request) when they are 16-byte aligned
             const int gs[3] = {32, 4, (aligned16 && !p.in_off) ? 2 : 1};   // packed by offsets: alignment unknown
             for (int k = 0; k < 3; ++k) {
                 p.range = ranges + 2 * k;
-                p.ticket = c->d_tile_ticket + 1 + k;
+                p.ticket = tickets + 1 + k;
                 AG_CUDA(c, ag_launch_batch(p, c->nr, decrypt, gs[k], c->ncta, c->nt, st));
                 c->launches++;
             }
             return AGCM_OK;
         }
-        p.ticket = c->d_tile_ticket + 1;
+        p.ticket = tickets + 1;
     }
     AG_CUDA(c, ag_launch_batch(p, c->nr, decrypt, g, ncta, c->nt, (cudaStream_t)stream));
     c->launches++;
@@ -1237,24 +1212,58 @@ static bool tile_eligible(const agcm_ctx* c, int lanes, const BatchParams& p, si
     return p.len + p.aad_len <= 16384 && n_msgs >= (size_t)c->ncta * (size_t)c->nt;   // at least a group of 32 per warp
 }
 
+// Fixed-size, 16-byte aligned records under per-message keys: stage them by TMA (k_batch_perkey_tile) when there
+// are enough messages to fill the grid; AGCM_PERKEY_TILE=0 / 1 keeps the thread-per-message loads / forces it (A/B runs)
+static bool perkey_tile_eligible(const agcm_ctx* c, const BatchParams& p, size_t n_msgs)
+{
+    const char* ev = getenv("AGCM_PERKEY_TILE");
+    if (ev && ev[0] == '0') return false;
+    if (!p.len || p.len >= (1ull << 31) || n_msgs >= (1ull << 31) - 32) return false;
+    if ((((uintptr_t)p.in | (uintptr_t)p.out) & 15) || (p.stride & 15) || p.stride >= (1ull << 40)) return false;
+    if (ev && ev[0] == '1') return true;
+    // Measured (tools/bench_variants.py --only perkey, AES-256, 64 B AAD): at a 4096 B pitch the tiled kernel wins
+    // (341 vs 294 GB/s: a lane per message at a large power-of-two pitch camps on few DRAM channels), at 1504 B
+    // the thread-per-message kernel does (353 vs 335: its aligned 128-bit accesses are only ~5 % of the pipe, and
+    // the tiled kernel pays a PRMT more on three lookups in four for dropping Te1), at 64 B too (167 vs 164):
+    // tile from 2 KiB records.
+    return p.len >= 2048 && n_msgs >= (size_t)c->ncta * 448u * 2;
+}
+
+// t.b = p and in / out tensor maps of 16-byte-granular extents (the pitch is a multiple of 16 and >= len: both fit)
+static int tile_records(agcm_ctx* c, TileParams& t, const BatchParams& p)
+{
+    memset(&t, 0, sizeof(t));
+    t.b = p;
+    const uint64_t len_up = (p.len + 15) & ~15ull, len_down = p.len & ~15ull;
+    int rc = tile_tensor_map(c, &t.tm_in, p.in, len_up, p.stride, p.n_msgs);
+    if (rc) return rc;
+    return tile_tensor_map(c, &t.tm_out, p.out, len_down ? len_down : 16, p.stride, p.n_msgs);   // len < 16: never stored through
+}
+
+// The ticket zeroed, then k_batch_perkey_tile (per-key batch) or k_batch_tile on as many CTAs as its groups of 32 need
+static int tile_launch(agcm_ctx* c, TileParams& t, int nr, int decrypt, int gather, cudaStream_t st)
+{
+    int rc = zeroed_ticket(c, 1, st, t.ticket);
+    if (rc) return rc;
+    if (t.b.keys) {
+        AG_CUDA(c, ag_launch_batch_perkey_tile(t, nr, decrypt, c->ncta, st));
+    } else {
+        const uint64_t groups = (t.b.n_msgs + 31) / 32, per_cta = (uint64_t)AG_STREAM_NT_MAX / 32;
+        const uint64_t need = (groups + per_cta - 1) / per_cta;
+        const int ncta = (int)(need < (uint64_t)c->ncta ? need : (uint64_t)c->ncta);
+        AG_CUDA(c, ag_launch_batch_tile(t, nr, decrypt, gather, ncta, st));
+    }
+    c->launches++;
+    return AGCM_OK;
+}
+
 static int batch_tile(agcm_ctx* c, int decrypt, BatchParams& p, size_t n_msgs, cudaStream_t st)
 {
     if (!c->key_set) return AGCM_E_NO_KEY;
-    if (!p.iv || !p.tag || (decrypt && !p.ok)) return AGCM_E_BAD_ARG;
-    AG_CUDA(c, cudaSetDevice(c->device));
-    if (!c->d_tile_ticket) AG_CUDA(c, cudaMalloc(&c->d_tile_ticket, 4 * sizeof(uint32_t)));
-    TileParams t;
-    memset(&t, 0, sizeof(t));
-    memcpy(p.rk, c->h_rk, sizeof(p.rk));
-    p.key = c->d_key;
-    p.te0 = c->d_te0;
-    p.n_msgs = n_msgs;
-    t.b = p;
-    // 16-byte-granular extents (the pitch is a multiple of 16 and >= len, so both fit inside a record's pitch)
-    const uint64_t len_up = (p.len + 15) & ~15ull, len_down = p.len & ~15ull;
-    int rc = tile_tensor_map(c, &t.tm_in, p.in, len_up, p.stride, n_msgs);
+    int rc = batch_bind_key(c, decrypt, p, n_msgs);
     if (rc) return rc;
-    rc = tile_tensor_map(c, &t.tm_out, p.out, len_down ? len_down : 16, p.stride, n_msgs);   // len < 16: never stored through
+    TileParams t;
+    rc = tile_records(c, t, p);
     if (rc) return rc;
     if (p.aad && p.aad_len && !((uintptr_t)p.aad & 15) && !(p.aad_stride & 15) && p.aad_len < (1ull << 31) &&
         p.aad_stride < (1ull << 40)) {
@@ -1262,14 +1271,7 @@ static int batch_tile(agcm_ctx* c, int decrypt, BatchParams& p, size_t n_msgs, c
         if (rc) return rc;
         t.aad_tiled = 1;
     }
-    t.ticket = c->d_tile_ticket;
-    AG_CUDA(c, cudaMemsetAsync(c->d_tile_ticket, 0, sizeof(uint32_t), st));
-    const uint64_t groups = (n_msgs + 31) / 32, per_cta = (uint64_t)AG_STREAM_NT_MAX / 32;
-    const uint64_t need = (groups + per_cta - 1) / per_cta;
-    const int ncta = (int)(need < (uint64_t)c->ncta ? need : (uint64_t)c->ncta);
-    AG_CUDA(c, ag_launch_batch_tile(t, c->nr, decrypt, 0, ncta, st));
-    c->launches++;
-    return AGCM_OK;
+    return tile_launch(c, t, c->nr, decrypt, 0, st);
 }
 
 // Slots (fixed 16-byte aligned pitch, a length per message) through the row-gathering form of the tiled kernel:
@@ -1292,23 +1294,18 @@ static bool tile_slots_eligible(const agcm_ctx* c, int lanes, const BatchParams&
 static int batch_tile_slots(agcm_ctx* c, int decrypt, BatchParams& p, size_t n_msgs, cudaStream_t st)
 {
     if (!c->key_set) return AGCM_E_NO_KEY;
-    if (!p.iv || !p.tag || (decrypt && !p.ok)) return AGCM_E_BAD_ARG;
-    AG_CUDA(c, cudaSetDevice(c->device));
-    if (!c->d_tile_ticket) AG_CUDA(c, cudaMalloc(&c->d_tile_ticket, 4 * sizeof(uint32_t)));
-    memcpy(p.rk, c->h_rk, sizeof(p.rk));
-    p.key = c->d_key;
-    p.te0 = c->d_te0;
-    p.n_msgs = n_msgs;
+    int rc = batch_bind_key(c, decrypt, p, n_msgs);
+    if (rc) return rc;
     // length order (longest first): the 32 messages a warp takes side by side are equally long
     if (n_msgs >= 64 && !getenv("AGCM_NO_LEN_SORT")) {
-        int rc_sort = len_sort(c, p, n_msgs, st);
-        if (rc_sort) return rc_sort;
+        rc = len_sort(c, p, n_msgs, st);
+        if (rc) return rc;
     }
     TileParams t;
     memset(&t, 0, sizeof(t));
     t.b = p;
     // whole slots as rows: a lane masks what lies past its message, and rows are stored only where whole blocks are
-    int rc = tile_tensor_map(c, &t.tm_in, p.in, p.stride, p.stride, n_msgs, 1);
+    rc = tile_tensor_map(c, &t.tm_in, p.in, p.stride, p.stride, n_msgs, 1);
     if (rc) return rc;
     rc = tile_tensor_map(c, &t.tm_out, p.out, p.stride, p.stride, n_msgs, 1);
     if (rc) return rc;
@@ -1317,25 +1314,18 @@ static int batch_tile_slots(agcm_ctx* c, int decrypt, BatchParams& p, size_t n_m
         if (rc) return rc;
         t.aad_tiled = 1;
     }
-    t.ticket = c->d_tile_ticket;
-    AG_CUDA(c, cudaMemsetAsync(c->d_tile_ticket, 0, sizeof(uint32_t), st));
-    const uint64_t groups = (n_msgs + 31) / 32, per_cta = (uint64_t)AG_STREAM_NT_MAX / 32;
-    const uint64_t need = (groups + per_cta - 1) / per_cta;
-    const int ncta = (int)(need < (uint64_t)c->ncta ? need : (uint64_t)c->ncta);
-    AG_CUDA(c, ag_launch_batch_tile(t, c->nr, decrypt, 1, ncta, st));
-    c->launches++;
-    return AGCM_OK;
+    return tile_launch(c, t, c->nr, decrypt, 1, st);
 }
 
-static int batch_offsets(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len_hint, const uint8_t* d_iv, int iv_is_j0,
-                         const uint8_t* d_aad, const uint64_t* d_aad_off, const uint8_t* d_in, const uint64_t* d_in_off,
-                         uint8_t* d_out, uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
+// Checks and BatchParams of an offset batch (message i at in_off[i]) under the context's key or d_keys
+static int offsets_params(BatchParams& p, const uint8_t* d_keys, const uint8_t* d_iv, int iv_is_j0, const uint8_t* d_aad,
+                          const uint64_t* d_aad_off, const uint8_t* d_in, const uint64_t* d_in_off, uint8_t* d_out,
+                          uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs)
 {
-    if (!c) return AGCM_E_BAD_ARG;
     if (n_msgs && (!d_in_off || !d_in || !d_out)) return AGCM_E_BAD_ARG;
     if ((d_aad == nullptr) != (d_aad_off == nullptr)) return AGCM_E_BAD_ARG;
-    BatchParams p;
     memset(&p, 0, sizeof(p));
+    p.keys = d_keys;
     p.iv = d_iv;
     p.iv_is_j0 = iv_is_j0 ? 1u : 0u;
     p.aad = d_aad;
@@ -1345,21 +1335,21 @@ static int batch_offsets(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len_h
     p.out = d_out;
     p.tag = d_tag;
     p.ok = d_ok;
-    return batch_common(c, decrypt, lanes, avg_len_hint, p, n_msgs, stream);
+    return AGCM_OK;
 }
 
-static int batch_uniform(agcm_ctx* c, int decrypt, int lanes, const uint8_t* d_iv, int iv_is_j0, const uint8_t* d_aad,
-                         uint64_t aad_len, uint64_t aad_stride, const uint8_t* d_in, uint8_t* d_out, uint64_t len,
-                         uint64_t stride, uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
+// Checks and BatchParams of a uniform batch (`len`-byte records at a pitch of `stride`) under the context's key or d_keys
+static int uniform_params(BatchParams& p, const uint8_t* d_keys, const uint8_t* d_iv, int iv_is_j0, const uint8_t* d_aad,
+                          uint64_t aad_len, uint64_t aad_stride, const uint8_t* d_in, uint8_t* d_out, uint64_t len,
+                          uint64_t stride, uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs)
 {
-    if (!c) return AGCM_E_BAD_ARG;
     if (n_msgs && len && (!d_in || !d_out)) return AGCM_E_BAD_ARG;
     if (stride < len || (aad_len && (!d_aad || aad_stride < aad_len))) return AGCM_E_BAD_LEN;
     // counter range AND the 32-bit block index of the unified AAD | payload | length sequence
     if (((len + 15) >> 4) > kMaxBlocks || ((aad_len + 15) >> 4) + ((len + 15) >> 4) + 1 > 0xFFFFFFFFull)
         return AGCM_E_COUNTER_OVERFLOW;
-    BatchParams p;
     memset(&p, 0, sizeof(p));
+    p.keys = d_keys;
     p.iv = d_iv;
     p.iv_is_j0 = iv_is_j0 ? 1u : 0u;
     p.aad = aad_len ? d_aad : nullptr;
@@ -1371,6 +1361,28 @@ static int batch_uniform(agcm_ctx* c, int decrypt, int lanes, const uint8_t* d_i
     p.stride = stride;
     p.aad_len = aad_len;
     p.aad_stride = aad_stride;
+    return AGCM_OK;
+}
+
+static int batch_offsets(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len_hint, const uint8_t* d_iv, int iv_is_j0,
+                         const uint8_t* d_aad, const uint64_t* d_aad_off, const uint8_t* d_in, const uint64_t* d_in_off,
+                         uint8_t* d_out, uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
+{
+    if (!c) return AGCM_E_BAD_ARG;
+    BatchParams p;
+    int rc = offsets_params(p, nullptr, d_iv, iv_is_j0, d_aad, d_aad_off, d_in, d_in_off, d_out, d_tag, d_ok, n_msgs);
+    if (rc) return rc;
+    return batch_common(c, decrypt, lanes, avg_len_hint, p, n_msgs, stream);
+}
+
+static int batch_uniform(agcm_ctx* c, int decrypt, int lanes, const uint8_t* d_iv, int iv_is_j0, const uint8_t* d_aad,
+                         uint64_t aad_len, uint64_t aad_stride, const uint8_t* d_in, uint8_t* d_out, uint64_t len,
+                         uint64_t stride, uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
+{
+    if (!c) return AGCM_E_BAD_ARG;
+    BatchParams p;
+    int rc = uniform_params(p, nullptr, d_iv, iv_is_j0, d_aad, aad_len, aad_stride, d_in, d_out, len, stride, d_tag, d_ok, n_msgs);
+    if (rc) return rc;
     const bool aligned16 = ((((uintptr_t)d_in | (uintptr_t)d_out) | stride) & 15) == 0;
     if (lanes == 2048 && !tile_eligible(c, lanes, p, n_msgs)) return AGCM_E_BAD_ARG;
     if (n_msgs && tile_eligible(c, lanes, p, n_msgs)) return batch_tile(c, decrypt, p, n_msgs, (cudaStream_t)stream);
@@ -1453,26 +1465,32 @@ int agcm_batch_derive_j0(agcm_ctx* c, const uint8_t* d_iv, const uint64_t* d_iv_
     return AGCM_OK;
 }
 
-static int perkey_common(agcm_ctx* c, int mode, int decrypt, BatchParams& p, size_t n_msgs, void* stream)
+// tile: through k_batch_perkey_tile (perkey_tile_eligible); a forced tiled call goes to the launch even when empty
+static int perkey_common(agcm_ctx* c, int mode, int decrypt, BatchParams& p, size_t n_msgs, bool tile, cudaStream_t st)
 {
     const int nr = mode_to_nr(mode);
     if (!nr) return AGCM_E_BAD_MODE;
-    if (n_msgs == 0) return AGCM_OK;
+    if (n_msgs == 0 && !tile) return AGCM_OK;
     if (!p.keys || !p.iv || !p.tag || (decrypt && !p.ok)) return AGCM_E_BAD_ARG;
     AG_CUDA(c, cudaSetDevice(c->device));
     p.key = nullptr;
     p.te0 = c->d_te0;
     p.n_msgs = n_msgs;
+    if (tile) {
+        TileParams t;
+        int rc = tile_records(c, t, p);
+        if (rc) return rc;
+        return tile_launch(c, t, nr, decrypt, 0, st);
+    }
     if ((p.in_off || p.aad_off) && n_msgs >= 1024 && n_msgs < 0xFFFFFF00ull && !c->no_ticket && !getenv("AGCM_NO_LEN_SORT")) {
         // messages of different lengths, a message per lane: take them in length order (as batch_common does), so that
         // the 32 messages of a warp are equally long; thread g then works on perm[g], perm[g + grid], ...
-        int rc = len_sort(c, p, n_msgs, (cudaStream_t)stream);
+        int rc = len_sort(c, p, n_msgs, st);
         if (rc) return rc;
-        if (!c->d_tile_ticket) AG_CUDA(c, cudaMalloc(&c->d_tile_ticket, 4 * sizeof(uint32_t)));
-        AG_CUDA(c, cudaMemsetAsync(c->d_tile_ticket, 0, sizeof(uint32_t), (cudaStream_t)stream));
-        p.ticket = c->d_tile_ticket;   // groups of 32 messages, longest first, to whichever warp is free
+        rc = zeroed_ticket(c, 1, st, p.ticket);   // groups of 32 messages, longest first, to whichever warp is free
+        if (rc) return rc;
     }
-    AG_CUDA(c, ag_launch_batch_perkey(p, nr, decrypt, c->ncta, (cudaStream_t)stream));
+    AG_CUDA(c, ag_launch_batch_perkey(p, nr, decrypt, c->ncta, st));
     c->launches++;
     return AGCM_OK;
 }
@@ -1482,20 +1500,10 @@ int agcm_batch_crypt_perkey(agcm_ctx* c, int mode, int decrypt, const uint8_t* d
                             uint8_t* d_out, uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
 {
     if (!c) return AGCM_E_BAD_ARG;
-    if (n_msgs && (!d_in_off || !d_in || !d_out)) return AGCM_E_BAD_ARG;
-    if ((d_aad == nullptr) != (d_aad_off == nullptr)) return AGCM_E_BAD_ARG;
     BatchParams p;
-    memset(&p, 0, sizeof(p));
-    p.keys = d_keys;
-    p.iv = d_iv12;
-    p.aad = d_aad;
-    p.aad_off = d_aad_off;
-    p.in = d_in;
-    p.in_off = d_in_off;
-    p.out = d_out;
-    p.tag = d_tag;
-    p.ok = d_ok;
-    return perkey_common(c, mode, decrypt, p, n_msgs, stream);
+    int rc = offsets_params(p, d_keys, d_iv12, 0, d_aad, d_aad_off, d_in, d_in_off, d_out, d_tag, d_ok, n_msgs);
+    if (rc) return rc;
+    return perkey_common(c, mode, decrypt, p, n_msgs, false, (cudaStream_t)stream);
 }
 
 int agcm_batch_crypt_perkey_uniform(agcm_ctx* c, int mode, int decrypt, const uint8_t* d_keys, const uint8_t* d_iv12,
@@ -1504,59 +1512,10 @@ int agcm_batch_crypt_perkey_uniform(agcm_ctx* c, int mode, int decrypt, const ui
                                     size_t n_msgs, void* stream)
 {
     if (!c) return AGCM_E_BAD_ARG;
-    if (n_msgs && len && (!d_in || !d_out)) return AGCM_E_BAD_ARG;
-    if (stride < len || (aad_len && (!d_aad || aad_stride < aad_len))) return AGCM_E_BAD_LEN;
-    if (((len + 15) >> 4) > kMaxBlocks || ((aad_len + 15) >> 4) + ((len + 15) >> 4) + 1 > 0xFFFFFFFFull)
-        return AGCM_E_COUNTER_OVERFLOW;
     BatchParams p;
-    memset(&p, 0, sizeof(p));
-    p.keys = d_keys;
-    p.iv = d_iv12;
-    p.aad = aad_len ? d_aad : nullptr;
-    p.in = d_in;
-    p.out = d_out;
-    p.tag = d_tag;
-    p.ok = d_ok;
-    p.len = len;
-    p.stride = stride;
-    p.aad_len = aad_len;
-    p.aad_stride = aad_stride;
-    // fixed-size, 16-byte aligned records: stage them by TMA (k_batch_perkey_tile) when there are
-    // enough messages to fill the grid; AGCM_PERKEY_TILE=0 keeps the thread-per-message loads (A/B runs)
-    {
-        const char* ev = getenv("AGCM_PERKEY_TILE");
-        const bool force = ev && ev[0] == '1', off = ev && ev[0] == '0';
-        const bool fits = len && len < (1ull << 31) && n_msgs < (1ull << 31) - 32 && !(((uintptr_t)d_in | (uintptr_t)d_out) & 15) &&
-                          !(stride & 15) && stride < (1ull << 40);
-        // Measured (tools/bench_variants.py --only perkey, AES-256, 64 B AAD): at a 4096 B pitch the tiled kernel wins
-        // (341 vs 294 GB/s: a lane per message at a large power-of-two pitch camps on few DRAM channels), at 1504 B
-        // the thread-per-message kernel does (353 vs 335: its aligned 128-bit accesses are only ~5 % of the pipe, and
-        // the tiled kernel pays a PRMT more on three lookups in four for dropping Te1), at 64 B too (167 vs 164):
-        // tile from 2 KiB records.
-        if (fits && !off && (force || (len >= 2048 && n_msgs >= (size_t)c->ncta * 448u * 2))) {
-            const int nr = mode_to_nr(mode);
-            if (!nr) return AGCM_E_BAD_MODE;
-            if (!p.keys || !p.iv || !p.tag || (decrypt && !p.ok)) return AGCM_E_BAD_ARG;
-            AG_CUDA(c, cudaSetDevice(c->device));
-            if (!c->d_tile_ticket) AG_CUDA(c, cudaMalloc(&c->d_tile_ticket, 4 * sizeof(uint32_t)));
-            TileParams t;
-            memset(&t, 0, sizeof(t));
-            p.te0 = c->d_te0;
-            p.n_msgs = n_msgs;
-            t.b = p;
-            const uint64_t len_up = (len + 15) & ~15ull, len_down = len & ~15ull;
-            int rc = tile_tensor_map(c, &t.tm_in, d_in, len_up, stride, n_msgs);
-            if (rc) return rc;
-            rc = tile_tensor_map(c, &t.tm_out, d_out, len_down ? len_down : 16, stride, n_msgs);
-            if (rc) return rc;
-            t.ticket = c->d_tile_ticket;
-            AG_CUDA(c, cudaMemsetAsync(c->d_tile_ticket, 0, sizeof(uint32_t), (cudaStream_t)stream));
-            AG_CUDA(c, ag_launch_batch_perkey_tile(t, nr, decrypt, c->ncta, (cudaStream_t)stream));
-            c->launches++;
-            return AGCM_OK;
-        }
-    }
-    return perkey_common(c, mode, decrypt, p, n_msgs, stream);
+    int rc = uniform_params(p, d_keys, d_iv12, 0, d_aad, aad_len, aad_stride, d_in, d_out, len, stride, d_tag, d_ok, n_msgs);
+    if (rc) return rc;
+    return perkey_common(c, mode, decrypt, p, n_msgs, perkey_tile_eligible(c, p, n_msgs), (cudaStream_t)stream);
 }
 
 // ---------------------------------------------------------------------------
@@ -1586,7 +1545,7 @@ static uint64_t pick_chunk(const agcm_ctx* c, uint64_t n_bytes)
 
 // chunked H2D -> fused kernel -> D2H of one counter range; the per-chunk partials
 // (each scaled for everything after it, including `blocks_after0`) land in
-// c->d_chunk_partials[0..n_chunks).  Leaves the slot streams running.
+// c->d_chunk_partials[0..n_chunks).  Waits for slots 1..kSlots-1 and leaves hs[0] running.
 static int host_pipeline(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], uint64_t first_block0, const uint8_t* h_in,
                          uint8_t* h_out, uint64_t n_bytes, uint64_t blocks_after0, uint64_t* n_chunks_out)
 {
@@ -1612,6 +1571,7 @@ static int host_pipeline(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], uin
         AG_CUDA(c, cudaMemcpyAsync(h_out + off, c->d_stage[s], nb, cudaMemcpyDeviceToHost, st));
         off += nb;
     }
+    for (int s = 1; s < kSlots; ++s) AG_CUDA(c, cudaStreamSynchronize(c->hs[s]));
     *n_chunks_out = n_chunks;
     return AGCM_OK;
 }
@@ -1625,13 +1585,11 @@ int agcm_stream_part_host(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], ui
     if (first_block > kMaxBlocks || nb > kMaxBlocks - first_block || blocks_after > kMaxBlocks - first_block - nb)
         return AGCM_E_COUNTER_OVERFLOW;
     if (blocks_after && (n_bytes & 15)) return AGCM_E_BAD_LEN;
-    AG_CUDA(c, cudaSetDevice(c->device));
-    int rc = ensure_pipeline(c);
+    int rc = host_begin(c, 0);
     if (rc) return rc;
     uint64_t n_chunks = 0;
     rc = host_pipeline(c, decrypt, h_iv12, first_block, h_in, h_out, n_bytes, blocks_after, &n_chunks);
     if (rc) return rc;
-    for (int s = 1; s < kSlots; ++s) AG_CUDA(c, cudaStreamSynchronize(c->hs[s]));
     // xor of the chunk partials = this range's partial (exponent 0: already scaled)
     uint8_t* d_p = c->d_scratch + SC_PART_CT;
     if (n_chunks == 0) {
@@ -1652,27 +1610,17 @@ int agcm_stream_finish_host(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], 
         return AGCM_E_BAD_ARG;
     if (!c->key_set) return AGCM_E_NO_KEY;
     if (n_parts < 0 || (size_t)n_parts > kMaxChunks) return AGCM_E_BAD_ARG;
-    AG_CUDA(c, cudaSetDevice(c->device));
-    int rc = ensure_pipeline(c);
+    int rc = host_begin(c, aad_len);
     if (rc) return rc;
     cudaStream_t st = c->hs[0];
-    {
-        int rc_aad = reserve_aad_stage(c, aad_len);
-        if (rc_aad) return rc_aad;
-    }
-    if (aad_len) AG_CUDA(c, cudaMemcpyAsync(c->d_aad_stage, h_aad, aad_len, cudaMemcpyHostToDevice, st));
+    if (aad_len) AG_CUDA(c, cudaMemcpyAsync(c->aad_stage.p, h_aad, aad_len, cudaMemcpyHostToDevice, st));
     if (n_parts) AG_CUDA(c, cudaMemcpyAsync(c->d_chunk_partials, h_partials16, 16 * (size_t)n_parts, cudaMemcpyHostToDevice, st));
     uint8_t* d_tag = c->d_scratch + SC_TAG;
     uint8_t* d_ok = c->d_scratch + SC_OK;
     if (decrypt) AG_CUDA(c, cudaMemcpyAsync(d_tag, h_tag, 16, cudaMemcpyHostToDevice, st));
-    rc = run_finish(c, decrypt, h_iv12, c->d_chunk_partials, n_parts, c->d_aad_stage, aad_len, ct_len, d_tag, d_ok, st);
+    rc = run_finish(c, decrypt, h_iv12, c->d_chunk_partials, n_parts, c->aad_stage.p, aad_len, ct_len, d_tag, d_ok, st);
     if (rc) return rc;
-    uint8_t okb = 1;
-    if (decrypt) AG_CUDA(c, cudaMemcpyAsync(&okb, d_ok, 1, cudaMemcpyDeviceToHost, st));
-    else AG_CUDA(c, cudaMemcpyAsync(h_tag, d_tag, 16, cudaMemcpyDeviceToHost, st));
-    AG_CUDA(c, cudaStreamSynchronize(st));
-    if (h_ok) *h_ok = okb ? 1 : 0;
-    return AGCM_OK;
+    return host_end(c, decrypt, h_tag, h_ok, st);
 }
 
 int agcm_stream_crypt_peer_host(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], uint64_t first_block, const uint8_t* h_in,
@@ -1682,23 +1630,19 @@ int agcm_stream_crypt_peer_host(agcm_ctx* c, int decrypt, const uint8_t h_iv12[1
     if (!c || !h_iv12 || !h_tag || (n_bytes && (!h_in || !h_out)) || (aad_len && !h_aad) || (decrypt && !h_ok))
         return AGCM_E_BAD_ARG;
     if (c->peer_world < 1) return AGCM_E_BAD_ARG;
-    AG_CUDA(c, cudaSetDevice(c->device));
-    int rc = ensure_pipeline(c);
-    if (rc) return rc;
-    rc = reserve_aad_stage(c, aad_len);
+    int rc = host_begin(c, aad_len);
     if (rc) return rc;
     cudaStream_t st = c->hs[0];
     uint32_t epoch = 0;
     rc = peer_begin(c, first_block, n_bytes, blocks_after, aad_len, total_len, st, &epoch);
     if (rc) return rc;
-    if (aad_len) AG_CUDA(c, cudaMemcpyAsync(c->d_aad_stage, h_aad, aad_len, cudaMemcpyHostToDevice, st));
+    if (aad_len) AG_CUDA(c, cudaMemcpyAsync(c->aad_stage.p, h_aad, aad_len, cudaMemcpyHostToDevice, st));
     uint8_t* d_tag = c->d_scratch + SC_TAG;
     uint8_t* d_ok = c->d_scratch + SC_OK;
     if (decrypt) AG_CUDA(c, cudaMemcpyAsync(d_tag, h_tag, 16, cudaMemcpyHostToDevice, st));
     uint64_t n_chunks = 0;
     rc = host_pipeline(c, decrypt, h_iv12, first_block, h_in, h_out, n_bytes, blocks_after, &n_chunks);
     if (rc) return rc;
-    for (int s = 1; s < kSlots; ++s) AG_CUDA(c, cudaStreamSynchronize(c->hs[s]));
     const uint8_t* d_p = nullptr;   // null = the zero partial of an empty range
     if (n_chunks) {
         AG_CUDA(c, ag_launch_xor_parts(c->d_chunk_partials, (uint32_t)n_chunks, c->d_scratch + SC_PART_CT, st));
@@ -1707,13 +1651,10 @@ int agcm_stream_crypt_peer_host(agcm_ctx* c, int decrypt, const uint8_t h_iv12[1
     }
     AG_CUDA(c, ag_launch_peer_post(c->d_peer_bufs, (uint32_t)c->peer_rank, (uint32_t)c->peer_world, epoch, d_p, st));
     c->launches++;
-    rc = peer_finish(c, decrypt, h_iv12, c->d_aad_stage, aad_len, total_len, d_tag, d_ok, st, epoch, false);
+    rc = peer_finish(c, decrypt, h_iv12, c->aad_stage.p, aad_len, total_len, d_tag, d_ok, st, epoch, false);
     if (rc) return rc;
-    uint8_t okb = 1;
-    if (decrypt) AG_CUDA(c, cudaMemcpyAsync(&okb, d_ok, 1, cudaMemcpyDeviceToHost, st));
-    else AG_CUDA(c, cudaMemcpyAsync(h_tag, d_tag, 16, cudaMemcpyDeviceToHost, st));
-    AG_CUDA(c, cudaStreamSynchronize(st));
-    if (h_ok) *h_ok = okb ? 1 : 0;
+    rc = host_end(c, decrypt, h_tag, h_ok, st);
+    if (rc) return rc;
     if (*(volatile uint32_t*)c->h_peer_status) return AGCM_E_PEER_TIMEOUT;
     return AGCM_OK;
 }
@@ -1725,14 +1666,9 @@ int agcm_stream_crypt_host(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], c
         return AGCM_E_BAD_ARG;
     if (!c->key_set) return AGCM_E_NO_KEY;
     if (((n_bytes + 15) >> 4) > kMaxBlocks) return AGCM_E_COUNTER_OVERFLOW;
-    AG_CUDA(c, cudaSetDevice(c->device));
-    int rc = ensure_pipeline(c);
+    int rc = host_begin(c, aad_len);
     if (rc) return rc;
-    {
-        int rc_aad = reserve_aad_stage(c, aad_len);
-        if (rc_aad) return rc_aad;
-    }
-    if (aad_len) AG_CUDA(c, cudaMemcpyAsync(c->d_aad_stage, h_aad, aad_len, cudaMemcpyHostToDevice, c->hs[0]));
+    if (aad_len) AG_CUDA(c, cudaMemcpyAsync(c->aad_stage.p, h_aad, aad_len, cudaMemcpyHostToDevice, c->hs[0]));
     uint8_t* d_tag = c->d_scratch + SC_TAG;
     uint8_t* d_ok = c->d_scratch + SC_OK;
     const uint64_t one_shot = (c->ramp_base && 2 * c->ramp_base < c->chunk_bytes) ? 2 * c->ramp_base : c->chunk_bytes;
@@ -1742,31 +1678,20 @@ int agcm_stream_crypt_host(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], c
         cudaStream_t st = c->hs[0];
         AG_CUDA(c, cudaMemcpyAsync(c->d_stage[0], h_in, n_bytes, cudaMemcpyHostToDevice, st));
         if (decrypt) AG_CUDA(c, cudaMemcpyAsync(d_tag, h_tag, 16, cudaMemcpyHostToDevice, st));
-        rc = agcm_stream_crypt(c, decrypt, h_iv12, c->d_aad_stage, aad_len, c->d_stage[0], c->d_stage[0], n_bytes, d_tag, d_ok,
+        rc = agcm_stream_crypt(c, decrypt, h_iv12, c->aad_stage.p, aad_len, c->d_stage[0], c->d_stage[0], n_bytes, d_tag, d_ok,
                                st);
         if (rc) return rc;
         AG_CUDA(c, cudaMemcpyAsync(h_out, c->d_stage[0], n_bytes, cudaMemcpyDeviceToHost, st));
-        uint8_t okb1 = 1;
-        if (decrypt) AG_CUDA(c, cudaMemcpyAsync(&okb1, d_ok, 1, cudaMemcpyDeviceToHost, st));
-        else AG_CUDA(c, cudaMemcpyAsync(h_tag, d_tag, 16, cudaMemcpyDeviceToHost, st));
-        AG_CUDA(c, cudaStreamSynchronize(st));
-        if (h_ok) *h_ok = okb1 ? 1 : 0;
-        return AGCM_OK;
+    } else {
+        uint64_t n_chunks = 0;
+        rc = host_pipeline(c, decrypt, h_iv12, 0, h_in, h_out, n_bytes, 0, &n_chunks);
+        if (rc) return rc;
+        if (decrypt) AG_CUDA(c, cudaMemcpyAsync(d_tag, h_tag, 16, cudaMemcpyHostToDevice, c->hs[0]));
+        rc = run_finish(c, decrypt, h_iv12, c->d_chunk_partials, (int)n_chunks, c->aad_stage.p, aad_len, n_bytes, d_tag, d_ok,
+                        c->hs[0]);
+        if (rc) return rc;
     }
-    uint64_t n_chunks = 0;
-    rc = host_pipeline(c, decrypt, h_iv12, 0, h_in, h_out, n_bytes, 0, &n_chunks);
-    if (rc) return rc;
-    for (int s = 1; s < kSlots; ++s) AG_CUDA(c, cudaStreamSynchronize(c->hs[s]));
-    if (decrypt) AG_CUDA(c, cudaMemcpyAsync(d_tag, h_tag, 16, cudaMemcpyHostToDevice, c->hs[0]));
-    rc = run_finish(c, decrypt, h_iv12, c->d_chunk_partials, (int)n_chunks, c->d_aad_stage, aad_len, n_bytes, d_tag, d_ok,
-                    c->hs[0]);
-    if (rc) return rc;
-    uint8_t okb = 1;
-    if (decrypt) AG_CUDA(c, cudaMemcpyAsync(&okb, d_ok, 1, cudaMemcpyDeviceToHost, c->hs[0]));
-    else AG_CUDA(c, cudaMemcpyAsync(h_tag, d_tag, 16, cudaMemcpyDeviceToHost, c->hs[0]));
-    AG_CUDA(c, cudaStreamSynchronize(c->hs[0]));
-    if (h_ok) *h_ok = okb ? 1 : 0;
-    return AGCM_OK;
+    return host_end(c, decrypt, h_tag, h_ok, c->hs[0]);
 }
 
 int agcm_stream_decrypt_verified_host(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len, const uint8_t* h_aad, uint64_t aad_len,
@@ -1775,33 +1700,25 @@ int agcm_stream_decrypt_verified_host(agcm_ctx* c, const uint8_t* h_iv, size_t i
     if (!c || !h_iv || !h_tag || !h_ok || (n_bytes && (!h_ct || !h_pt)) || (aad_len && !h_aad)) return AGCM_E_BAD_ARG;
     if (!c->key_set) return AGCM_E_NO_KEY;
     if (((n_bytes + 15) >> 4) > kMaxBlocks) return AGCM_E_COUNTER_OVERFLOW;
-    AG_CUDA(c, cudaSetDevice(c->device));
-    int rc = ensure_pipeline(c);
+    int rc = host_begin(c, aad_len);
     if (rc) return rc;
-    rc = reserve_aad_stage(c, aad_len);
+    rc = grow(c, c->verify, n_bytes);   // the ciphertext stays in HBM between the two passes
     if (rc) return rc;
-    if (n_bytes > c->verify_cap) {   // the ciphertext stays in HBM between the two passes
-        AG_CUDA(c, cudaFree(c->d_verify));
-        c->d_verify = nullptr;
-        c->verify_cap = 0;
-        AG_CUDA(c, cudaMalloc(&c->d_verify, n_bytes));
-        c->verify_cap = n_bytes;
-    }
     uint8_t j0[16];
-    rc = agcm_derive_j0(c, h_iv, iv_len, j0);
+    rc = resolve_j0(c, h_iv, iv_len, j0, c->hs[0]);
     if (rc) return rc;
     J0Scope scope(c, j0);
     const uint64_t nblocks = (n_bytes + 15) >> 4, chunk = pick_chunk(c, n_bytes);
     const uint64_t n_chunks = (n_bytes + chunk - 1) / chunk;
     if (n_chunks > SC_PARTS_MAX) return AGCM_E_BAD_LEN;
     // pass 1: copy in and absorb, chunk by chunk (the copy of chunk k+1 overlaps the GHASH of chunk k)
-    if (aad_len) AG_CUDA(c, cudaMemcpyAsync(c->d_aad_stage, h_aad, aad_len, cudaMemcpyHostToDevice, c->hs[0]));
+    if (aad_len) AG_CUDA(c, cudaMemcpyAsync(c->aad_stage.p, h_aad, aad_len, cudaMemcpyHostToDevice, c->hs[0]));
     for (uint64_t k = 0; k < n_chunks; ++k) {
         const int s = (int)(k % kSlots);
         const uint64_t off = k * chunk, nb = (n_bytes - off) < chunk ? (n_bytes - off) : chunk;
         const uint64_t after = nblocks - (off >> 4) - ((nb + 15) >> 4);
-        AG_CUDA(c, cudaMemcpyAsync(c->d_verify + off, h_ct + off, nb, cudaMemcpyHostToDevice, c->hs[s]));
-        rc = run_stream(c, AG_MODE_GHASH_ONLY, j0, 0, c->d_verify + off, nullptr, nb, after, c->d_stage_parts[s],
+        AG_CUDA(c, cudaMemcpyAsync(c->verify.p + off, h_ct + off, nb, cudaMemcpyHostToDevice, c->hs[s]));
+        rc = run_stream(c, AG_MODE_GHASH_ONLY, j0, 0, c->verify.p + off, nullptr, nb, after, c->d_stage_parts[s],
                         c->d_chunk_partials + 16 * k, c->hs[s], c->d_counters + 1 + s);
         if (rc) return rc;
     }
@@ -1809,21 +1726,18 @@ int agcm_stream_decrypt_verified_host(agcm_ctx* c, const uint8_t* h_iv, size_t i
     uint8_t* d_tag = c->d_scratch + SC_TAG;
     uint8_t* d_ok = c->d_scratch + SC_OK;
     AG_CUDA(c, cudaMemcpyAsync(d_tag, h_tag, 16, cudaMemcpyHostToDevice, c->hs[0]));
-    rc = run_finish(c, 1, j0, c->d_chunk_partials, (int)n_chunks, c->d_aad_stage, aad_len, n_bytes, d_tag, d_ok, c->hs[0]);
+    rc = run_finish(c, 1, j0, c->d_chunk_partials, (int)n_chunks, c->aad_stage.p, aad_len, n_bytes, d_tag, d_ok, c->hs[0]);
     if (rc) return rc;
-    uint8_t okb = 0;
-    AG_CUDA(c, cudaMemcpyAsync(&okb, d_ok, 1, cudaMemcpyDeviceToHost, c->hs[0]));
-    AG_CUDA(c, cudaStreamSynchronize(c->hs[0]));
-    *h_ok = okb ? 1 : 0;
-    if (!okb) return AGCM_OK;   // not authentic: no plaintext byte leaves the device
+    rc = host_end(c, 1, nullptr, h_ok, c->hs[0]);
+    if (rc || !*h_ok) return rc;   // not authentic: no plaintext byte leaves the device
     // pass 2: GCTR in place, chunk by chunk, copy out
     for (uint64_t k = 0; k < n_chunks; ++k) {
         const int s = (int)(k % kSlots);
         const uint64_t off = k * chunk, nb = (n_bytes - off) < chunk ? (n_bytes - off) : chunk;
-        rc = run_stream(c, AG_MODE_CTR_ONLY, j0, off >> 4, c->d_verify + off, c->d_verify + off, nb, 0, c->d_stage_parts[s], nullptr,
+        rc = run_stream(c, AG_MODE_CTR_ONLY, j0, off >> 4, c->verify.p + off, c->verify.p + off, nb, 0, c->d_stage_parts[s], nullptr,
                         c->hs[s], c->d_counters + 1 + s);
         if (rc) return rc;
-        AG_CUDA(c, cudaMemcpyAsync(h_pt + off, c->d_verify + off, nb, cudaMemcpyDeviceToHost, c->hs[s]));
+        AG_CUDA(c, cudaMemcpyAsync(h_pt + off, c->verify.p + off, nb, cudaMemcpyDeviceToHost, c->hs[s]));
     }
     for (int s = 0; s < kSlots; ++s) AG_CUDA(c, cudaStreamSynchronize(c->hs[s]));
     return AGCM_OK;
@@ -1835,16 +1749,13 @@ int agcm_stream_crypt_iv_host(agcm_ctx* c, int decrypt, const uint8_t* h_iv, siz
 {
     if (!c || !h_iv) return AGCM_E_BAD_ARG;
     if (iv_len == 12) return agcm_stream_crypt_host(c, decrypt, h_iv, h_aad, aad_len, h_in, h_out, n_bytes, h_tag, h_ok);
-    AG_CUDA(c, cudaSetDevice(c->device));
-    int rc = ensure_pipeline(c);
+    int rc = host_begin(c, 0);
     if (rc) return rc;
     uint8_t j0[16];
-    rc = derive_j0(c, h_iv, iv_len, j0, c->hs[0]);
+    rc = resolve_j0(c, h_iv, iv_len, j0, c->hs[0]);
     if (rc) return rc;
-    c->j0ctr = ((uint32_t)j0[12] << 24) | ((uint32_t)j0[13] << 16) | ((uint32_t)j0[14] << 8) | (uint32_t)j0[15];
-    rc = agcm_stream_crypt_host(c, decrypt, j0, h_aad, aad_len, h_in, h_out, n_bytes, h_tag, h_ok);
-    c->j0ctr = 1;
-    return rc;
+    J0Scope scope(c, j0);
+    return agcm_stream_crypt_host(c, decrypt, j0, h_aad, aad_len, h_in, h_out, n_bytes, h_tag, h_ok);
 }
 
 int agcm_batch_crypt_uniform_host(agcm_ctx* c, int decrypt, int lanes, const uint8_t* h_iv12, const uint8_t* h_aad,
@@ -1856,8 +1767,7 @@ int agcm_batch_crypt_uniform_host(agcm_ctx* c, int decrypt, int lanes, const uin
     if (!c->key_set) return AGCM_E_NO_KEY;
     if (stride < len || (aad_len && aad_stride < aad_len)) return AGCM_E_BAD_LEN;
     if (n_msgs == 0) return AGCM_OK;
-    AG_CUDA(c, cudaSetDevice(c->device));
-    int rc = ensure_pipeline(c);
+    int rc = host_begin(c, 0);
     if (rc) return rc;
     // messages per chunk: payload fits the stage buffer, side data fits the aux buffer
     const uint64_t per_msg_aux = 12 + 16 + 1 + aad_stride + 16;

@@ -49,7 +49,7 @@ constexpr uint32_t AG_TILE_BOX_BYTES = 32, AG_TILE_BOX_MSGS = 32;
 // of different lengths in fixed-pitch slots, taken in the order b.perm
 cudaError_t ag_launch_batch_tile(const TileParams& p, int nr, int decrypt, int gather, int ncta, cudaStream_t st);
 cudaError_t ag_launch_batch_perkey_tile(const TileParams& p, int nr, int decrypt, int max_cta, cudaStream_t st);
-// k_batch_warp + k_batch_warp_reduce + k_batch_split_finish (p.split, p.seg_parts, p.seg_acc, p.ticket set)
+// k_batch_warp, units combined in the same launch (p.split, p.seg_acc, p.unit_desc, p.msg_*, p.ticket set)
 cudaError_t ag_launch_batch_warp(const BatchParams& p, int nr, int decrypt, int ncta, cudaStream_t st);
 // counting sort of a ragged batch by message length (longest first): perm[n_msgs], scratch hist[4096], and the
 // [start, end) slices of the order that hold the long / medium / short messages (ranges6)

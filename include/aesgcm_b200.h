@@ -214,7 +214,7 @@ int agcm_stream_crypt_peer_async(agcm_ctx* ctx, int decrypt, const uint8_t h_iv1
  * message (1,2,4,8,16,32; 1024 = one whole CTA per message; 1024+S, S a power of two up to 256 =
  * one CTA per 1/S of a message: counter-range segments whose scaled GHASH partials a second launch
  * XORs into the tag; 4096+S, 1 <= S <= 65536 = one WARP per 1/S of a message, units handed out by
- * an atomic ticket and the lane combine deferred to a second launch -- the layout chosen for
+ * an atomic ticket and the lane combine deferred to the end of the same launch -- the layout chosen for
  * messages from about 32 KiB; 2048 = the TMA-staged message-per-lane kernel, uniform and slots forms only,
  * 16-byte aligned buffers and pitch) or 0 = choose from n_msgs and avg_len_hint.  Every choice
  * produces the same bytes.  The segment / unit layouts keep their partials in a per-context

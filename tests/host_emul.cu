@@ -206,8 +206,8 @@ void perkey_nk(const BatchParams& p)
 
 // k_batch_warp's BALANCED partition on a virtual grid of n_warps warps (uniform records): warp w
 // owns the w-th equal share of the AAD axis and of the payload axis of the concatenated messages; every unit's 32 lane
-// accumulators are combined as k_batch_warp_reduce does (serial Horner with H, times H^after) and
-// XORed into the message accumulator; k_batch_warp_finish's tag step at the end.
+// accumulators are combined as k_batch_warp's combine rounds do (serial Horner with H, times H^after) and
+// XORed into the message accumulator; the tag step of the same kernel at the end.
 template <int NR, bool DEC>
 static void batch_balanced_nr(const BatchParams& p, uint32_t n_warps, const gf128& H)
 {

@@ -328,6 +328,21 @@ def test_decrypt_verified_releases_nothing_on_a_bad_tag(engine, oracle, torch_mo
         engine.stream_decrypt_verified_device(iv, d_aad, d_ct, d_pt, _dev(torch, np.frombuffer(tag, dtype=np.uint8)), d_ok, n_bytes=n)
         torch.cuda.synchronize()
         assert int(d_ok.item()) == 1 and d_pt[:n].cpu().numpy().tobytes() == pt.tobytes()
+        if ivl != 12:
+            # device form on a side stream, right behind the encryption that produced its ciphertext there (no
+            # synchronise in between): the J0 of the long IV has to be derived in that stream's order
+            d_src = _dev(torch, pt)
+            side = torch.cuda.Stream()
+            side.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(side):
+                d_ct2 = torch.empty_like(d_src)
+                d_tag2 = torch.zeros(16, dtype=torch.uint8, device="cuda")
+                engine.stream_crypt_device(0, iv, d_aad, d_src, d_ct2, d_tag2)
+                d_back = torch.full_like(d_src, 0x5A)
+                d_ok2 = torch.zeros(1, dtype=torch.uint8, device="cuda")
+                engine.stream_decrypt_verified_device(iv, d_aad, d_ct2, d_back, d_tag2, d_ok2)
+            side.synchronize()
+            assert int(d_ok2.item()) == 1 and torch.equal(d_back, d_src)
 
 
 @pytest.mark.parametrize("kb", [16, 24, 32])
