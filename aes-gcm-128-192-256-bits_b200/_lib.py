@@ -73,6 +73,20 @@ SIGNATURES = {
                                         c_sz, c_vp]),
     "agcm_batch_crypt_perkey_uniform": (c_int, [c_vp, c_int, c_int, c_u8p, c_u8p, c_u8p, c_u64, c_u64, c_u8p, c_u8p,
                                                 c_u64, c_u64, c_u8p, c_u8p, c_sz, c_vp]),
+    "agcm_batch_decrypt_verified": (c_int, [c_vp, c_int, c_u64, c_u8p, c_u8p, c_u8p, c_u8p, c_u8p, c_u8p, c_u8p, c_u8p, c_sz,
+                                            c_vp]),
+    "agcm_batch_decrypt_verified_j0": (c_int, [c_vp, c_int, c_u64, c_u8p, c_u8p, c_u8p, c_u8p, c_u8p, c_u8p, c_u8p, c_u8p, c_sz,
+                                               c_vp]),
+    "agcm_batch_decrypt_verified_uniform": (c_int, [c_vp, c_int, c_u8p, c_u8p, c_u64, c_u64, c_u8p, c_u8p, c_u64, c_u64, c_u8p,
+                                                    c_u8p, c_sz, c_vp]),
+    "agcm_batch_decrypt_verified_uniform_j0": (c_int, [c_vp, c_int, c_u8p, c_u8p, c_u64, c_u64, c_u8p, c_u8p, c_u64, c_u64, c_u8p,
+                                                       c_u8p, c_sz, c_vp]),
+    "agcm_batch_decrypt_verified_slots": (c_int, [c_vp, c_int, c_u8p, c_u8p, c_u8p, c_u64, c_u64, c_u8p, c_u8p, c_u8p, c_u64,
+                                                  c_u64, c_u8p, c_u8p, c_sz, c_vp]),
+    "agcm_batch_decrypt_verified_perkey": (c_int, [c_vp, c_int, c_u8p, c_u8p, c_u8p, c_u8p, c_u8p, c_u8p, c_u8p, c_u8p, c_u8p,
+                                                   c_sz, c_vp]),
+    "agcm_batch_decrypt_verified_perkey_uniform": (c_int, [c_vp, c_int, c_u8p, c_u8p, c_u8p, c_u64, c_u64, c_u8p, c_u8p, c_u64,
+                                                           c_u64, c_u8p, c_u8p, c_sz, c_vp]),
     "agcm_stream_crypt_host": (c_int, [c_vp, c_int, c_u8p, c_u8p, c_u64, c_u8p, c_u8p, c_u64, c_u8p,
                                        ctypes.POINTER(c_int)]),
     "agcm_stream_crypt_iv_host": (c_int, [c_vp, c_int, c_u8p, c_sz, c_u8p, c_u64, c_u8p, c_u8p, c_u64, c_u8p,

@@ -1064,8 +1064,9 @@ static int batch_bind_key(agcm_ctx* c, int decrypt, BatchParams& p, size_t n_msg
     return AGCM_OK;
 }
 
+// verify: pass 1 of the verify-then-release decrypt -- the tag-only flavour of the lane-group / warp-unit kernels
 static int batch_common(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len, BatchParams& p, size_t n_msgs, void* stream,
-                        bool aligned16 = true)
+                        bool aligned16 = true, bool verify = false)
 {
     if (!c->key_set) return AGCM_E_NO_KEY;
     if (n_msgs == 0) return AGCM_OK;
@@ -1073,8 +1074,9 @@ static int batch_common(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len, B
     if (rc) return rc;
     const bool ragged = p.in_off || p.aad_off || p.len_arr || p.aad_len_arr;   // messages of different lengths
     const uint64_t real_blocks = !ragged ? ((p.len + 15) >> 4) + (p.aad ? (p.aad_len + 15) >> 4 : 0) : 0;
-    const int g = pick_lanes(c, lanes, n_msgs, avg_len, aligned16, real_blocks);
+    int g = pick_lanes(c, lanes, n_msgs, avg_len, aligned16, real_blocks);
     if (g < 0) return AGCM_E_BAD_ARG;
+    if (verify && g >= 1024 && g <= 4096) g = 4097;   // no CTA layout for the tag-only pass: a warp per message
     if (g > 4096) {
         // a warp per unit (k_batch_warp): balanced static partition for uniform batches, `split`
         // segments per message by ticket for offset batches
@@ -1114,7 +1116,8 @@ static int batch_common(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len, B
             rc = zeroed_ticket(c, 1, (cudaStream_t)stream, p.ticket);
             if (rc) return rc;
         }
-        AG_CUDA(c, ag_launch_batch_warp(p, c->nr, decrypt, ncta_w, (cudaStream_t)stream));
+        AG_CUDA(c, verify ? ag_launch_batch_warp_verify(p, c->nr, ncta_w, (cudaStream_t)stream)
+                          : ag_launch_batch_warp(p, c->nr, decrypt, ncta_w, (cudaStream_t)stream));
         c->launches++;
         return AGCM_OK;
     }
@@ -1159,14 +1162,44 @@ static int batch_common(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len, B
             for (int k = 0; k < 3; ++k) {
                 p.range = ranges + 2 * k;
                 p.ticket = tickets + 1 + k;
-                AG_CUDA(c, ag_launch_batch(p, c->nr, decrypt, gs[k], c->ncta, c->nt, st));
+                AG_CUDA(c, verify ? ag_launch_batch_verify(p, c->nr, gs[k], c->ncta, c->nt, st)
+                                  : ag_launch_batch(p, c->nr, decrypt, gs[k], c->ncta, c->nt, st));
                 c->launches++;
             }
             return AGCM_OK;
         }
         p.ticket = tickets + 1;
     }
-    AG_CUDA(c, ag_launch_batch(p, c->nr, decrypt, g, ncta, c->nt, (cudaStream_t)stream));
+    AG_CUDA(c, verify ? ag_launch_batch_verify(p, c->nr, g, ncta, c->nt, (cudaStream_t)stream)
+                      : ag_launch_batch(p, c->nr, decrypt, g, ncta, c->nt, (cudaStream_t)stream));
+    c->launches++;
+    return AGCM_OK;
+}
+
+// Verify-then-release decrypt of a shared-key batch (p as the releasing decrypt would take it, d_out = the plaintext):
+// pass 1 writes ok[] only (avg_len: the work estimate of a GHASH-only pass), pass 2 (k_batch_ctr_gated) runs GCTR over
+// the messages whose ok[m] is 1.  Both in stream order, no host round trip.  lanes: 0, the lane groups and 4096 + S.
+static int batch_verified(agcm_ctx* c, int lanes, uint64_t avg_len, BatchParams& p, size_t n_msgs, void* stream, bool aligned16)
+{
+    if (!p.tag || !p.ok) return AGCM_E_BAD_ARG;
+    if (lanes >= 1024 && lanes <= 4096) return AGCM_E_BAD_ARG;   // the CTA and TMA-staged layouts have no tag-only form
+    if (!c->key_set) return AGCM_E_NO_KEY;
+    if (n_msgs == 0) return AGCM_OK;
+    int rc = batch_common(c, 1, lanes, avg_len, p, n_msgs, stream, aligned16, true);
+    if (rc) return rc;
+    // pass 2 takes the batch in its own order (flat slots): no sort, no tickets, no AAD
+    BatchParams g = p;
+    g.perm = nullptr;
+    g.range = nullptr;
+    g.ticket = nullptr;
+    g.aad = nullptr;
+    g.aad_off = nullptr;
+    g.aad_len_arr = nullptr;
+    // blocks per record pitch: the whole slot (slots form), the record (uniform form; the pitch past it is never touched)
+    const uint64_t bpr = p.len_arr ? (p.stride + 15) >> 4 : (p.len + 15) >> 4;
+    const uint64_t n_slots = p.in_off ? 0 : bpr * (uint64_t)n_msgs;
+    if (!p.in_off && n_slots == 0) return AGCM_OK;   // nothing to release
+    AG_CUDA(c, ag_launch_batch_ctr_gated(g, c->nr, n_slots, bpr, c->ncta, (cudaStream_t)stream));
     c->launches++;
     return AGCM_OK;
 }
@@ -1422,18 +1455,17 @@ int agcm_batch_crypt_uniform_j0(agcm_ctx* c, int decrypt, int lanes, const uint8
                          stream);
 }
 
-int agcm_batch_crypt_slots(agcm_ctx* c, int decrypt, int lanes, const uint8_t* d_iv12, const uint8_t* d_aad,
-                           const uint32_t* d_aad_len, uint64_t aad_len, uint64_t aad_stride, const uint8_t* d_in, uint8_t* d_out,
-                           const uint32_t* d_len, uint64_t stride, uint64_t avg_len_hint, uint8_t* d_tag, uint8_t* d_ok,
-                           size_t n_msgs, void* stream)
+// Checks and BatchParams of a slots batch (message i: d_len[i] bytes at i * stride)
+static int slots_params(BatchParams& p, const uint8_t* d_iv12, const uint8_t* d_aad, const uint32_t* d_aad_len, uint64_t aad_len,
+                        uint64_t aad_stride, const uint8_t* d_in, uint8_t* d_out, const uint32_t* d_len, uint64_t stride,
+                        uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs)
 {
-    if (!c || !d_len) return AGCM_E_BAD_ARG;
+    if (!d_len) return AGCM_E_BAD_ARG;
     if (n_msgs && stride && (!d_in || !d_out)) return AGCM_E_BAD_ARG;
     const bool has_aad = d_aad && (d_aad_len || aad_len);
     if (has_aad && (aad_stride < aad_len || aad_stride == 0)) return AGCM_E_BAD_LEN;
     if (((stride + 15) >> 4) > kMaxBlocks || ((aad_stride + 15) >> 4) + ((stride + 15) >> 4) + 1 > 0xFFFFFFFFull)
         return AGCM_E_COUNTER_OVERFLOW;   // no slot can hold a message beyond the limits
-    BatchParams p;
     memset(&p, 0, sizeof(p));
     p.iv = d_iv12;
     p.aad = has_aad ? d_aad : nullptr;
@@ -1447,10 +1479,94 @@ int agcm_batch_crypt_slots(agcm_ctx* c, int decrypt, int lanes, const uint8_t* d
     p.aad_len = has_aad ? aad_len : 0;
     p.aad_stride = has_aad ? aad_stride : 0;
     p.aad_len_arr = has_aad ? d_aad_len : nullptr;
+    return AGCM_OK;
+}
+
+int agcm_batch_crypt_slots(agcm_ctx* c, int decrypt, int lanes, const uint8_t* d_iv12, const uint8_t* d_aad,
+                           const uint32_t* d_aad_len, uint64_t aad_len, uint64_t aad_stride, const uint8_t* d_in, uint8_t* d_out,
+                           const uint32_t* d_len, uint64_t stride, uint64_t avg_len_hint, uint8_t* d_tag, uint8_t* d_ok,
+                           size_t n_msgs, void* stream)
+{
+    if (!c) return AGCM_E_BAD_ARG;
+    BatchParams p;
+    int rc = slots_params(p, d_iv12, d_aad, d_aad_len, aad_len, aad_stride, d_in, d_out, d_len, stride, d_tag, d_ok, n_msgs);
+    if (rc) return rc;
     const bool aligned16 = ((((uintptr_t)d_in | (uintptr_t)d_out) | stride) & 15) == 0;
     if (lanes == 2048 && !tile_slots_eligible(c, lanes, p, n_msgs)) return AGCM_E_BAD_ARG;   // needs 16-byte aligned slots
     if (n_msgs && tile_slots_eligible(c, lanes, p, n_msgs)) return batch_tile_slots(c, decrypt, p, n_msgs, (cudaStream_t)stream);
     return batch_common(c, decrypt, lanes, avg_len_hint ? avg_len_hint : stride / 2, p, n_msgs, stream, aligned16);
+}
+
+// ---- verify-then-release batch decrypt: the same checks as the releasing forms, then batch_verified ------------------
+static int batch_offsets_verified(agcm_ctx* c, int lanes, uint64_t avg_len_hint, const uint8_t* d_iv, int iv_is_j0,
+                                  const uint8_t* d_aad, const uint64_t* d_aad_off, const uint8_t* d_ct, const uint64_t* d_in_off,
+                                  uint8_t* d_pt, const uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
+{
+    if (!c) return AGCM_E_BAD_ARG;
+    BatchParams p;
+    int rc = offsets_params(p, nullptr, d_iv, iv_is_j0, d_aad, d_aad_off, d_ct, d_in_off, d_pt, const_cast<uint8_t*>(d_tag), d_ok,
+                            n_msgs);
+    if (rc) return rc;
+    return batch_verified(c, lanes, avg_len_hint / 4, p, n_msgs, stream, true);   // a payload block weighs what an AAD block does
+}
+
+static int batch_uniform_verified(agcm_ctx* c, int lanes, const uint8_t* d_iv, int iv_is_j0, const uint8_t* d_aad, uint64_t aad_len,
+                                  uint64_t aad_stride, const uint8_t* d_ct, uint8_t* d_pt, uint64_t len, uint64_t stride,
+                                  const uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
+{
+    if (!c) return AGCM_E_BAD_ARG;
+    BatchParams p;
+    int rc = uniform_params(p, nullptr, d_iv, iv_is_j0, d_aad, aad_len, aad_stride, d_ct, d_pt, len, stride,
+                            const_cast<uint8_t*>(d_tag), d_ok, n_msgs);
+    if (rc) return rc;
+    const bool aligned16 = ((((uintptr_t)d_ct | (uintptr_t)d_pt) | stride) & 15) == 0;
+    return batch_verified(c, lanes, (len + (d_aad ? aad_len : 0)) / 4, p, n_msgs, stream, aligned16);
+}
+
+int agcm_batch_decrypt_verified(agcm_ctx* c, int lanes, uint64_t avg_len_hint, const uint8_t* d_iv12, const uint8_t* d_aad,
+                                const uint64_t* d_aad_off, const uint8_t* d_ct, const uint64_t* d_in_off, uint8_t* d_pt,
+                                const uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
+{
+    return batch_offsets_verified(c, lanes, avg_len_hint, d_iv12, 0, d_aad, d_aad_off, d_ct, d_in_off, d_pt, d_tag, d_ok, n_msgs,
+                                  stream);
+}
+
+int agcm_batch_decrypt_verified_j0(agcm_ctx* c, int lanes, uint64_t avg_len_hint, const uint8_t* d_j0, const uint8_t* d_aad,
+                                   const uint64_t* d_aad_off, const uint8_t* d_ct, const uint64_t* d_in_off, uint8_t* d_pt,
+                                   const uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
+{
+    return batch_offsets_verified(c, lanes, avg_len_hint, d_j0, 1, d_aad, d_aad_off, d_ct, d_in_off, d_pt, d_tag, d_ok, n_msgs,
+                                  stream);
+}
+
+int agcm_batch_decrypt_verified_uniform(agcm_ctx* c, int lanes, const uint8_t* d_iv12, const uint8_t* d_aad, uint64_t aad_len,
+                                        uint64_t aad_stride, const uint8_t* d_ct, uint8_t* d_pt, uint64_t len, uint64_t stride,
+                                        const uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
+{
+    return batch_uniform_verified(c, lanes, d_iv12, 0, d_aad, aad_len, aad_stride, d_ct, d_pt, len, stride, d_tag, d_ok, n_msgs,
+                                  stream);
+}
+
+int agcm_batch_decrypt_verified_uniform_j0(agcm_ctx* c, int lanes, const uint8_t* d_j0, const uint8_t* d_aad, uint64_t aad_len,
+                                           uint64_t aad_stride, const uint8_t* d_ct, uint8_t* d_pt, uint64_t len, uint64_t stride,
+                                           const uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
+{
+    return batch_uniform_verified(c, lanes, d_j0, 1, d_aad, aad_len, aad_stride, d_ct, d_pt, len, stride, d_tag, d_ok, n_msgs,
+                                  stream);
+}
+
+int agcm_batch_decrypt_verified_slots(agcm_ctx* c, int lanes, const uint8_t* d_iv12, const uint8_t* d_aad, const uint32_t* d_aad_len,
+                                      uint64_t aad_len, uint64_t aad_stride, const uint8_t* d_ct, uint8_t* d_pt, const uint32_t* d_len,
+                                      uint64_t stride, uint64_t avg_len_hint, const uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs,
+                                      void* stream)
+{
+    if (!c) return AGCM_E_BAD_ARG;
+    BatchParams p;
+    int rc = slots_params(p, d_iv12, d_aad, d_aad_len, aad_len, aad_stride, d_ct, d_pt, d_len, stride, const_cast<uint8_t*>(d_tag),
+                          d_ok, n_msgs);
+    if (rc) return rc;
+    const bool aligned16 = ((((uintptr_t)d_ct | (uintptr_t)d_pt) | stride) & 15) == 0;
+    return batch_verified(c, lanes, (avg_len_hint ? avg_len_hint : stride / 2) / 4, p, n_msgs, stream, aligned16);
 }
 
 int agcm_batch_derive_j0(agcm_ctx* c, const uint8_t* d_iv, const uint64_t* d_iv_off, uint64_t iv_len, size_t n_msgs,
@@ -1516,6 +1632,31 @@ int agcm_batch_crypt_perkey_uniform(agcm_ctx* c, int mode, int decrypt, const ui
     int rc = uniform_params(p, d_keys, d_iv12, 0, d_aad, aad_len, aad_stride, d_in, d_out, len, stride, d_tag, d_ok, n_msgs);
     if (rc) return rc;
     return perkey_common(c, mode, decrypt, p, n_msgs, perkey_tile_eligible(c, p, n_msgs), (cudaStream_t)stream);
+}
+
+// verify-then-release, per-key: one launch of k_batch_perkey_verified (decrypt == 2 at the launcher)
+int agcm_batch_decrypt_verified_perkey(agcm_ctx* c, int mode, const uint8_t* d_keys, const uint8_t* d_iv12, const uint8_t* d_aad,
+                                       const uint64_t* d_aad_off, const uint8_t* d_ct, const uint64_t* d_in_off, uint8_t* d_pt,
+                                       const uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
+{
+    if (!c || !d_tag || !d_ok) return AGCM_E_BAD_ARG;
+    BatchParams p;
+    int rc = offsets_params(p, d_keys, d_iv12, 0, d_aad, d_aad_off, d_ct, d_in_off, d_pt, const_cast<uint8_t*>(d_tag), d_ok, n_msgs);
+    if (rc) return rc;
+    return perkey_common(c, mode, 2, p, n_msgs, false, (cudaStream_t)stream);
+}
+
+int agcm_batch_decrypt_verified_perkey_uniform(agcm_ctx* c, int mode, const uint8_t* d_keys, const uint8_t* d_iv12,
+                                               const uint8_t* d_aad, uint64_t aad_len, uint64_t aad_stride, const uint8_t* d_ct,
+                                               uint8_t* d_pt, uint64_t len, uint64_t stride, const uint8_t* d_tag, uint8_t* d_ok,
+                                               size_t n_msgs, void* stream)
+{
+    if (!c || !d_tag || !d_ok) return AGCM_E_BAD_ARG;
+    BatchParams p;
+    int rc = uniform_params(p, d_keys, d_iv12, 0, d_aad, aad_len, aad_stride, d_ct, d_pt, len, stride, const_cast<uint8_t*>(d_tag),
+                            d_ok, n_msgs);
+    if (rc) return rc;
+    return perkey_common(c, mode, 2, p, n_msgs, false, (cudaStream_t)stream);
 }
 
 // ---------------------------------------------------------------------------

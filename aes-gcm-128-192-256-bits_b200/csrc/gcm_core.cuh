@@ -563,15 +563,16 @@ AG_HD MsgDesc ag_batch_range(const MsgDesc& w, uint64_t w0, uint64_t w1, uint64_
 }
 
 // Segment `seg` of S equal-WORK segments of message w (the length block and E_K(J0) with segment S-1).
-AG_HD MsgDesc ag_batch_segment(const MsgDesc& w, uint32_t seg, uint32_t S, uint64_t* after)
+// ptw as in ag_batch_range (1: a tag-only pass, where a payload block costs what an AAD block costs).
+AG_HD MsgDesc ag_batch_segment(const MsgDesc& w, uint32_t seg, uint32_t S, uint64_t* after, uint64_t ptw = 4)
 {
     const uint64_t a = (w.aad_len + 15) >> 4, n = (w.len + 15) >> 4;
-    const uint64_t W = a + 4 * n, per = (W + S - 1) / S;
+    const uint64_t W = a + ptw * n, per = (W + S - 1) / S;
     uint64_t w0 = (uint64_t)seg * per, w1 = w0 + per;
     if (w0 > W) w0 = W;
     if (w1 > W) w1 = W;
     if (seg == S - 1) w1 = W + AG_FINISH_WEIGHT;
-    return ag_batch_range(w, w0, w1, after);
+    return ag_batch_range(w, w0, w1, after, ptw);
 }
 
 // Lane t of G over the unified sequence [AAD blocks | CT blocks | length block]
@@ -583,7 +584,9 @@ AG_HD MsgDesc ag_batch_segment(const MsgDesc& w, uint32_t seg, uint32_t S, uint6
 // before row u is processed (one row of software prefetch); a payload block is loaded at the top
 // of its own row and consumed after the AES rounds.
 // SEQ: the lane walks CONSECUTIVE payload blocks (G == 1), so unaligned output can leave granule by granule.
-template <int NR, bool DEC, bool SEQ = false, class CACHE, class TE, class GH>
+// VERIFY: the tag-only flavour of a decrypt (pass 1 of the verify-then-release batch): payload blocks are absorbed
+// like AAD rows -- no keystream, no store -- and only the lane that meets the length block runs AES (E_K(J0)).
+template <int NR, bool DEC, bool SEQ = false, bool VERIFY = false, class CACHE, class TE, class GH>
 AG_HD gf128 ag_batch_lane(const uint32_t* rk, const AesCtrConst& cc, CACHE& cache, const MsgDesc& d, uint32_t t,
                           uint32_t G, TE&& te, GH&& gh_g, uint32_t ej0[4])
 {
@@ -593,6 +596,7 @@ AG_HD gf128 ag_batch_lane(const uint32_t* rk, const AesCtrConst& cc, CACHE& cach
     const uint32_t rows = (mb + G - 1) / G;
     const uint32_t pad = rows * G - mb;   // < G
     const uint32_t atail = (uint32_t)(d.aad_len & 15), tail = (uint32_t)(d.len & 15);
+    const uint32_t a_gh = VERIFY ? a + n : a;   // blocks of the GHASH-only prefix of the unified sequence
     gf128 y = gf_zero();
     uint32_t i = t - pad;                 // wraps while inside the front padding (row 0 only)
     bool have = t >= pad;
@@ -610,20 +614,33 @@ AG_HD gf128 ag_batch_lane(const uint32_t* rk, const AesCtrConst& cc, CACHE& cach
     carry.init();
     const bool wide_st = SEQ && (((uintptr_t)d.out & 15) != 0);
 #endif
-    if (rows && have && i < a) ag_load_block_win<SEQ>(d.aad, i, (i == a - 1 && atail) ? atail : 16u, nxt, win_aad, lc_aad);
+    // block i < a_gh of the GHASH-only prefix: an AAD block or (VERIFY) a payload block
+#define AG_LOAD_GH(i, x)                                                                                                 \
+    if constexpr (VERIFY) {                                                                                              \
+        if ((i) >= a) ag_load_block_win<SEQ>(d.in, (i) - a, ((i) == a + n - 1 && tail) ? tail : 16u, x, win_in, lc_in);    \
+        else ag_load_block_win<SEQ>(d.aad, (i), ((i) == a - 1 && atail) ? atail : 16u, x, win_aad, lc_aad);             \
+    } else ag_load_block_win<SEQ>(d.aad, (i), ((i) == a - 1 && atail) ? atail : 16u, x, win_aad, lc_aad)
+    if (rows && have && i < a_gh) { AG_LOAD_GH(i, nxt); }
     // Rows 0 .. aad_rows-1 hold AAD blocks only (row u spans blocks uG-pad .. uG+G-1-pad): they run in
     // a loop of their own -- prefetch, one table product, one XOR, like k_stream<GHASH_ONLY> -- so
     // that bulk AAD is not dragged through the AES-sized body of the general loop below.
-    const uint32_t aad_rows = (uint32_t)(((uint64_t)a + pad) / G);
+    const uint32_t aad_rows = (uint32_t)(((uint64_t)a_gh + pad) / G);
     uint32_t u = 0;
 #if defined(__CUDA_ARCH__)
     // 16-byte aligned AAD: whole blocks move with one 128-bit load each, TWO rows ahead of the product
     // that consumes them (a GHASH-only row is short: one row of prefetch does not cover a DRAM round trip)
-    if (aad_rows > 2 && ((uintptr_t)d.aad & 15) == 0) {
+    // (VERIFY: any alignment -- the prefix spans two buffers, and ag_load_block_win picks the access per block)
+    if (aad_rows > 2 && (VERIFY || ((uintptr_t)d.aad & 15) == 0)) {
         const uint32_t a_full = (uint32_t)(d.aad_len >> 4);   // blocks below this index are whole
         auto ldq = [&](uint32_t bi) {
             uint4 v = make_uint4(0, 0, 0, 0);
-            if (bi < a_full) {
+            if constexpr (VERIFY) {
+                if (bi < a_gh) {
+                    uint32_t x[4];
+                    AG_LOAD_GH(bi, x);
+                    v = make_uint4(x[0], x[1], x[2], x[3]);
+                }
+            } else if (bi < a_full) {
                 v = *reinterpret_cast<const uint4*>(d.aad + 16 * (uint64_t)bi);
             } else if (bi < a) {
                 uint32_t x[4];
@@ -649,7 +666,7 @@ AG_HD gf128 ag_batch_lane(const uint32_t* rk, const AesCtrConst& cc, CACHE& cach
             }
         }
         // hand over to the general loop with its one-row prefetch: nxt holds row aad_rows' AAD block (if it is one)
-        if (!(u < rows && i < a)) { nxt[0] = nxt[1] = nxt[2] = nxt[3] = 0; }
+        if (!(u < rows && i < a_gh)) { nxt[0] = nxt[1] = nxt[2] = nxt[3] = 0; }
     }
 #endif
     for (; u < aad_rows; ++u) {
@@ -657,7 +674,7 @@ AG_HD gf128 ag_batch_lane(const uint32_t* rk, const AesCtrConst& cc, CACHE& cach
         const uint32_t s0 = nxt[0], s1 = nxt[1], s2 = nxt[2], s3 = nxt[3];
         i += G;
         have = true;
-        if (u + 1 < rows && i < a) ag_load_block_win<SEQ>(d.aad, i, (i == a - 1 && atail) ? atail : 16u, nxt, win_aad, lc_aad);
+        if (u + 1 < rows && i < a_gh) { AG_LOAD_GH(i, nxt); }
         if (u) y = gf_mul_table(y, gh_g);
         if (hv) {
             y.w[0] ^= ag_bswap32(s0);
@@ -672,14 +689,15 @@ AG_HD gf128 ag_batch_lane(const uint32_t* rk, const AesCtrConst& cc, CACHE& cach
         uint32_t s[4] = {nxt[0], nxt[1], nxt[2], nxt[3]};
         i += G;
         have = true;
-        if (u + 1 < rows && i < a) ag_load_block_win<SEQ>(d.aad, i, (i == a - 1 && atail) ? atail : 16u, nxt, win_aad, lc_aad);
+        if (u + 1 < rows && i < a_gh) { AG_LOAD_GH(i, nxt); }
         if (u) y = gf_mul_table(y, gh_g);
         if (!hv) continue;
-        if (ic >= a) {
+        if (ic >= a_gh) {
             // The length block always lands on lane G-1 of the last row.  That lane has no payload
             // block in this row, so it spends the row's AES pass on E_K(J0) (counter 1,
-            // src/aes_icb.vhd:34,99): the tag mask costs no pass of its own.
-            const bool is_len = d.last && (ic == a + n);
+            // src/aes_icb.vhd:34,99): the tag mask costs no pass of its own.  (VERIFY: past the
+            // GHASH-only prefix there is nothing but the length block.)
+            const bool is_len = VERIFY || (d.last && (ic == a + n));
             const uint32_t j = ic - a;
             const uint32_t nv = (j == n - 1 && tail) ? tail : 16u;
             uint32_t x[4] = {0, 0, 0, 0};
@@ -722,5 +740,69 @@ AG_HD gf128 ag_batch_lane(const uint32_t* rk, const AesCtrConst& cc, CACHE& cach
 #if defined(__CUDA_ARCH__)
     if (SEQ) carry.flush();
 #endif
+#undef AG_LOAD_GH
     return y;
+}
+
+// ---- pass 2 of the verify-then-release batch: GCTR gated by the ok flags of pass 1 ---------------
+// Counter mode needs no per-message combine, so the payload blocks of the whole batch are cut FLAT into slots, and
+// neighbouring threads take neighbouring slots -- neighbouring blocks of one record, so that 128-bit accesses
+// coalesce without any staging.  A message whose ok[m] is 0 is skipped: its output range is never written.
+//   uniform / slots: slot s = block s % bpr of message s / bpr (bpr = blocks per record pitch); slot blocks past
+//                    the message's length are skipped;
+//   offsets:         slot s = the bytes [in_off[0] + 16 s, + 16) of the input: it owns every block whose first byte
+//                    lies there (at most one per message; several when messages are shorter than a block).
+constexpr uint32_t AG_GATED_ROWS = 8;   // slots per lane and warp chunk (a warp works 32 x AG_GATED_ROWS slots)
+
+// First message of an offset batch that ends past input byte in_off[0] + 16 s (n_msgs if none): binary search.
+AG_HD uint64_t ag_gated_first_msg(const BatchParams& p, uint64_t s)
+{
+    const uint64_t lo = p.in_off[0] + 16 * s;
+    uint64_t l = 0, h = p.n_msgs;   // answer in [l, h]
+    while (l < h) {
+        const uint64_t mid = l + ((h - l) >> 1);
+        if (p.in_off[mid + 1] <= lo) l = mid + 1;
+        else h = mid;
+    }
+    return l;
+}
+
+// Block j of message m (payload at byte offset off of in / out, len bytes), if ok[m] says so.
+template <int NR, class TE>
+AG_HD void ag_gated_ctr_block(const BatchParams& p, uint64_t m, uint32_t j, uint64_t off, uint64_t len, TE&& te)
+{
+    if (p.ok[m] == 0) return;
+    uint32_t iv[3], j0ctr;
+    ag_batch_iv(p, m, iv, &j0ctr);
+    const uint64_t left = len - 16 * (uint64_t)j;
+    const uint32_t nv = left < 16 ? (uint32_t)left : 16u;
+    uint32_t x[4], ks[4];
+    ag_load_block(p.in + off + 16 * (uint64_t)j, nv, x);
+    aes_rounds_from<1, NR>(p.rk, iv[0] ^ p.rk[0], iv[1] ^ p.rk[1], iv[2] ^ p.rk[2], ag_bswap32(j0ctr + 1u + j) ^ p.rk[3], te,
+                           ks);   // inc32: wraps mod 2^32
+    const uint32_t o[4] = {x[0] ^ ks[0], x[1] ^ ks[1], x[2] ^ ks[2], x[3] ^ ks[3]};
+    ag_store_block(p.out + off + 16 * (uint64_t)j, nv, o);   // nv < 16: exactly the message's last bytes
+}
+
+// Slot s.  m: offsets form only -- a message index at or before the slot's first one (from ag_gated_first_msg or the
+// lane's previous slot); advanced past the messages that end before the slot.
+template <int NR, class TE>
+AG_HD void ag_gated_ctr_slot(const BatchParams& p, uint64_t s, uint64_t bpr, uint64_t& m, TE&& te)
+{
+    if (p.in_off) {
+        const uint64_t lo = p.in_off[0] + 16 * s, hi = lo + 16;
+        while (m < p.n_msgs && p.in_off[m + 1] <= lo) ++m;
+        for (uint64_t q = m; q < p.n_msgs; ++q) {
+            const uint64_t o0 = p.in_off[q], o1 = p.in_off[q + 1];
+            if (o0 >= hi) break;
+            const uint64_t j = lo > o0 ? (lo - o0 + 15) >> 4 : 0;   // the message's block that starts in [lo, hi)
+            const uint64_t b = o0 + 16 * j;
+            if (b < hi && b < o1) ag_gated_ctr_block<NR>(p, q, (uint32_t)j, o0, o1 - o0, te);
+        }
+        return;
+    }
+    const uint64_t mm = ((s | bpr) >> 32) ? s / bpr : (uint64_t)((uint32_t)s / (uint32_t)bpr);
+    const uint32_t j = (uint32_t)(s - mm * bpr);
+    const uint64_t len = p.len_arr ? (p.len_arr[mm] < p.stride ? p.len_arr[mm] : p.stride) : p.len;
+    if (16 * (uint64_t)j < len) ag_gated_ctr_block<NR>(p, mm, j, mm * p.stride, len, te);
 }

@@ -55,7 +55,14 @@ cudaError_t ag_launch_batch_warp(const BatchParams& p, int nr, int decrypt, int 
 // [start, end) slices of the order that hold the long / medium / short messages (ranges6)
 cudaError_t ag_launch_len_sort(const BatchParams& p, uint32_t* hist4096, uint32_t* ranges6, uint32_t* perm, cudaStream_t st);
 cudaError_t ag_launch_batch_cta(const BatchParams& p, int nr, int decrypt, int ncta, int nt, cudaStream_t st);
+// decrypt == 2: verify-then-release (k_batch_perkey_verified: the payload is written only where the tag matched)
 cudaError_t ag_launch_batch_perkey(const BatchParams& p, int nr, int decrypt, int max_cta, cudaStream_t st);
+// verify-then-release batch decrypt under the shared key: pass 1 = the tag-only flavour of k_batch (lane groups of g) or
+// k_batch_warp (writes ok[] only); pass 2 = k_batch_ctr_gated over n_slots flat slots (bpr: blocks per record pitch of
+// the uniform / slots forms; both unused for offsets), which writes only the messages whose ok[m] is 1
+cudaError_t ag_launch_batch_verify(const BatchParams& p, int nr, int g, int ncta, int nt, cudaStream_t st);
+cudaError_t ag_launch_batch_warp_verify(const BatchParams& p, int nr, int ncta, cudaStream_t st);
+cudaError_t ag_launch_batch_ctr_gated(const BatchParams& p, int nr, uint64_t n_slots, uint64_t bpr, int max_cta, cudaStream_t st);
 cudaError_t ag_launch_key_expand(const uint8_t* keys, uint64_t n_keys, int key_bytes, const uint32_t* te0,
                                  uint8_t* round_keys, cudaStream_t st);
 // The key as k_key_setup takes it: raw key bytes, or the Nr+1 pre-expanded stages, as LE words.

@@ -46,11 +46,13 @@ __global__ void k_batch_j0(const KeyDev* kd, const uint8_t* __restrict__ iv, con
 // ===========================================================================
 // Batched messages under one shared key: G lanes per message, persistent grid.
 // Tables: T_a = H^G (row Horner), T_b = H (lane combine).
+// VERIFY: the tag-only pass of the verify-then-release decrypt (k_batch_verify): writes ok[] and nothing else.
 // ===========================================================================
-template <int NR, bool DEC, int G>
-__global__ void __launch_bounds__(AG_STREAM_NT_MAX, 1) k_batch(const __grid_constant__ BatchParams p)
+template <int NR, bool DEC, int G, bool VERIFY>
+// (tid / nt are read in the kernel, whose launch bounds give the compiler their range)
+__device__ __forceinline__ void batch_groups(const BatchParams& p, uint32_t tid, uint32_t nt)
 {
-    const uint32_t tid = threadIdx.x, lane = tid & 31, nt = blockDim.x;
+    const uint32_t lane = tid & 31;
     constexpr int LG = (G == 1) ? 0 : (G == 2) ? 1 : (G == 4) ? 2 : (G == 8) ? 3 : (G == 16) ? 4 : 5;
     if (p.range && p.range[0] >= p.range[1]) return;   // an empty length class: not even the tables
     stage_te0(p.te0);
@@ -102,7 +104,7 @@ __global__ void __launch_bounds__(AG_STREAM_NT_MAX, 1) k_batch(const __grid_cons
                 iv0 = ivw[0]; iv1 = ivw[1]; iv2 = ivw[2];
             }
             cc = aes_ctr_precompute(p.rk, iv0, iv1, iv2, te);
-            y = ag_batch_lane<NR, DEC, G == 1>(p.rk, cc, cache, d, t, (uint32_t)G, te, gh_g, e);
+            y = ag_batch_lane<NR, DEC, G == 1, VERIFY>(p.rk, cc, cache, d, t, (uint32_t)G, te, gh_g, e);
         }
         __syncwarp();
         // R = sum_t Y_t H^(G-t)
@@ -147,6 +149,18 @@ __global__ void __launch_bounds__(AG_STREAM_NT_MAX, 1) k_batch(const __grid_cons
         }
         __syncwarp();
     }
+}
+
+template <int NR, bool DEC, int G>
+__global__ void __launch_bounds__(AG_STREAM_NT_MAX, 1) k_batch(const __grid_constant__ BatchParams p)
+{
+    batch_groups<NR, DEC, G, false>(p, threadIdx.x, blockDim.x);
+}
+
+template <int NR, int G>
+__global__ void __launch_bounds__(AG_STREAM_NT_MAX, 1) k_batch_verify(const __grid_constant__ BatchParams p)
+{
+    batch_groups<NR, true, G, true>(p, threadIdx.x, blockDim.x);
 }
 
 // ===========================================================================
@@ -509,9 +523,10 @@ __global__ void __launch_bounds__(AG_STREAM_NT_MAX, 1) k_batch_cta(const __grid_
 // side), which also scale by H^after and XOR the unit into its message's accumulator; the lane
 // that completes a message's last unit writes (or checks) the tag.  One launch.  Linearity of GHASH
 // in its input, as in src/gcm_ghash.vhd:317-344.  Tables: T_a = H^32, T_b = H.
+// VERIFY: the tag-only pass of the verify-then-release decrypt (k_batch_warp_verify).
 // ===========================================================================
-template <int NR, bool DEC>
-__global__ void __launch_bounds__(AG_STREAM_NT_MAX, 1) k_batch_warp(const __grid_constant__ BatchParams p)
+template <int NR, bool DEC, bool VERIFY>
+__device__ __forceinline__ void batch_warp_units(const BatchParams& p)
 {
     const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     stage_te0(p.te0);
@@ -600,7 +615,7 @@ __global__ void __launch_bounds__(AG_STREAM_NT_MAX, 1) k_batch_warp(const __grid
         AesCtrSeqCache cache;
         cache.key = 0xFFFFFFFFu;
         uint32_t e[4] = {0, 0, 0, 0};
-        const gf128 y = ag_batch_lane<NR, DEC>(p.rk, cc, cache, du, lane, 32u, te, gh, e);
+        const gf128 y = ag_batch_lane<NR, DEC, false, VERIFY>(p.rk, cc, cache, du, lane, 32u, te, gh, e);
         __stcg(p.seg_acc + id * 32 + lane, make_uint4(y.w[0], y.w[1], y.w[2], y.w[3]));
         if (lane == 0) {
             __stcg(p.unit_desc + 2 * id, m + 1);
@@ -642,11 +657,59 @@ __global__ void __launch_bounds__(AG_STREAM_NT_MAX, 1) k_batch_warp(const __grid
             const uint64_t m = u / S;
             uint64_t after = 0;
             MsgDesc d = ag_batch_msg(p, m);
-            if (S > 1) d = ag_batch_segment(d, (uint32_t)(u - m * S), S, &after);
+            if (S > 1) d = ag_batch_segment(d, (uint32_t)(u - m * S), S, &after, VERIFY ? 1 : 4);
             run_unit(u, m, d, after);
         }
     }
     if (n_pend) combine();
+}
+
+template <int NR, bool DEC>
+__global__ void __launch_bounds__(AG_STREAM_NT_MAX, 1) k_batch_warp(const __grid_constant__ BatchParams p)
+{
+    batch_warp_units<NR, DEC, false>(p);
+}
+
+template <int NR>
+__global__ void __launch_bounds__(AG_STREAM_NT_MAX, 1) k_batch_warp_verify(const __grid_constant__ BatchParams p)
+{
+    batch_warp_units<NR, true, true>(p);
+}
+
+// ===========================================================================
+// Pass 2 of the verify-then-release batch decrypt: GCTR over the payload blocks of the whole batch cut flat into
+// slots (ag_gated_ctr_slot), skipping every message whose tag pass 1 rejected -- the batch analogue of
+// k_stream<CTR_ONLY> with its gate.  A warp takes 32 x AG_GATED_ROWS consecutive slots per chunk, lane l the slots
+// l, l + 32, ...; in an offset batch lane 0 finds the chunk's first message by binary search over in_off and every
+// lane walks forward from there.  A slot that falls in a rejected message costs one flag load.
+// ===========================================================================
+// n_slots: slots of the uniform / slots forms (offsets: from in_off, which lives on the device)
+template <int NR>
+__global__ void __launch_bounds__(AG_STREAM_NT_MAX, 1) k_batch_ctr_gated(const __grid_constant__ BatchParams p, uint64_t n_slots,
+                                                                       uint64_t bpr)
+{
+    const uint32_t tid = threadIdx.x, lane = tid & 31;
+    stage_te0(p.te0);
+    __syncthreads();
+    expand_aes_tables();
+    __syncthreads();
+    TeSmem te{ag_smem, lane * 4};
+    constexpr uint64_t CH = 32ull * AG_GATED_ROWS;
+    if (p.in_off) n_slots = (p.in_off[p.n_msgs] - p.in_off[0] + 15) >> 4;
+    const uint64_t n_chunks = (n_slots + CH - 1) / CH;
+    const uint64_t warps = (uint64_t)gridDim.x * (blockDim.x >> 5);
+    for (uint64_t c = (uint64_t)blockIdx.x * (blockDim.x >> 5) + (tid >> 5); c < n_chunks; c += warps) {
+        uint64_t m = 0;
+        if (p.in_off) {
+            if (lane == 0) m = ag_gated_first_msg(p, c * CH);
+            m = __shfl_sync(0xffffffffu, m, 0);
+        }
+#pragma unroll 1
+        for (uint32_t k = 0; k < AG_GATED_ROWS; ++k) {
+            const uint64_t s = c * CH + 32 * k + lane;
+            if (s < n_slots) ag_gated_ctr_slot<NR>(p, s, bpr, m, te);
+        }
+    }
 }
 
 // Tag finish of the split layout: one thread per message XORs its S scaled partials
@@ -803,6 +866,47 @@ static cudaError_t launch_batch_g(const BatchParams& p, int g, int ncta, int nt,
     return cudaErrorInvalidValue;
 }
 
+template <int NR, int G>
+static cudaError_t launch_batch_verify_t(const BatchParams& p, int ncta, int nt, cudaStream_t st)
+{
+    cudaError_t e = cudaFuncSetAttribute(k_batch_verify<NR, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
+    if (e != cudaSuccess) return e;
+    k_batch_verify<NR, G><<<ncta, nt, kSmemBytes, st>>>(p);
+    return cudaGetLastError();
+}
+
+template <int NR>
+static cudaError_t launch_batch_verify_g(const BatchParams& p, int g, int ncta, int nt, cudaStream_t st)
+{
+    switch (g) {
+        case 1: return launch_batch_verify_t<NR, 1>(p, ncta, nt, st);
+        case 2: return launch_batch_verify_t<NR, 2>(p, ncta, nt, st);
+        case 4: return launch_batch_verify_t<NR, 4>(p, ncta, nt, st);
+        case 8: return launch_batch_verify_t<NR, 8>(p, ncta, nt, st);
+        case 16: return launch_batch_verify_t<NR, 16>(p, ncta, nt, st);
+        case 32: return launch_batch_verify_t<NR, 32>(p, ncta, nt, st);
+    }
+    return cudaErrorInvalidValue;
+}
+
+template <int NR>
+static cudaError_t launch_batch_warp_verify_t(const BatchParams& p, int ncta, cudaStream_t st)
+{
+    cudaError_t e = cudaFuncSetAttribute(k_batch_warp_verify<NR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
+    if (e != cudaSuccess) return e;
+    k_batch_warp_verify<NR><<<ncta, AG_STREAM_NT_MAX, kSmemBytes, st>>>(p);
+    return cudaGetLastError();
+}
+
+template <int NR>
+static cudaError_t launch_ctr_gated_t(const BatchParams& p, uint64_t n_slots, uint64_t bpr, int ncta, cudaStream_t st)
+{
+    cudaError_t e = cudaFuncSetAttribute(k_batch_ctr_gated<NR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
+    if (e != cudaSuccess) return e;
+    k_batch_ctr_gated<NR><<<ncta, AG_STREAM_NT_MAX, kSmemBytes, st>>>(p, n_slots, bpr);
+    return cudaGetLastError();
+}
+
 template <int NR, bool DEC>
 static cudaError_t launch_batch_cta_t(const BatchParams& p, int ncta, int nt, cudaStream_t st)
 {
@@ -875,6 +979,40 @@ cudaError_t ag_launch_batch(const BatchParams& p, int nr, int decrypt, int g, in
         case 10: return decrypt ? launch_batch_g<10, true>(p, g, ncta, nt, st) : launch_batch_g<10, false>(p, g, ncta, nt, st);
         case 12: return decrypt ? launch_batch_g<12, true>(p, g, ncta, nt, st) : launch_batch_g<12, false>(p, g, ncta, nt, st);
         case 14: return decrypt ? launch_batch_g<14, true>(p, g, ncta, nt, st) : launch_batch_g<14, false>(p, g, ncta, nt, st);
+    }
+    return cudaErrorInvalidValue;
+}
+
+cudaError_t ag_launch_batch_verify(const BatchParams& p, int nr, int g, int ncta, int nt, cudaStream_t st)
+{
+    switch (nr) {
+        case 10: return launch_batch_verify_g<10>(p, g, ncta, nt, st);
+        case 12: return launch_batch_verify_g<12>(p, g, ncta, nt, st);
+        case 14: return launch_batch_verify_g<14>(p, g, ncta, nt, st);
+    }
+    return cudaErrorInvalidValue;
+}
+
+cudaError_t ag_launch_batch_warp_verify(const BatchParams& p, int nr, int ncta, cudaStream_t st)
+{
+    switch (nr) {
+        case 10: return launch_batch_warp_verify_t<10>(p, ncta, st);
+        case 12: return launch_batch_warp_verify_t<12>(p, ncta, st);
+        case 14: return launch_batch_warp_verify_t<14>(p, ncta, st);
+    }
+    return cudaErrorInvalidValue;
+}
+
+cudaError_t ag_launch_batch_ctr_gated(const BatchParams& p, int nr, uint64_t n_slots, uint64_t bpr, int max_cta, cudaStream_t st)
+{
+    const uint64_t chunks = (n_slots + 32ull * AG_GATED_ROWS - 1) / (32ull * AG_GATED_ROWS), per_cta = AG_STREAM_NT_MAX / 32;
+    const uint64_t need = (chunks + per_cta - 1) / per_cta;
+    const int ncta = p.in_off ? max_cta : (int)(need < (uint64_t)max_cta ? need : (uint64_t)max_cta);
+    if (ncta == 0) return cudaSuccess;
+    switch (nr) {
+        case 10: return launch_ctr_gated_t<10>(p, n_slots, bpr, ncta, st);
+        case 12: return launch_ctr_gated_t<12>(p, n_slots, bpr, ncta, st);
+        case 14: return launch_ctr_gated_t<14>(p, n_slots, bpr, ncta, st);
     }
     return cudaErrorInvalidValue;
 }

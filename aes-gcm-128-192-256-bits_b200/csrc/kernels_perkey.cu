@@ -180,6 +180,58 @@ __global__ void __launch_bounds__(PK_NT, 1) k_batch_perkey(const __grid_constant
     }
 }
 
+
+// Verify-then-release form (agcm_batch_decrypt_verified_perkey*): the set-up and message loop of k_batch_perkey (kept as
+// a kernel of its own, so that k_batch_perkey's code stays as it is); each lane checks its message's tag first and
+// decrypts it only if it matched (ag_perkey_message<.., VERIFY>), ok[m] either way.
+template <int NK, bool WIDE>
+__global__ void __launch_bounds__(PK_NT, 1) k_batch_perkey_verified(const __grid_constant__ BatchParams p)
+{
+    const uint32_t tid = threadIdx.x, lane = tid & 31;
+    // Te0 | Te1 only
+    for (uint32_t idx = tid; idx < 256 * 32; idx += blockDim.x) {
+        const uint32_t x = idx >> 5, l = idx & 31;
+        const uint32_t t = __ldg(p.te0 + x);
+        uint32_t* a = reinterpret_cast<uint32_t*>(ag_smem + SM_AES_A + x * 256 + l * 4);
+        a[0] = t;
+        a[32] = ag_rotl32(t, 8);
+    }
+    __syncthreads();
+    TeSmem2 te{ag_smem, lane * 4};
+    SubWordSmem sb{ag_smem, lane * 4};
+    const uint32_t s0 = (uint32_t)__cvta_generic_to_shared(ag_smem) + PK_GH4;
+    const uint32_t s_al = (s0 + 2047u) & ~2047u;
+    Rows4Smem rows{s_al + (tid >> 3) * 2048u + (tid & 7) * 16u};
+    SubCacheSmem subc{s_al + PK_NT * 256u + tid * 4u};
+
+    // Static stride, or (p.ticket: offset batches in length order) the next 32 messages of the order to whichever warp
+    // is free: a warp that drew long messages must not also own a fixed share of all the later ones.
+    uint64_t g = (uint64_t)blockIdx.x * blockDim.x + tid;
+    for (;; g += (uint64_t)gridDim.x * blockDim.x) {
+        if (p.ticket) {
+            uint32_t t = 0;
+            if (lane == 0) t = atomicAdd(p.ticket, 1u);
+            t = __shfl_sync(0xffffffffu, t, 0);
+            if ((uint64_t)t * 32 >= p.n_msgs) break;
+            g = (uint64_t)t * 32 + lane;
+            if (g >= p.n_msgs) continue;   // the last group may be short (the warp's next draw ends the loop)
+        } else if (g >= p.n_msgs) {
+            break;
+        }
+        const uint64_t m = p.perm ? p.perm[g] : g;   // length order for offset batches: a warp's 32 messages are equally long
+        const MsgDesc d = ag_batch_msg(p, m);
+        uint32_t key[8], iv[3];
+        load_words(p.keys + m * (uint64_t)(4 * NK), NK, key);
+        load_words(p.iv + 12 * m, 3, iv);
+        uint32_t x[4], tg[4];
+        ag_load_block(p.tag + 16 * m, 16, x);   // expected tag in, computed tag out
+        tg[0] = x[0]; tg[1] = x[1]; tg[2] = x[2]; tg[3] = x[3];
+        ag_perkey_message<NK, true, WIDE, true>(key, iv[0], iv[1], iv[2], d, te, sb, rows, subc, tg);
+        p.ok[m] = ((x[0] ^ tg[0]) | (x[1] ^ tg[1]) | (x[2] ^ tg[2]) | (x[3] ^ tg[3])) ? 0 : 1;
+    }
+}
+
+
 // ---------------------------------------------------------------------------
 // The same kernel for FIXED-SIZE records, staged by TMA like k_batch_tile: one lane per message,
 // box {32 bytes x 32 messages} per warp and tile, two tiles per warp, groups of 32 messages by
@@ -359,6 +411,7 @@ cudaError_t ag_launch_batch_perkey_tile(const TileParams& p, int nr, int decrypt
     return cudaErrorInvalidValue;
 }
 
+// decrypt == 2: the verify-then-release form (k_batch_perkey_verified)
 template <int NK>
 static cudaError_t launch_perkey_t(const BatchParams& p, int decrypt, int ncta, cudaStream_t st)
 {
@@ -371,6 +424,7 @@ static cudaError_t launch_perkey_t(const BatchParams& p, int decrypt, int ncta, 
     // realigned wide access when a message may sit at an odd address: batches packed by offsets, or records whose
     // buffers or pitch are not 16-byte aligned
     const bool wide = p.in_off || p.aad_off || ((((uintptr_t)p.in | (uintptr_t)p.out) | p.stride) & 15) != 0;
+    if (decrypt == 2) return wide ? go(k_batch_perkey_verified<NK, true>) : go(k_batch_perkey_verified<NK, false>);
     if (wide) return decrypt ? go(k_batch_perkey<NK, true, true>) : go(k_batch_perkey<NK, false, true>);
     return decrypt ? go(k_batch_perkey<NK, true, false>) : go(k_batch_perkey<NK, false, false>);
 }

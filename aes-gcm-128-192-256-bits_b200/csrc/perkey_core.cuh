@@ -253,7 +253,11 @@ AG_HD gf128 gf_mul_table4(const gf128& x, ROWS&& rows)
 // WIDE: the message may sit at an odd address (batches packed by offsets): whole blocks are then read as realigned
 // 16-byte granules and written through a carried granule, as in the single-lane layout of the shared-key batches
 // (gcm_core.cuh: AgWideWindow, AgLoadCarry, AgStoreCarry) instead of byte by byte.
-template <int NK, bool DEC, bool WIDE = false, class TE, class SB, class ROWS, class SUBC>
+// VERIFY (verify-then-release decrypt, DEC): `tag` holds the EXPECTED tag on entry.  Phase 1 absorbs AAD | CT | length
+// block without a keystream; only if the computed tag matches does phase 2 run GCTR over the same ciphertext (read a
+// second time, mostly from L2) and write the payload.  Returns the computed tag in `tag` either way.  One lane does
+// both phases: a second launch would rebuild the key schedule and the private GHASH table.
+template <int NK, bool DEC, bool WIDE = false, bool VERIFY = false, class TE, class SB, class ROWS, class SUBC>
 AG_HD void ag_perkey_message(const uint32_t* key, uint32_t iv0, uint32_t iv1, uint32_t iv2, const MsgDesc& d, TE&& te,
                              SB&& sb, ROWS&& rows, SUBC&& subc, uint32_t tag[4])
 {
@@ -288,6 +292,11 @@ AG_HD void ag_perkey_message(const uint32_t* key, uint32_t iv0, uint32_t iv1, ui
         const uint32_t nv = left < 16 ? (uint32_t)left : 16u;
         uint32_t x[4], ks[4];
         ag_load_block_win<WIDE>(d.in, (uint32_t)j, nv, x, win_in, lc_in);
+        if constexpr (VERIFY) {
+            y = gf_xor(y, gf_from_le_words(x[0], x[1], x[2], x[3]));
+            y = gf_mul_table4(y, rows);
+            continue;
+        }
         perkey_ctr_block<NK>(st, 2u + (uint32_t)j, te, subc, ks);
         uint32_t o[4] = {x[0] ^ ks[0], x[1] ^ ks[1], x[2] ^ ks[2], x[3] ^ ks[3]};
 #if defined(__CUDA_ARCH__)
@@ -317,6 +326,32 @@ AG_HD void ag_perkey_message(const uint32_t* key, uint32_t iv0, uint32_t iv1, ui
     y.w[2] ^= (uint32_t)(cb >> 32);
     y.w[3] ^= (uint32_t)cb;
     y = gf_mul_table4(y, rows);
+    if constexpr (VERIFY) {
+        const bool match = ((tag[0] ^ ag_bswap32(y.w[0]) ^ e[0]) | (tag[1] ^ ag_bswap32(y.w[1]) ^ e[1]) |
+                            (tag[2] ^ ag_bswap32(y.w[2]) ^ e[2]) | (tag[3] ^ ag_bswap32(y.w[3]) ^ e[3])) == 0;
+        lc_in.j = 0xFFFFFFFFu;
+        for (uint64_t j = 0; match && j < n; ++j) {   // phase 2: release
+            const uint64_t left = d.len - 16 * j;
+            const uint32_t nv = left < 16 ? (uint32_t)left : 16u;
+            uint32_t x[4], ks[4];
+            ag_load_block_win<WIDE>(d.in, (uint32_t)j, nv, x, win_in, lc_in);
+            perkey_ctr_block<NK>(st, 2u + (uint32_t)j, te, subc, ks);
+            const uint32_t o[4] = {x[0] ^ ks[0], x[1] ^ ks[1], x[2] ^ ks[2], x[3] ^ ks[3]};
+#if defined(__CUDA_ARCH__)
+            if (wide_st && nv == 16) {
+                carry.put(d.out + 16 * j, o);
+            } else {
+                if (WIDE) carry.flush();
+                ag_store_block(d.out + 16 * j, nv, o);
+            }
+#else
+            ag_store_block(d.out + 16 * j, nv, o);
+#endif
+        }
+#if defined(__CUDA_ARCH__)
+        if (WIDE) carry.flush();
+#endif
+    }
     tag[0] = ag_bswap32(y.w[0]) ^ e[0];
     tag[1] = ag_bswap32(y.w[1]) ^ e[1];
     tag[2] = ag_bswap32(y.w[2]) ^ e[2];

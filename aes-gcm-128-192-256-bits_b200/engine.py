@@ -376,6 +376,45 @@ class GcmEngine:
                                                 int(aad_len), int(aad_stride), _dptr(data_in), _dptr(data_out), _dptr(lens),
                                                 int(stride), int(avg_len_hint), _dptr(tags), _dptr(ok), n, _stream(stream)))
 
+    # Verify-then-release forms of the batch decrypts above: message i's plaintext is written only if ok[i] == 1, and no
+    # other byte of data_out is touched (failed messages, gaps, slot and record padding).  data_out may be data_in.
+    def batch_decrypt_verified_device(self, ivs, aad, aad_off, data_in, in_off, data_out, tags, ok, lanes=0, avg_len_hint=0,
+                                      stream=None, j0=False):
+        n = in_off.numel() - 1
+        fn = self._L.agcm_batch_decrypt_verified_j0 if j0 else self._L.agcm_batch_decrypt_verified
+        self._ck(fn(self._ctx, int(lanes), int(avg_len_hint), _dptr(ivs), _dptr(aad), _dptr(aad_off), _dptr(data_in),
+                    _dptr(in_off), _dptr(data_out), _dptr(tags), _dptr(ok), n, _stream(stream)))
+
+    def batch_decrypt_verified_uniform_device(self, ivs, aad, aad_len, aad_stride, data_in, data_out, length, stride, tags, ok,
+                                              n_msgs=None, lanes=0, stream=None, j0=False):
+        n = ivs.numel() // (16 if j0 else 12) if n_msgs is None else int(n_msgs)
+        fn = self._L.agcm_batch_decrypt_verified_uniform_j0 if j0 else self._L.agcm_batch_decrypt_verified_uniform
+        self._ck(fn(self._ctx, int(lanes), _dptr(ivs), _dptr(aad), int(aad_len), int(aad_stride), _dptr(data_in),
+                    _dptr(data_out), int(length), int(stride), _dptr(tags), _dptr(ok), n, _stream(stream)))
+
+    def batch_decrypt_verified_slots_device(self, ivs, aad, aad_lens, aad_len, aad_stride, data_in, data_out, lens, stride, tags,
+                                            ok, n_msgs=None, lanes=0, avg_len_hint=0, stream=None):
+        n = lens.numel() if n_msgs is None else int(n_msgs)
+        self._ck(self._L.agcm_batch_decrypt_verified_slots(self._ctx, int(lanes), _dptr(ivs), _dptr(aad), _dptr(aad_lens),
+                                                           int(aad_len), int(aad_stride), _dptr(data_in), _dptr(data_out),
+                                                           _dptr(lens), int(stride), int(avg_len_hint), _dptr(tags), _dptr(ok),
+                                                           n, _stream(stream)))
+
+    def batch_decrypt_verified_perkey_device(self, mode, keys, ivs, aad, aad_off, data_in, in_off, data_out, tags, ok,
+                                             stream=None):
+        n = in_off.numel() - 1
+        self._ck(self._L.agcm_batch_decrypt_verified_perkey(self._ctx, int(mode), _dptr(keys), _dptr(ivs), _dptr(aad),
+                                                            _dptr(aad_off), _dptr(data_in), _dptr(in_off), _dptr(data_out),
+                                                            _dptr(tags), _dptr(ok), n, _stream(stream)))
+
+    def batch_decrypt_verified_perkey_uniform_device(self, mode, keys, ivs, aad, aad_len, aad_stride, data_in, data_out, length,
+                                                     stride, tags, ok, n_msgs=None, stream=None):
+        n = ivs.numel() // 12 if n_msgs is None else int(n_msgs)
+        self._ck(self._L.agcm_batch_decrypt_verified_perkey_uniform(self._ctx, int(mode), _dptr(keys), _dptr(ivs), _dptr(aad),
+                                                                    int(aad_len), int(aad_stride), _dptr(data_in),
+                                                                    _dptr(data_out), int(length), int(stride), _dptr(tags),
+                                                                    _dptr(ok), n, _stream(stream)))
+
     def batch_crypt_perkey_device(self, mode, decrypt, keys, ivs, aad, aad_off, data_in, in_off, data_out, tags, ok=None,
                                   stream=None):
         """One distinct raw key per message (keys: CUDA uint8 [n, mode/8]); BASELINE config 4."""

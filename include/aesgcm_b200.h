@@ -133,6 +133,44 @@ int agcm_stream_decrypt_verified(agcm_ctx* ctx, const uint8_t* h_iv, size_t iv_l
                                  const uint8_t* d_ct, uint8_t* d_pt, uint64_t n_bytes, const uint8_t* d_tag, uint8_t* d_ok,
                                  void* stream);
 
+/* VERIFY-THEN-RELEASE BATCHES: agcm_batch_decrypt_verified* take the arguments of their releasing counterparts
+ * (agcm_batch_crypt, _j0, _uniform, _uniform_j0, _slots, _perkey, _perkey_uniform) minus `decrypt`, and guarantee:
+ *   - d_ok[i] = 1 if message i's tag matches, else 0;
+ *   - the plaintext bytes of message i are written if and only if d_ok[i] == 1;
+ *   - no other byte of d_pt is ever written: not a failed message, not the gaps between offsets, not slot padding past
+ *     d_len[i], not record padding past len.  d_ct == d_pt (exactly aliased) is allowed: a failed message then still
+ *     holds its ciphertext.
+ * Argument checks, error codes and length limits are those of the counterpart; d_tag and d_ok are required
+ * (AGCM_E_BAD_ARG).  n_msgs == 0 returns AGCM_OK and launches nothing.  Shared key: two passes in stream order, no host
+ * round trip -- pass 1 absorbs AAD | CT | length block with no keystream (the lane-group or warp-unit layouts; lanes
+ * chooses this pass only and takes 0, 1, 2, 4, 8, 16, 32 or 4096 + S; 1024, 1024 + S and 2048 are AGCM_E_BAD_ARG),
+ * pass 2 runs GCTR over the payload of the whole batch cut flat into blocks, skipping every message whose flag is 0.
+ * Per key: one launch, each lane checks its message's tag and then, only if it matched, decrypts it (the TMA-staged
+ * per-key kernel has no verified form).  Scratch as for the other batch calls: one such call in flight per context. */
+int agcm_batch_decrypt_verified(agcm_ctx* ctx, int lanes, uint64_t avg_len_hint, const uint8_t* d_iv12, const uint8_t* d_aad,
+                                const uint64_t* d_aad_off, const uint8_t* d_ct, const uint64_t* d_in_off, uint8_t* d_pt,
+                                const uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream);
+int agcm_batch_decrypt_verified_j0(agcm_ctx* ctx, int lanes, uint64_t avg_len_hint, const uint8_t* d_j0, const uint8_t* d_aad,
+                                   const uint64_t* d_aad_off, const uint8_t* d_ct, const uint64_t* d_in_off, uint8_t* d_pt,
+                                   const uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream);
+int agcm_batch_decrypt_verified_uniform(agcm_ctx* ctx, int lanes, const uint8_t* d_iv12, const uint8_t* d_aad, uint64_t aad_len,
+                                        uint64_t aad_stride, const uint8_t* d_ct, uint8_t* d_pt, uint64_t len, uint64_t stride,
+                                        const uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream);
+int agcm_batch_decrypt_verified_uniform_j0(agcm_ctx* ctx, int lanes, const uint8_t* d_j0, const uint8_t* d_aad, uint64_t aad_len,
+                                           uint64_t aad_stride, const uint8_t* d_ct, uint8_t* d_pt, uint64_t len, uint64_t stride,
+                                           const uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream);
+int agcm_batch_decrypt_verified_slots(agcm_ctx* ctx, int lanes, const uint8_t* d_iv12, const uint8_t* d_aad,
+                                      const uint32_t* d_aad_len, uint64_t aad_len, uint64_t aad_stride, const uint8_t* d_ct,
+                                      uint8_t* d_pt, const uint32_t* d_len, uint64_t stride, uint64_t avg_len_hint,
+                                      const uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream);
+int agcm_batch_decrypt_verified_perkey(agcm_ctx* ctx, int mode, const uint8_t* d_keys, const uint8_t* d_iv12, const uint8_t* d_aad,
+                                       const uint64_t* d_aad_off, const uint8_t* d_ct, const uint64_t* d_in_off, uint8_t* d_pt,
+                                       const uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream);
+int agcm_batch_decrypt_verified_perkey_uniform(agcm_ctx* ctx, int mode, const uint8_t* d_keys, const uint8_t* d_iv12,
+                                               const uint8_t* d_aad, uint64_t aad_len, uint64_t aad_stride, const uint8_t* d_ct,
+                                               uint8_t* d_pt, uint64_t len, uint64_t stride, const uint8_t* d_tag, uint8_t* d_ok,
+                                               size_t n_msgs, void* stream);
+
 /* The same for an IV of ANY length (SP 800-38D 7.1: J0 = GHASH_H(IV || 0^(s+64) || [len(IV)]_64),
  * derived on the device; iv_len == 12 is the plain call above).  The reference IP fixes the IV at
  * 96 bits (src/gcm_pkg.vhd:17), so this goes beyond it; pycryptodome's AES.new(nonce=...), which
