@@ -1064,9 +1064,10 @@ static int batch_bind_key(agcm_ctx* c, int decrypt, BatchParams& p, size_t n_msg
     return AGCM_OK;
 }
 
-// verify: pass 1 of the verify-then-release decrypt -- the tag-only flavour of the lane-group / warp-unit kernels
+// decrypt == AG_DECRYPT_VERIFIED: pass 1 of the verify-then-release decrypt -- the tag-only flavour of the lane-group /
+// warp-unit kernels
 static int batch_common(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len, BatchParams& p, size_t n_msgs, void* stream,
-                        bool aligned16 = true, bool verify = false)
+                        bool aligned16 = true)
 {
     if (!c->key_set) return AGCM_E_NO_KEY;
     if (n_msgs == 0) return AGCM_OK;
@@ -1076,7 +1077,7 @@ static int batch_common(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len, B
     const uint64_t real_blocks = !ragged ? ((p.len + 15) >> 4) + (p.aad ? (p.aad_len + 15) >> 4 : 0) : 0;
     int g = pick_lanes(c, lanes, n_msgs, avg_len, aligned16, real_blocks);
     if (g < 0) return AGCM_E_BAD_ARG;
-    if (verify && g >= 1024 && g <= 4096) g = 4097;   // no CTA layout for the tag-only pass: a warp per message
+    if (decrypt == AG_DECRYPT_VERIFIED && g >= 1024 && g <= 4096) g = 4097;   // no CTA layout for the tag-only pass: a warp per message
     if (g > 4096) {
         // a warp per unit (k_batch_warp): balanced static partition for uniform batches, `split`
         // segments per message by ticket for offset batches
@@ -1116,8 +1117,7 @@ static int batch_common(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len, B
             rc = zeroed_ticket(c, 1, (cudaStream_t)stream, p.ticket);
             if (rc) return rc;
         }
-        AG_CUDA(c, verify ? ag_launch_batch_warp_verify(p, c->nr, ncta_w, (cudaStream_t)stream)
-                          : ag_launch_batch_warp(p, c->nr, decrypt, ncta_w, (cudaStream_t)stream));
+        AG_CUDA(c, ag_launch_batch_warp(p, c->nr, decrypt, ncta_w, (cudaStream_t)stream));
         c->launches++;
         return AGCM_OK;
     }
@@ -1162,16 +1162,14 @@ static int batch_common(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len, B
             for (int k = 0; k < 3; ++k) {
                 p.range = ranges + 2 * k;
                 p.ticket = tickets + 1 + k;
-                AG_CUDA(c, verify ? ag_launch_batch_verify(p, c->nr, gs[k], c->ncta, c->nt, st)
-                                  : ag_launch_batch(p, c->nr, decrypt, gs[k], c->ncta, c->nt, st));
+                AG_CUDA(c, ag_launch_batch(p, c->nr, decrypt, gs[k], c->ncta, c->nt, st));
                 c->launches++;
             }
             return AGCM_OK;
         }
         p.ticket = tickets + 1;
     }
-    AG_CUDA(c, verify ? ag_launch_batch_verify(p, c->nr, g, ncta, c->nt, (cudaStream_t)stream)
-                      : ag_launch_batch(p, c->nr, decrypt, g, ncta, c->nt, (cudaStream_t)stream));
+    AG_CUDA(c, ag_launch_batch(p, c->nr, decrypt, g, ncta, c->nt, (cudaStream_t)stream));
     c->launches++;
     return AGCM_OK;
 }
@@ -1185,7 +1183,7 @@ static int batch_verified(agcm_ctx* c, int lanes, uint64_t avg_len, BatchParams&
     if (lanes >= 1024 && lanes <= 4096) return AGCM_E_BAD_ARG;   // the CTA and TMA-staged layouts have no tag-only form
     if (!c->key_set) return AGCM_E_NO_KEY;
     if (n_msgs == 0) return AGCM_OK;
-    int rc = batch_common(c, 1, lanes, avg_len, p, n_msgs, stream, aligned16, true);
+    int rc = batch_common(c, AG_DECRYPT_VERIFIED, lanes, avg_len, p, n_msgs, stream, aligned16);
     if (rc) return rc;
     // pass 2 takes the batch in its own order (flat slots): no sort, no tickets, no AAD
     BatchParams g = p;
@@ -1397,7 +1395,8 @@ static int uniform_params(BatchParams& p, const uint8_t* d_keys, const uint8_t* 
     return AGCM_OK;
 }
 
-static int batch_offsets(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len_hint, const uint8_t* d_iv, int iv_is_j0,
+// The releasing forms take any nonzero `decrypt` as a decrypt; AG_DECRYPT_VERIFIED comes only from the verified forms.
+static int batch_offsets(agcm_ctx* c, bool decrypt, int lanes, uint64_t avg_len_hint, const uint8_t* d_iv, int iv_is_j0,
                          const uint8_t* d_aad, const uint64_t* d_aad_off, const uint8_t* d_in, const uint64_t* d_in_off,
                          uint8_t* d_out, uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
 {
@@ -1408,7 +1407,7 @@ static int batch_offsets(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len_h
     return batch_common(c, decrypt, lanes, avg_len_hint, p, n_msgs, stream);
 }
 
-static int batch_uniform(agcm_ctx* c, int decrypt, int lanes, const uint8_t* d_iv, int iv_is_j0, const uint8_t* d_aad,
+static int batch_uniform(agcm_ctx* c, bool decrypt, int lanes, const uint8_t* d_iv, int iv_is_j0, const uint8_t* d_aad,
                          uint64_t aad_len, uint64_t aad_stride, const uint8_t* d_in, uint8_t* d_out, uint64_t len,
                          uint64_t stride, uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
 {
@@ -1493,8 +1492,8 @@ int agcm_batch_crypt_slots(agcm_ctx* c, int decrypt, int lanes, const uint8_t* d
     if (rc) return rc;
     const bool aligned16 = ((((uintptr_t)d_in | (uintptr_t)d_out) | stride) & 15) == 0;
     if (lanes == 2048 && !tile_slots_eligible(c, lanes, p, n_msgs)) return AGCM_E_BAD_ARG;   // needs 16-byte aligned slots
-    if (n_msgs && tile_slots_eligible(c, lanes, p, n_msgs)) return batch_tile_slots(c, decrypt, p, n_msgs, (cudaStream_t)stream);
-    return batch_common(c, decrypt, lanes, avg_len_hint ? avg_len_hint : stride / 2, p, n_msgs, stream, aligned16);
+    if (n_msgs && tile_slots_eligible(c, lanes, p, n_msgs)) return batch_tile_slots(c, decrypt != 0, p, n_msgs, (cudaStream_t)stream);
+    return batch_common(c, decrypt != 0, lanes, avg_len_hint ? avg_len_hint : stride / 2, p, n_msgs, stream, aligned16);
 }
 
 // ---- verify-then-release batch decrypt: the same checks as the releasing forms, then batch_verified ------------------
@@ -1619,7 +1618,7 @@ int agcm_batch_crypt_perkey(agcm_ctx* c, int mode, int decrypt, const uint8_t* d
     BatchParams p;
     int rc = offsets_params(p, d_keys, d_iv12, 0, d_aad, d_aad_off, d_in, d_in_off, d_out, d_tag, d_ok, n_msgs);
     if (rc) return rc;
-    return perkey_common(c, mode, decrypt, p, n_msgs, false, (cudaStream_t)stream);
+    return perkey_common(c, mode, decrypt != 0, p, n_msgs, false, (cudaStream_t)stream);
 }
 
 int agcm_batch_crypt_perkey_uniform(agcm_ctx* c, int mode, int decrypt, const uint8_t* d_keys, const uint8_t* d_iv12,
@@ -1631,10 +1630,10 @@ int agcm_batch_crypt_perkey_uniform(agcm_ctx* c, int mode, int decrypt, const ui
     BatchParams p;
     int rc = uniform_params(p, d_keys, d_iv12, 0, d_aad, aad_len, aad_stride, d_in, d_out, len, stride, d_tag, d_ok, n_msgs);
     if (rc) return rc;
-    return perkey_common(c, mode, decrypt, p, n_msgs, perkey_tile_eligible(c, p, n_msgs), (cudaStream_t)stream);
+    return perkey_common(c, mode, decrypt != 0, p, n_msgs, perkey_tile_eligible(c, p, n_msgs), (cudaStream_t)stream);
 }
 
-// verify-then-release, per-key: one launch of k_batch_perkey_verified (decrypt == 2 at the launcher)
+// verify-then-release, per-key: one launch of k_batch_perkey_verified
 int agcm_batch_decrypt_verified_perkey(agcm_ctx* c, int mode, const uint8_t* d_keys, const uint8_t* d_iv12, const uint8_t* d_aad,
                                        const uint64_t* d_aad_off, const uint8_t* d_ct, const uint64_t* d_in_off, uint8_t* d_pt,
                                        const uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
@@ -1643,7 +1642,7 @@ int agcm_batch_decrypt_verified_perkey(agcm_ctx* c, int mode, const uint8_t* d_k
     BatchParams p;
     int rc = offsets_params(p, d_keys, d_iv12, 0, d_aad, d_aad_off, d_ct, d_in_off, d_pt, const_cast<uint8_t*>(d_tag), d_ok, n_msgs);
     if (rc) return rc;
-    return perkey_common(c, mode, 2, p, n_msgs, false, (cudaStream_t)stream);
+    return perkey_common(c, mode, AG_DECRYPT_VERIFIED, p, n_msgs, false, (cudaStream_t)stream);
 }
 
 int agcm_batch_decrypt_verified_perkey_uniform(agcm_ctx* c, int mode, const uint8_t* d_keys, const uint8_t* d_iv12,
@@ -1656,7 +1655,7 @@ int agcm_batch_decrypt_verified_perkey_uniform(agcm_ctx* c, int mode, const uint
     int rc = uniform_params(p, d_keys, d_iv12, 0, d_aad, aad_len, aad_stride, d_ct, d_pt, len, stride, const_cast<uint8_t*>(d_tag),
                             d_ok, n_msgs);
     if (rc) return rc;
-    return perkey_common(c, mode, 2, p, n_msgs, false, (cudaStream_t)stream);
+    return perkey_common(c, mode, AG_DECRYPT_VERIFIED, p, n_msgs, false, (cudaStream_t)stream);
 }
 
 // ---------------------------------------------------------------------------

@@ -475,6 +475,27 @@ struct BatchParams {
     uint64_t n_ids;            // unit ids in use: 2 x (n_warps + n_msgs) (balanced) or n_msgs * split (ticket)
 };
 
+// 1 if the computed tag equals the expected one, else 0; every word is compared (no early exit)
+AG_HD uint8_t ag_tag_eq(const uint32_t x[4], const uint32_t tg[4])
+{
+    const uint32_t diff = (x[0] ^ tg[0]) | (x[1] ^ tg[1]) | (x[2] ^ tg[2]) | (x[3] ^ tg[3]);
+    return diff ? 0 : 1;
+}
+
+// The computed tag of batch message m: decrypt, checked against the expected tag into ok[m]; encrypt, stored
+template <bool DEC>
+AG_HD void ag_tag_out(const BatchParams& p, uint64_t m, const uint32_t tg[4])
+{
+    uint8_t* tp = p.tag + 16 * m;
+    if (DEC) {
+        uint32_t x[4];
+        ag_load_block(tp, 16, x);
+        p.ok[m] = ag_tag_eq(x, tg);
+    } else {
+        ag_store_block(tp, 16, tg);
+    }
+}
+
 // One message, or one counter-range segment of it (ag_batch_segment).
 struct MsgDesc {
     const uint8_t* in;

@@ -192,10 +192,7 @@ __device__ void finish_warp(const FinishArgs& p, gf128 s)
         uint32_t t[4] = {ag_bswap32(s.w[0]) ^ e[0], ag_bswap32(s.w[1]) ^ e[1], ag_bswap32(s.w[2]) ^ e[2],
                          ag_bswap32(s.w[3]) ^ e[3]};
         ag_store_block(p.tag_calc, 16, t);
-        if (p.tag_expected && p.ok) {
-            const uint32_t diff = (exp_tag[0] ^ t[0]) | (exp_tag[1] ^ t[1]) | (exp_tag[2] ^ t[2]) | (exp_tag[3] ^ t[3]);
-            *p.ok = diff ? 0 : 1;
-        }
+        if (p.tag_expected && p.ok) *p.ok = ag_tag_eq(exp_tag, t);
     }
 }
 
@@ -407,44 +404,16 @@ __global__ void __launch_bounds__(32) k_xor_parts(const uint8_t* __restrict__ pa
 // ===========================================================================
 size_t ag_smem_bytes() { return kSmemBytes; }
 
-template <int NR, int MODE>
-static cudaError_t launch_stream_t(const StreamParams& p, int ncta, int nt, cudaStream_t st)
+cudaError_t ag_launch_stream(const StreamParams& p, int nr, int mode, int ncta, int nt, cudaStream_t st)
 {
     // 128-bit path when both buffers are 16-byte aligned (GHASH-only has no output buffer)
     const bool aligned = (((uintptr_t)p.in | (uintptr_t)p.out) & 15) == 0;
-    cudaError_t e;
-    if (aligned) {
-        e = cudaFuncSetAttribute(k_stream<NR, MODE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
-        if (e != cudaSuccess) return e;
-        k_stream<NR, MODE, true><<<ncta, nt, kSmemBytes, st>>>(p);
-    } else {
-        e = cudaFuncSetAttribute(k_stream<NR, MODE, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
-        if (e != cudaSuccess) return e;
-        k_stream<NR, MODE, false><<<ncta, nt, kSmemBytes, st>>>(p);
-    }
-    return cudaGetLastError();
-}
-
-template <int NR>
-static cudaError_t launch_stream_nr(const StreamParams& p, int mode, int ncta, int nt, cudaStream_t st)
-{
-    switch (mode) {
-        case AG_MODE_ENC: return launch_stream_t<NR, AG_MODE_ENC>(p, ncta, nt, st);
-        case AG_MODE_DEC: return launch_stream_t<NR, AG_MODE_DEC>(p, ncta, nt, st);
-        case AG_MODE_GHASH_ONLY: return launch_stream_t<NR, AG_MODE_GHASH_ONLY>(p, ncta, nt, st);
-        case AG_MODE_CTR_ONLY: return launch_stream_t<NR, AG_MODE_CTR_ONLY>(p, ncta, nt, st);
-    }
-    return cudaErrorInvalidValue;
-}
-
-cudaError_t ag_launch_stream(const StreamParams& p, int nr, int mode, int ncta, int nt, cudaStream_t st)
-{
-    switch (nr) {
-        case 10: return launch_stream_nr<10>(p, mode, ncta, nt, st);
-        case 12: return launch_stream_nr<12>(p, mode, ncta, nt, st);
-        case 14: return launch_stream_nr<14>(p, mode, ncta, nt, st);
-    }
-    return cudaErrorInvalidValue;
+    return ag_with_nr(nr, [&](auto NR) {
+        return ag_with<AG_MODE_ENC, AG_MODE_DEC, AG_MODE_GHASH_ONLY, AG_MODE_CTR_ONLY>(mode, [&](auto MODE) {
+            return aligned ? ag_launch_smem(k_stream<NR, MODE, true>, ncta, nt, kSmemBytes, st, p)
+                           : ag_launch_smem(k_stream<NR, MODE, false>, ncta, nt, kSmemBytes, st, p);
+        });
+    });
 }
 
 cudaError_t ag_launch_key_expand(const uint8_t* keys, uint64_t n_keys, int key_bytes, const uint32_t* te0,

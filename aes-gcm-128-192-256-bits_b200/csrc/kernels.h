@@ -34,6 +34,12 @@ struct PeerFinishParams {
     volatile uint32_t* status_host;  // same, in mapped pinned host memory (read by the next call without a sync)
 };
 
+// `decrypt` of the batch launchers: 0 encrypt, 1 decrypt, or AG_DECRYPT_VERIFIED, the verify-then-release decrypt of
+// the launchers that have such a form (ag_launch_batch, ag_launch_batch_warp: the tag-only pass, which writes ok[]
+// only; ag_launch_batch_perkey: k_batch_perkey_verified, which writes a message's payload only where its tag matched).
+// The others refuse it with cudaErrorInvalidValue.
+constexpr int AG_DECRYPT_VERIFIED = 2;
+
 cudaError_t ag_launch_stream(const StreamParams& p, int nr, int mode, int ncta, int nt, cudaStream_t st);
 cudaError_t ag_launch_batch(const BatchParams& p, int nr, int decrypt, int g, int ncta, int nt, cudaStream_t st);
 // k_batch_tile: fixed-size records as a 2-D tensor [message][byte], staged by TMA
@@ -55,13 +61,10 @@ cudaError_t ag_launch_batch_warp(const BatchParams& p, int nr, int decrypt, int 
 // [start, end) slices of the order that hold the long / medium / short messages (ranges6)
 cudaError_t ag_launch_len_sort(const BatchParams& p, uint32_t* hist4096, uint32_t* ranges6, uint32_t* perm, cudaStream_t st);
 cudaError_t ag_launch_batch_cta(const BatchParams& p, int nr, int decrypt, int ncta, int nt, cudaStream_t st);
-// decrypt == 2: verify-then-release (k_batch_perkey_verified: the payload is written only where the tag matched)
 cudaError_t ag_launch_batch_perkey(const BatchParams& p, int nr, int decrypt, int max_cta, cudaStream_t st);
-// verify-then-release batch decrypt under the shared key: pass 1 = the tag-only flavour of k_batch (lane groups of g) or
-// k_batch_warp (writes ok[] only); pass 2 = k_batch_ctr_gated over n_slots flat slots (bpr: blocks per record pitch of
-// the uniform / slots forms; both unused for offsets), which writes only the messages whose ok[m] is 1
-cudaError_t ag_launch_batch_verify(const BatchParams& p, int nr, int g, int ncta, int nt, cudaStream_t st);
-cudaError_t ag_launch_batch_warp_verify(const BatchParams& p, int nr, int ncta, cudaStream_t st);
+// verify-then-release batch decrypt under the shared key: pass 1 = ag_launch_batch or ag_launch_batch_warp with
+// AG_DECRYPT_VERIFIED; pass 2 = k_batch_ctr_gated over n_slots flat slots (bpr: blocks per record pitch of the uniform /
+// slots forms; both unused for offsets), which writes only the messages whose ok[m] is 1
 cudaError_t ag_launch_batch_ctr_gated(const BatchParams& p, int nr, uint64_t n_slots, uint64_t bpr, int max_cta, cudaStream_t st);
 cudaError_t ag_launch_key_expand(const uint8_t* keys, uint64_t n_keys, int key_bytes, const uint32_t* te0,
                                  uint8_t* round_keys, cudaStream_t st);

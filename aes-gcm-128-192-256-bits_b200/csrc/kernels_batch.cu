@@ -135,17 +135,9 @@ __device__ __forceinline__ void batch_groups(const BatchParams& p, uint32_t tid,
             }
         }
         if (valid && t == G - 1) {
-            uint32_t tg[4] = {ag_bswap32(r.w[0]) ^ e[0], ag_bswap32(r.w[1]) ^ e[1], ag_bswap32(r.w[2]) ^ e[2],
-                              ag_bswap32(r.w[3]) ^ e[3]};
-            uint8_t* tp = p.tag + 16 * m;
-            if (DEC) {
-                uint32_t x[4];
-                ag_load_block(tp, 16, x);
-                const uint32_t diff = (x[0] ^ tg[0]) | (x[1] ^ tg[1]) | (x[2] ^ tg[2]) | (x[3] ^ tg[3]);
-                p.ok[m] = diff ? 0 : 1;
-            } else {
-                ag_store_block(tp, 16, tg);
-            }
+            const uint32_t tg[4] = {ag_bswap32(r.w[0]) ^ e[0], ag_bswap32(r.w[1]) ^ e[1], ag_bswap32(r.w[2]) ^ e[2],
+                                    ag_bswap32(r.w[3]) ^ e[3]};
+            ag_tag_out<DEC>(p, m, tg);
         }
         __syncwarp();
     }
@@ -371,17 +363,7 @@ __global__ void __launch_bounds__(AG_STREAM_NT_MAX, 1) k_batch_tile(const __grid
             aes_ctr_block_seq<NR>(p.rk, cc, cache, j0ctr, te, e);
             const uint32_t tg[4] = {ag_bswap32(y.w[0]) ^ e[0], ag_bswap32(y.w[1]) ^ e[1], ag_bswap32(y.w[2]) ^ e[2],
                                     ag_bswap32(y.w[3]) ^ e[3]};
-            if (valid) {
-                uint8_t* tp = p.tag + 16 * m;
-                if (DEC) {
-                    uint32_t x[4];
-                    ag_load_block(tp, 16, x);
-                    const uint32_t diff = (x[0] ^ tg[0]) | (x[1] ^ tg[1]) | (x[2] ^ tg[2]) | (x[3] ^ tg[3]);
-                    p.ok[m] = diff ? 0 : 1;
-                } else {
-                    ag_store_block(tp, 16, tg);
-                }
-            }
+            if (valid) ag_tag_out<DEC>(p, m, tg);
         }
         if (issuer) ag_bulk_wait_read0();   // both tiles are free again for the next group
         __syncwarp();
@@ -487,17 +469,9 @@ __global__ void __launch_bounds__(AG_STREAM_NT_MAX, 1) k_batch_cta(const __grid_
                     }
                 }
             } else if (tid == 0) {
-                uint32_t tg[4] = {ag_bswap32(r.w[0]) ^ ej[0], ag_bswap32(r.w[1]) ^ ej[1], ag_bswap32(r.w[2]) ^ ej[2],
-                                  ag_bswap32(r.w[3]) ^ ej[3]};
-                uint8_t* tp = p.tag + 16 * m;
-                if (DEC) {
-                    uint32_t x[4];
-                    ag_load_block(tp, 16, x);
-                    const uint32_t diff = (x[0] ^ tg[0]) | (x[1] ^ tg[1]) | (x[2] ^ tg[2]) | (x[3] ^ tg[3]);
-                    p.ok[m] = diff ? 0 : 1;
-                } else {
-                    ag_store_block(tp, 16, tg);
-                }
+                const uint32_t tg[4] = {ag_bswap32(r.w[0]) ^ ej[0], ag_bswap32(r.w[1]) ^ ej[1], ag_bswap32(r.w[2]) ^ ej[2],
+                                        ag_bswap32(r.w[3]) ^ ej[3]};
+                ag_tag_out<DEC>(p, m, tg);
             }
         }
         __syncthreads();
@@ -560,15 +534,7 @@ __device__ __forceinline__ void batch_warp_units(const BatchParams& p)
         const uint32_t a0 = atomicOr(dst + 0, 0u), a1 = atomicOr(dst + 1, 0u), a2 = atomicOr(dst + 2, 0u), a3 = atomicOr(dst + 3, 0u);
         const uint4 e = __ldcg(reinterpret_cast<const uint4*>(p.msg_ej0 + 4 * m));
         const uint32_t tg[4] = {ag_bswap32(a0) ^ e.x, ag_bswap32(a1) ^ e.y, ag_bswap32(a2) ^ e.z, ag_bswap32(a3) ^ e.w};
-        uint8_t* tp = p.tag + 16 * m;
-        if (DEC) {
-            uint32_t x[4];
-            ag_load_block(tp, 16, x);
-            const uint32_t diff = (x[0] ^ tg[0]) | (x[1] ^ tg[1]) | (x[2] ^ tg[2]) | (x[3] ^ tg[3]);
-            p.ok[m] = diff ? 0 : 1;
-        } else {
-            ag_store_block(tp, 16, tg);
-        }
+        ag_tag_out<DEC>(p, m, tg);
     };
 
     // Combine round: lane i takes pending unit i.  R = sum_t Y_t H^(32-t) by a serial Horner over the
@@ -726,16 +692,8 @@ __global__ void k_batch_split_finish(const __grid_constant__ BatchParams p)
         r[0] ^= q.x; r[1] ^= q.y; r[2] ^= q.z; r[3] ^= q.w;
     }
     const uint4 e = *reinterpret_cast<const uint4*>(p.seg_parts + 4 * (p.n_msgs * S + m));
-    uint32_t tg[4] = {ag_bswap32(r[0]) ^ e.x, ag_bswap32(r[1]) ^ e.y, ag_bswap32(r[2]) ^ e.z, ag_bswap32(r[3]) ^ e.w};
-    uint8_t* tp = p.tag + 16 * m;
-    if (DEC) {
-        uint32_t x[4];
-        ag_load_block(tp, 16, x);
-        const uint32_t diff = (x[0] ^ tg[0]) | (x[1] ^ tg[1]) | (x[2] ^ tg[2]) | (x[3] ^ tg[3]);
-        p.ok[m] = diff ? 0 : 1;
-    } else {
-        ag_store_block(tp, 16, tg);
-    }
+    const uint32_t tg[4] = {ag_bswap32(r[0]) ^ e.x, ag_bswap32(r[1]) ^ e.y, ag_bswap32(r[2]) ^ e.z, ag_bswap32(r[3]) ^ e.w};
+    ag_tag_out<DEC>(p, m, tg);
 }
 
 // ===========================================================================
@@ -843,164 +801,54 @@ cudaError_t ag_launch_len_sort(const BatchParams& p, uint32_t* hist4096, uint32_
 // ===========================================================================
 // launchers (called from capi.cu)
 // ===========================================================================
-template <int NR, bool DEC, int G>
-static cudaError_t launch_batch_t(const BatchParams& p, int ncta, int nt, cudaStream_t st)
-{
-    cudaError_t e = cudaFuncSetAttribute(k_batch<NR, DEC, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
-    if (e != cudaSuccess) return e;
-    k_batch<NR, DEC, G><<<ncta, nt, kSmemBytes, st>>>(p);
-    return cudaGetLastError();
-}
-
-template <int NR, bool DEC>
-static cudaError_t launch_batch_g(const BatchParams& p, int g, int ncta, int nt, cudaStream_t st)
-{
-    switch (g) {
-        case 1: return launch_batch_t<NR, DEC, 1>(p, ncta, nt, st);
-        case 2: return launch_batch_t<NR, DEC, 2>(p, ncta, nt, st);
-        case 4: return launch_batch_t<NR, DEC, 4>(p, ncta, nt, st);
-        case 8: return launch_batch_t<NR, DEC, 8>(p, ncta, nt, st);
-        case 16: return launch_batch_t<NR, DEC, 16>(p, ncta, nt, st);
-        case 32: return launch_batch_t<NR, DEC, 32>(p, ncta, nt, st);
-    }
-    return cudaErrorInvalidValue;
-}
-
-template <int NR, int G>
-static cudaError_t launch_batch_verify_t(const BatchParams& p, int ncta, int nt, cudaStream_t st)
-{
-    cudaError_t e = cudaFuncSetAttribute(k_batch_verify<NR, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
-    if (e != cudaSuccess) return e;
-    k_batch_verify<NR, G><<<ncta, nt, kSmemBytes, st>>>(p);
-    return cudaGetLastError();
-}
-
-template <int NR>
-static cudaError_t launch_batch_verify_g(const BatchParams& p, int g, int ncta, int nt, cudaStream_t st)
-{
-    switch (g) {
-        case 1: return launch_batch_verify_t<NR, 1>(p, ncta, nt, st);
-        case 2: return launch_batch_verify_t<NR, 2>(p, ncta, nt, st);
-        case 4: return launch_batch_verify_t<NR, 4>(p, ncta, nt, st);
-        case 8: return launch_batch_verify_t<NR, 8>(p, ncta, nt, st);
-        case 16: return launch_batch_verify_t<NR, 16>(p, ncta, nt, st);
-        case 32: return launch_batch_verify_t<NR, 32>(p, ncta, nt, st);
-    }
-    return cudaErrorInvalidValue;
-}
-
-template <int NR>
-static cudaError_t launch_batch_warp_verify_t(const BatchParams& p, int ncta, cudaStream_t st)
-{
-    cudaError_t e = cudaFuncSetAttribute(k_batch_warp_verify<NR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
-    if (e != cudaSuccess) return e;
-    k_batch_warp_verify<NR><<<ncta, AG_STREAM_NT_MAX, kSmemBytes, st>>>(p);
-    return cudaGetLastError();
-}
-
-template <int NR>
-static cudaError_t launch_ctr_gated_t(const BatchParams& p, uint64_t n_slots, uint64_t bpr, int ncta, cudaStream_t st)
-{
-    cudaError_t e = cudaFuncSetAttribute(k_batch_ctr_gated<NR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
-    if (e != cudaSuccess) return e;
-    k_batch_ctr_gated<NR><<<ncta, AG_STREAM_NT_MAX, kSmemBytes, st>>>(p, n_slots, bpr);
-    return cudaGetLastError();
-}
-
-template <int NR, bool DEC>
-static cudaError_t launch_batch_cta_t(const BatchParams& p, int ncta, int nt, cudaStream_t st)
-{
-    cudaError_t e = cudaFuncSetAttribute(k_batch_cta<NR, DEC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
-    if (e != cudaSuccess) return e;
-    k_batch_cta<NR, DEC><<<ncta, nt, kSmemBytes, st>>>(p);
-    e = cudaGetLastError();
-    if (e != cudaSuccess || p.split <= 1) return e;
-    k_batch_split_finish<DEC><<<(unsigned)((p.n_msgs + 127) / 128), 128, 0, st>>>(p);
-    return cudaGetLastError();
-}
-
-template <int NR, bool DEC, bool GATHER>
-static cudaError_t launch_batch_tile_t(const TileParams& p, int ncta, cudaStream_t st)
-{
-    cudaError_t e = cudaFuncSetAttribute(k_batch_tile<NR, DEC, GATHER>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTileSmemBytes);
-    if (e != cudaSuccess) return e;
-    k_batch_tile<NR, DEC, GATHER><<<ncta, AG_STREAM_NT_MAX, kTileSmemBytes, st>>>(p);
-    return cudaGetLastError();
-}
-
-template <bool GATHER>
-static cudaError_t launch_batch_tile_g(const TileParams& p, int nr, int decrypt, int ncta, cudaStream_t st)
-{
-    switch (nr) {
-        case 10: return decrypt ? launch_batch_tile_t<10, true, GATHER>(p, ncta, st) : launch_batch_tile_t<10, false, GATHER>(p, ncta, st);
-        case 12: return decrypt ? launch_batch_tile_t<12, true, GATHER>(p, ncta, st) : launch_batch_tile_t<12, false, GATHER>(p, ncta, st);
-        case 14: return decrypt ? launch_batch_tile_t<14, true, GATHER>(p, ncta, st) : launch_batch_tile_t<14, false, GATHER>(p, ncta, st);
-    }
-    return cudaErrorInvalidValue;
-}
-
 cudaError_t ag_launch_batch_tile(const TileParams& p, int nr, int decrypt, int gather, int ncta, cudaStream_t st)
 {
-    return gather ? launch_batch_tile_g<true>(p, nr, decrypt, ncta, st) : launch_batch_tile_g<false>(p, nr, decrypt, ncta, st);
+    return ag_with_nr(nr, [&](auto NR) {
+        return ag_with_dec(decrypt, [&](auto DEC) {
+            return gather ? ag_launch_smem(k_batch_tile<NR, DEC, true>, ncta, AG_STREAM_NT_MAX, kTileSmemBytes, st, p)
+                          : ag_launch_smem(k_batch_tile<NR, DEC, false>, ncta, AG_STREAM_NT_MAX, kTileSmemBytes, st, p);
+        });
+    });
 }
 
-template <int NR, bool DEC>
-static cudaError_t launch_batch_warp_t(const BatchParams& p, int ncta, cudaStream_t st)
-{
-    cudaError_t e = cudaFuncSetAttribute(k_batch_warp<NR, DEC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
-    if (e != cudaSuccess) return e;
-    k_batch_warp<NR, DEC><<<ncta, AG_STREAM_NT_MAX, kSmemBytes, st>>>(p);
-    return cudaGetLastError();
-}
+static cudaError_t launch_batch_warp_verify(const BatchParams& p, int nr, int ncta, cudaStream_t st);
 
 cudaError_t ag_launch_batch_warp(const BatchParams& p, int nr, int decrypt, int ncta, cudaStream_t st)
 {
-    switch (nr) {
-        case 10: return decrypt ? launch_batch_warp_t<10, true>(p, ncta, st) : launch_batch_warp_t<10, false>(p, ncta, st);
-        case 12: return decrypt ? launch_batch_warp_t<12, true>(p, ncta, st) : launch_batch_warp_t<12, false>(p, ncta, st);
-        case 14: return decrypt ? launch_batch_warp_t<14, true>(p, ncta, st) : launch_batch_warp_t<14, false>(p, ncta, st);
-    }
-    return cudaErrorInvalidValue;
+    if (decrypt == AG_DECRYPT_VERIFIED) return launch_batch_warp_verify(p, nr, ncta, st);
+    return ag_with_nr(nr, [&](auto NR) {
+        return ag_with_dec(decrypt, [&](auto DEC) { return ag_launch_smem(k_batch_warp<NR, DEC>, ncta, AG_STREAM_NT_MAX, kSmemBytes, st, p); });
+    });
 }
 
 cudaError_t ag_launch_batch_cta(const BatchParams& p, int nr, int decrypt, int ncta, int nt, cudaStream_t st)
 {
-    switch (nr) {
-        case 10: return decrypt ? launch_batch_cta_t<10, true>(p, ncta, nt, st) : launch_batch_cta_t<10, false>(p, ncta, nt, st);
-        case 12: return decrypt ? launch_batch_cta_t<12, true>(p, ncta, nt, st) : launch_batch_cta_t<12, false>(p, ncta, nt, st);
-        case 14: return decrypt ? launch_batch_cta_t<14, true>(p, ncta, nt, st) : launch_batch_cta_t<14, false>(p, ncta, nt, st);
-    }
-    return cudaErrorInvalidValue;
+    return ag_with_nr(nr, [&](auto NR) {
+        return ag_with_dec(decrypt, [&](auto DEC) {
+            cudaError_t e = ag_launch_smem(k_batch_cta<NR, DEC>, ncta, nt, kSmemBytes, st, p);
+            if (e != cudaSuccess || p.split <= 1) return e;
+            k_batch_split_finish<DEC><<<(unsigned)((p.n_msgs + 127) / 128), 128, 0, st>>>(p);
+            return cudaGetLastError();
+        });
+    });
 }
 
 cudaError_t ag_launch_batch(const BatchParams& p, int nr, int decrypt, int g, int ncta, int nt, cudaStream_t st)
 {
-    switch (nr) {
-        case 10: return decrypt ? launch_batch_g<10, true>(p, g, ncta, nt, st) : launch_batch_g<10, false>(p, g, ncta, nt, st);
-        case 12: return decrypt ? launch_batch_g<12, true>(p, g, ncta, nt, st) : launch_batch_g<12, false>(p, g, ncta, nt, st);
-        case 14: return decrypt ? launch_batch_g<14, true>(p, g, ncta, nt, st) : launch_batch_g<14, false>(p, g, ncta, nt, st);
-    }
-    return cudaErrorInvalidValue;
+    return ag_with_nr(nr, [&](auto NR) {
+        return ag_with<1, 2, 4, 8, 16, 32>(g, [&](auto G) {
+            if (decrypt == AG_DECRYPT_VERIFIED) return ag_launch_smem(k_batch_verify<NR, G>, ncta, nt, kSmemBytes, st, p);
+            return ag_with_dec(decrypt, [&](auto DEC) { return ag_launch_smem(k_batch<NR, DEC, G>, ncta, nt, kSmemBytes, st, p); });
+        });
+    });
 }
 
-cudaError_t ag_launch_batch_verify(const BatchParams& p, int nr, int g, int ncta, int nt, cudaStream_t st)
+// Defined past ag_launch_batch, so that k_batch_warp_verify is instantiated after k_batch_verify (and k_batch_warp before
+// k_batch).  The order of instantiation moves the register allocation of the AES-128 warp-unit kernels; in this order
+// they spill no more than they did with a launcher per kernel.
+static cudaError_t launch_batch_warp_verify(const BatchParams& p, int nr, int ncta, cudaStream_t st)
 {
-    switch (nr) {
-        case 10: return launch_batch_verify_g<10>(p, g, ncta, nt, st);
-        case 12: return launch_batch_verify_g<12>(p, g, ncta, nt, st);
-        case 14: return launch_batch_verify_g<14>(p, g, ncta, nt, st);
-    }
-    return cudaErrorInvalidValue;
-}
-
-cudaError_t ag_launch_batch_warp_verify(const BatchParams& p, int nr, int ncta, cudaStream_t st)
-{
-    switch (nr) {
-        case 10: return launch_batch_warp_verify_t<10>(p, ncta, st);
-        case 12: return launch_batch_warp_verify_t<12>(p, ncta, st);
-        case 14: return launch_batch_warp_verify_t<14>(p, ncta, st);
-    }
-    return cudaErrorInvalidValue;
+    return ag_with_nr(nr, [&](auto NR) { return ag_launch_smem(k_batch_warp_verify<NR>, ncta, AG_STREAM_NT_MAX, kSmemBytes, st, p); });
 }
 
 cudaError_t ag_launch_batch_ctr_gated(const BatchParams& p, int nr, uint64_t n_slots, uint64_t bpr, int max_cta, cudaStream_t st)
@@ -1009,12 +857,9 @@ cudaError_t ag_launch_batch_ctr_gated(const BatchParams& p, int nr, uint64_t n_s
     const uint64_t need = (chunks + per_cta - 1) / per_cta;
     const int ncta = p.in_off ? max_cta : (int)(need < (uint64_t)max_cta ? need : (uint64_t)max_cta);
     if (ncta == 0) return cudaSuccess;
-    switch (nr) {
-        case 10: return launch_ctr_gated_t<10>(p, n_slots, bpr, ncta, st);
-        case 12: return launch_ctr_gated_t<12>(p, n_slots, bpr, ncta, st);
-        case 14: return launch_ctr_gated_t<14>(p, n_slots, bpr, ncta, st);
-    }
-    return cudaErrorInvalidValue;
+    return ag_with_nr(nr, [&](auto NR) {
+        return ag_launch_smem(k_batch_ctr_gated<NR>, ncta, AG_STREAM_NT_MAX, kSmemBytes, st, p, n_slots, bpr);
+    });
 }
 
 cudaError_t ag_launch_batch_j0(const KeyDev* kd, const uint8_t* iv, const uint64_t* iv_off, uint64_t iv_len, uint64_t n,

@@ -127,10 +127,14 @@ __device__ __forceinline__ void load_words(const uint8_t* p, int n_words, uint32
 
 }  // namespace
 
-template <int NK, bool DEC, bool WIDE>
-__global__ void __launch_bounds__(PK_NT, 1) k_batch_perkey(const __grid_constant__ BatchParams p)
+// One lane per message.  VERIFY: the verify-then-release form (k_batch_perkey_verified, agcm_batch_decrypt_verified_perkey*):
+// each lane checks its message's tag first and decrypts it only if it matched (ag_perkey_message<.., VERIFY>), ok[m]
+// either way.
+template <int NK, bool DEC, bool WIDE, bool VERIFY>
+// (tid is read in the kernel, whose launch bounds give the compiler its range)
+__device__ __forceinline__ void batch_perkey(const BatchParams& p, uint32_t tid)
 {
-    const uint32_t tid = threadIdx.x, lane = tid & 31;
+    const uint32_t lane = tid & 31;
     // Te0 | Te1 only
     for (uint32_t idx = tid; idx < 256 * 32; idx += blockDim.x) {
         const uint32_t x = idx >> 5, l = idx & 31;
@@ -166,69 +170,30 @@ __global__ void __launch_bounds__(PK_NT, 1) k_batch_perkey(const __grid_constant
         uint32_t key[8], iv[3];
         load_words(p.keys + m * (uint64_t)(4 * NK), NK, key);
         load_words(p.iv + 12 * m, 3, iv);
-        uint32_t tg[4];
-        ag_perkey_message<NK, DEC, WIDE>(key, iv[0], iv[1], iv[2], d, te, sb, rows, subc, tg);
-        uint8_t* tp = p.tag + 16 * m;
-        if (DEC) {
-            uint32_t x[4];
-            ag_load_block(tp, 16, x);
-            const uint32_t diff = (x[0] ^ tg[0]) | (x[1] ^ tg[1]) | (x[2] ^ tg[2]) | (x[3] ^ tg[3]);
-            p.ok[m] = diff ? 0 : 1;
+        if (VERIFY) {
+            uint32_t x[4], tg[4];
+            ag_load_block(p.tag + 16 * m, 16, x);   // expected tag in, computed tag out
+            tg[0] = x[0]; tg[1] = x[1]; tg[2] = x[2]; tg[3] = x[3];
+            ag_perkey_message<NK, true, WIDE, true>(key, iv[0], iv[1], iv[2], d, te, sb, rows, subc, tg);
+            p.ok[m] = ag_tag_eq(x, tg);
         } else {
-            ag_store_block(tp, 16, tg);
+            uint32_t tg[4];
+            ag_perkey_message<NK, DEC, WIDE>(key, iv[0], iv[1], iv[2], d, te, sb, rows, subc, tg);
+            ag_tag_out<DEC>(p, m, tg);
         }
     }
 }
 
+template <int NK, bool DEC, bool WIDE>
+__global__ void __launch_bounds__(PK_NT, 1) k_batch_perkey(const __grid_constant__ BatchParams p)
+{
+    batch_perkey<NK, DEC, WIDE, false>(p, threadIdx.x);
+}
 
-// Verify-then-release form (agcm_batch_decrypt_verified_perkey*): the set-up and message loop of k_batch_perkey (kept as
-// a kernel of its own, so that k_batch_perkey's code stays as it is); each lane checks its message's tag first and
-// decrypts it only if it matched (ag_perkey_message<.., VERIFY>), ok[m] either way.
 template <int NK, bool WIDE>
 __global__ void __launch_bounds__(PK_NT, 1) k_batch_perkey_verified(const __grid_constant__ BatchParams p)
 {
-    const uint32_t tid = threadIdx.x, lane = tid & 31;
-    // Te0 | Te1 only
-    for (uint32_t idx = tid; idx < 256 * 32; idx += blockDim.x) {
-        const uint32_t x = idx >> 5, l = idx & 31;
-        const uint32_t t = __ldg(p.te0 + x);
-        uint32_t* a = reinterpret_cast<uint32_t*>(ag_smem + SM_AES_A + x * 256 + l * 4);
-        a[0] = t;
-        a[32] = ag_rotl32(t, 8);
-    }
-    __syncthreads();
-    TeSmem2 te{ag_smem, lane * 4};
-    SubWordSmem sb{ag_smem, lane * 4};
-    const uint32_t s0 = (uint32_t)__cvta_generic_to_shared(ag_smem) + PK_GH4;
-    const uint32_t s_al = (s0 + 2047u) & ~2047u;
-    Rows4Smem rows{s_al + (tid >> 3) * 2048u + (tid & 7) * 16u};
-    SubCacheSmem subc{s_al + PK_NT * 256u + tid * 4u};
-
-    // Static stride, or (p.ticket: offset batches in length order) the next 32 messages of the order to whichever warp
-    // is free: a warp that drew long messages must not also own a fixed share of all the later ones.
-    uint64_t g = (uint64_t)blockIdx.x * blockDim.x + tid;
-    for (;; g += (uint64_t)gridDim.x * blockDim.x) {
-        if (p.ticket) {
-            uint32_t t = 0;
-            if (lane == 0) t = atomicAdd(p.ticket, 1u);
-            t = __shfl_sync(0xffffffffu, t, 0);
-            if ((uint64_t)t * 32 >= p.n_msgs) break;
-            g = (uint64_t)t * 32 + lane;
-            if (g >= p.n_msgs) continue;   // the last group may be short (the warp's next draw ends the loop)
-        } else if (g >= p.n_msgs) {
-            break;
-        }
-        const uint64_t m = p.perm ? p.perm[g] : g;   // length order for offset batches: a warp's 32 messages are equally long
-        const MsgDesc d = ag_batch_msg(p, m);
-        uint32_t key[8], iv[3];
-        load_words(p.keys + m * (uint64_t)(4 * NK), NK, key);
-        load_words(p.iv + 12 * m, 3, iv);
-        uint32_t x[4], tg[4];
-        ag_load_block(p.tag + 16 * m, 16, x);   // expected tag in, computed tag out
-        tg[0] = x[0]; tg[1] = x[1]; tg[2] = x[2]; tg[3] = x[3];
-        ag_perkey_message<NK, true, WIDE, true>(key, iv[0], iv[1], iv[2], d, te, sb, rows, subc, tg);
-        p.ok[m] = ((x[0] ^ tg[0]) | (x[1] ^ tg[1]) | (x[2] ^ tg[2]) | (x[3] ^ tg[3])) ? 0 : 1;
-    }
+    batch_perkey<NK, true, WIDE, true>(p, threadIdx.x);
 }
 
 
@@ -365,37 +330,11 @@ __global__ void __launch_bounds__(PKT_NT, 1) k_batch_perkey_tile(const __grid_co
         y = gf_mul_table4(y, rows);
         const uint32_t tg[4] = {ag_bswap32(y.w[0]) ^ e[0], ag_bswap32(y.w[1]) ^ e[1], ag_bswap32(y.w[2]) ^ e[2],
                                 ag_bswap32(y.w[3]) ^ e[3]};
-        if (valid) {
-            uint8_t* tp = p.tag + 16 * m;
-            if (DEC) {
-                uint32_t x[4];
-                ag_load_block(tp, 16, x);
-                const uint32_t diff = (x[0] ^ tg[0]) | (x[1] ^ tg[1]) | (x[2] ^ tg[2]) | (x[3] ^ tg[3]);
-                p.ok[m] = diff ? 0 : 1;
-            } else {
-                ag_store_block(tp, 16, tg);
-            }
-        }
+        if (valid) ag_tag_out<DEC>(p, m, tg);
         if (lane == 0) ag_bulk_wait_read0();
         __syncwarp();
     }
     if (lane == 0) ag_bulk_wait0();
-}
-
-template <int NK>
-static cudaError_t launch_perkey_tile_t(const TileParams& p, int decrypt, int ncta, cudaStream_t st)
-{
-    cudaError_t e;
-    if (decrypt) {
-        e = cudaFuncSetAttribute(k_batch_perkey_tile<NK, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PKT_SMEM);
-        if (e != cudaSuccess) return e;
-        k_batch_perkey_tile<NK, true><<<ncta, PKT_NT, PKT_SMEM, st>>>(p);
-    } else {
-        e = cudaFuncSetAttribute(k_batch_perkey_tile<NK, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PKT_SMEM);
-        if (e != cudaSuccess) return e;
-        k_batch_perkey_tile<NK, false><<<ncta, PKT_NT, PKT_SMEM, st>>>(p);
-    }
-    return cudaGetLastError();
 }
 
 cudaError_t ag_launch_batch_perkey_tile(const TileParams& p, int nr, int decrypt, int max_cta, cudaStream_t st)
@@ -403,41 +342,22 @@ cudaError_t ag_launch_batch_perkey_tile(const TileParams& p, int nr, int decrypt
     const uint64_t groups = (p.b.n_msgs + 31) / 32, per_cta = PKT_NT / 32;
     const uint64_t need = (groups + per_cta - 1) / per_cta;
     const int ncta = (int)(need < (uint64_t)max_cta ? need : (uint64_t)max_cta);
-    switch (nr) {
-        case 10: return launch_perkey_tile_t<4>(p, decrypt, ncta, st);
-        case 12: return launch_perkey_tile_t<6>(p, decrypt, ncta, st);
-        case 14: return launch_perkey_tile_t<8>(p, decrypt, ncta, st);
-    }
-    return cudaErrorInvalidValue;
-}
-
-// decrypt == 2: the verify-then-release form (k_batch_perkey_verified)
-template <int NK>
-static cudaError_t launch_perkey_t(const BatchParams& p, int decrypt, int ncta, cudaStream_t st)
-{
-    auto go = [&](auto kernel) {
-        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PK_SMEM);
-        if (e != cudaSuccess) return e;
-        kernel<<<ncta, PK_NT, PK_SMEM, st>>>(p);
-        return cudaGetLastError();
-    };
-    // realigned wide access when a message may sit at an odd address: batches packed by offsets, or records whose
-    // buffers or pitch are not 16-byte aligned
-    const bool wide = p.in_off || p.aad_off || ((((uintptr_t)p.in | (uintptr_t)p.out) | p.stride) & 15) != 0;
-    if (decrypt == 2) return wide ? go(k_batch_perkey_verified<NK, true>) : go(k_batch_perkey_verified<NK, false>);
-    if (wide) return decrypt ? go(k_batch_perkey<NK, true, true>) : go(k_batch_perkey<NK, false, true>);
-    return decrypt ? go(k_batch_perkey<NK, true, false>) : go(k_batch_perkey<NK, false, false>);
+    return ag_with_nr(nr, [&](auto NR) {
+        return ag_with_dec(decrypt, [&](auto DEC) { return ag_launch_smem(k_batch_perkey_tile<NR - 6, DEC>, ncta, PKT_NT, PKT_SMEM, st, p); });
+    });
 }
 
 cudaError_t ag_launch_batch_perkey(const BatchParams& p, int nr, int decrypt, int max_cta, cudaStream_t st)
 {
     const uint64_t need = (p.n_msgs + PK_NT - 1) / PK_NT;
     const int ncta = (int)(need < (uint64_t)max_cta ? need : (uint64_t)max_cta);
-    switch (nr) {
-        case 10: return launch_perkey_t<4>(p, decrypt, ncta, st);
-        case 12: return launch_perkey_t<6>(p, decrypt, ncta, st);
-        case 14: return launch_perkey_t<8>(p, decrypt, ncta, st);
-    }
-    return cudaErrorInvalidValue;
+    // realigned wide access when a message may sit at an odd address: batches packed by offsets, or records whose
+    // buffers or pitch are not 16-byte aligned
+    const bool wide = p.in_off || p.aad_off || ((((uintptr_t)p.in | (uintptr_t)p.out) | p.stride) & 15) != 0;
+    return ag_with_nr(nr, [&](auto NR) {
+        constexpr int NK = NR - 6;   // key words
+        auto go = [&](auto kernel) { return ag_launch_smem(kernel, ncta, PK_NT, PK_SMEM, st, p); };
+        if (decrypt == AG_DECRYPT_VERIFIED) return wide ? go(k_batch_perkey_verified<NK, true>) : go(k_batch_perkey_verified<NK, false>);
+        return ag_with_dec(decrypt, [&](auto DEC) { return wide ? go(k_batch_perkey<NK, DEC, true>) : go(k_batch_perkey<NK, DEC, false>); });
+    });
 }
-

@@ -1,7 +1,7 @@
 // Shared-memory tables and warp helpers shared by every data-path kernel of the engine
 // (kernels.cu: stream / key / finish / peer; kernels_batch.cu: shared-key batches; kernels_perkey.cu:
-// per-message keys).  Device-only; everything lives in an anonymous namespace, one copy per
-// translation unit.
+// per-message keys), and the launch and dispatch helpers of their launchers.  Everything lives in an
+// anonymous namespace, one copy per translation unit.
 //
 // Shared-memory plan (one persistent 512-thread CTA per SM, 194 KB of the 227 KB):
 //
@@ -25,6 +25,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <type_traits>
 #include "gcm_core.cuh"
 #include "kernels.h"
 
@@ -146,5 +147,41 @@ __device__ gf128 warp_gf_pow(const KeyDev* kd, uint64_t e)
 constexpr size_t kSmemBytes = SM_MISC + 2048;
 // k_batch_tile / k_batch_perkey_tile: one TMA box = 32 messages x 32 bytes
 constexpr uint32_t TILE_BYTES = 1024;
+
+// Launch of a kernel with `smem` bytes of dynamic shared memory (past the 48 KB default, which needs the opt-in)
+template <typename... KArgs, typename... Args>
+cudaError_t ag_launch_smem(void (*kernel)(KArgs...), int ncta, int nt, size_t smem, cudaStream_t st, const Args&... args)
+{
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    kernel<<<ncta, nt, smem, st>>>(args...);
+    return cudaGetLastError();
+}
+
+// A run-time value as a template argument: f(std::integral_constant<int, V>) for the V of Vs equal to v,
+// cudaErrorInvalidValue if there is none
+template <int... Vs, typename F>
+cudaError_t ag_with(int v, F&& f)
+{
+    cudaError_t e = cudaErrorInvalidValue;
+    (void)((v == Vs && ((e = f(std::integral_constant<int, Vs>{})), true)) || ...);
+    return e;
+}
+
+// NR = 10 / 12 / 14 AES rounds
+template <typename F>
+cudaError_t ag_with_nr(int nr, F&& f)
+{
+    return ag_with<10, 12, 14>(nr, f);
+}
+
+// DEC for the kernels that have no tag-only form: AG_DECRYPT_VERIFIED is refused, so that it can never select a
+// decrypt that releases plaintext
+template <typename F>
+cudaError_t ag_with_dec(int decrypt, F&& f)
+{
+    if (decrypt == AG_DECRYPT_VERIFIED) return cudaErrorInvalidValue;
+    return decrypt ? f(std::true_type{}) : f(std::false_type{});
+}
 
 }  // namespace
