@@ -2,67 +2,13 @@
 matches, and no other byte of the output is ever written.
 
 CPU: the tag-only flavour of the shared-key lane code, the gated GCTR slot mapping and the verified per-key message,
-run on the host by tests/host_emul_verified.cu, against the oracle.  GPU: all seven entry points on random batches with about
+run on the host by tests/host_emul.cu, against the oracle.  GPU: all seven entry points on random batches with about
 10 % of the messages corrupted, against the oracle, with the output prefilled by a sentinel."""
-import ctypes
-import os
-import shutil
-import subprocess
-
 import numpy as np
 import pytest
 
-from conftest import ROOT, u8p, u64p
-
-SENTINEL = 0xA5
-CSRC = os.path.join(ROOT, "aes-gcm-128-192-256-bits_b200", "csrc")
-
-
-@pytest.fixture(scope="module")
-def emul_v():
-    """Host build of tests/host_emul_verified.cu, rebuilt when it or any header it includes changes."""
-    nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
-    if not os.path.exists(nvcc):
-        pytest.skip("nvcc not available")
-    bdir = os.path.join(ROOT, "tests", "_build")
-    os.makedirs(bdir, exist_ok=True)
-    so = os.path.join(bdir, "libhost_emul_verified.so")
-    src = os.path.join(ROOT, "tests", "host_emul_verified.cu")
-    deps = [src] + [os.path.join(CSRC, f) for f in ("gcm_core.cuh", "aes_core.cuh", "gf128.cuh", "perkey_core.cuh")]
-    if not os.path.exists(so) or any(os.path.getmtime(d) > os.path.getmtime(so) for d in deps):
-        subprocess.check_call([nvcc, "-w", "-O2", "-std=c++17", "-shared", "-Xcompiler", "-fPIC", "-o", so, src])
-    return ctypes.CDLL(so)
-
-
-def _u32p(a):
-    return a.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32))
-
-
-def _corrupt(rng, n, lens, alens, tags, data, aad, in_off, aad_off, frac=0.1):
-    """Flip a tag bit, a ciphertext byte or an AAD byte of about frac of the messages.  -> expected ok flags."""
-    ok = np.ones(n, np.uint8)
-    for m in rng.choice(n, max(1, int(frac * n)), replace=False):
-        kind = int(rng.integers(0, 3))
-        if kind == 1 and lens[m]:
-            data[int(in_off[m]) + int(rng.integers(0, lens[m]))] ^= 1 << int(rng.integers(0, 8))
-        elif kind == 2 and alens[m]:
-            aad[int(aad_off[m]) + int(rng.integers(0, alens[m]))] ^= 1 << int(rng.integers(0, 8))
-        else:
-            tags[16 * m + int(rng.integers(0, 16))] ^= 1 << int(rng.integers(0, 8))
-        ok[m] = 0
-    return ok
-
-
-def _ragged(rng, n, max_len=300, max_aad=300):
-    lens = rng.integers(0, max_len, n)
-    lens[:6] = [0, 1, 15, 16, 17, 16 * 7 + 3][:min(6, n)]
-    alens = rng.integers(0, max_aad + 1, n)
-    return lens, alens
-
-
-def _rk(oracle, key):
-    rk = np.frombuffer(oracle.key_expand(key.tobytes()), dtype=np.uint8).copy()
-    return rk, len(rk) // 16 - 1
+from batch_cases import (AG_DECRYPT_VERIFIED, SENTINEL, corrupt, emul, emul_batch, emul_ctr_gated,  # noqa: F401 (emul)
+                         expand_key, expect_offsets, offsets_case)
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -70,42 +16,20 @@ def _rk(oracle, key):
 # ---------------------------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("kb", [16, 24, 32])
 @pytest.mark.parametrize("G,S", [(1, 1), (2, 1), (4, 1), (32, 1), (32, 4), (32, 16)])
-def test_emul_offsets_verify_then_gated(emul_v, oracle, kb, G, S):
+def test_emul_offsets_verify_then_gated(emul, oracle, kb, G, S):
+    """The batch starts at byte 5 of its buffer: bytes before in_off[0] stay untouched."""
     rng = np.random.default_rng(1000 + kb + 7 * G + S)
-    n = 40
-    lens, alens = _ragged(rng, n)
-    lens[6] = 16 * 40 + 9
-    base = 5   # the batch starts past byte 0 of the buffer: bytes before in_off[0] stay untouched
-    in_off = (base + np.concatenate([[0], np.cumsum(lens)])).astype(np.uint64)
-    aad_off = np.concatenate([[0], np.cumsum(alens)]).astype(np.uint64)
-    data = rng.integers(0, 256, int(in_off[-1]) + 7, dtype=np.uint8)
-    aad = rng.integers(0, 256, int(aad_off[-1]) + 1, dtype=np.uint8)
-    ivs = rng.integers(0, 256, 12 * n, dtype=np.uint8)
-    key = rng.integers(0, 256, kb, dtype=np.uint8)
-    rk, nr = _rk(oracle, key)
-    pt, tags = oracle.gcm_batch(key, kb, True, ivs, aad, aad_off, data, in_off, decrypt=True)
-    want_ok = _corrupt(rng, n, lens, alens, tags, data, aad, in_off, aad_off)
-    ok = np.full(n, 7, np.uint8)
-    assert emul_v.emul_batch_verify(u8p(rk), nr, G, S, u8p(ivs), 0, u8p(aad), u64p(aad_off), ctypes.c_uint64(0),
-                                    ctypes.c_uint64(0), u8p(data), u64p(in_off), ctypes.c_uint64(0), ctypes.c_uint64(0), None,
-                                    u8p(tags), u8p(ok), ctypes.c_uint64(n)) == 0
+    c = offsets_case(oracle, rng, 40, kb, lens=(16 * 40 + 9,), shift=5)
+    want_ok = corrupt(rng, c)
+    _, _, ok = emul_batch(emul, c, AG_DECRYPT_VERIFIED, G, S)
     assert (ok == want_ok).all(), (kb, G, S)
     for n_warps in (1, 3):
-        out = np.full_like(data, SENTINEL)
-        assert emul_v.emul_batch_ctr_gated(u8p(rk), nr, u8p(ivs), 0, u8p(data), u64p(in_off), ctypes.c_uint64(0),
-                                           ctypes.c_uint64(0), None, u8p(out), u8p(ok), ctypes.c_uint64(n),
-                                           ctypes.c_uint64(n_warps)) == 0
-        want = np.full_like(data, SENTINEL)
-        for m in range(n):
-            a, b = int(in_off[m]), int(in_off[m + 1])
-            if want_ok[m]:
-                want[a:b] = pt[a:b]
-        assert (out == want).all(), (kb, G, S, n_warps)
+        assert (emul_ctr_gated(emul, c, ok, n_warps) == expect_offsets(c, want_ok)).all(), (kb, G, S, n_warps)
 
 
 @pytest.mark.parametrize("kb", [16, 24, 32])
 @pytest.mark.parametrize("form", ["uniform", "slots"])
-def test_emul_fixed_pitch_verify_then_gated(emul_v, oracle, kb, form):
+def test_emul_fixed_pitch_verify_then_gated(emul, oracle, kb, form):
     rng = np.random.default_rng(2000 + kb + len(form))
     n, stride, astride = 37, 16 * 9 + 5, 70
     length = stride - 4 if form == "uniform" else stride
@@ -116,7 +40,7 @@ def test_emul_fixed_pitch_verify_then_gated(emul_v, oracle, kb, form):
     abuf = rng.integers(0, 256, n * astride, dtype=np.uint8)
     ivs = rng.integers(0, 256, 12 * n, dtype=np.uint8)
     key = rng.integers(0, 256, kb, dtype=np.uint8)
-    rk, nr = _rk(oracle, key)
+    rk, nr = expand_key(oracle, key)
     rec = [buf[m * stride:m * stride + int(lens_cl[m])] for m in range(n)]
     in_off = np.concatenate([[0], np.cumsum(lens_cl)]).astype(np.uint64)
     packed = np.concatenate(rec) if in_off[-1] else np.zeros(0, np.uint8)
@@ -127,87 +51,55 @@ def test_emul_fixed_pitch_verify_then_gated(emul_v, oracle, kb, form):
     for m in rng.choice(n, 5, replace=False):
         tags[16 * m + 3] ^= 0x20
         want_ok[m] = 0
-    ok = np.zeros(n, np.uint8)
-    lens32 = lens.astype(np.uint32)
-    len_arr = _u32p(lens32) if form == "slots" else None
-    assert emul_v.emul_batch_verify(u8p(rk), nr, 2, 1, u8p(ivs), 0, u8p(abuf), None, ctypes.c_uint64(alen),
-                                    ctypes.c_uint64(astride), u8p(buf), None, ctypes.c_uint64(length), ctypes.c_uint64(stride),
-                                    len_arr, u8p(tags), u8p(ok), ctypes.c_uint64(n)) == 0
+    c = dict(n=n, rk=rk, nr=nr, ivs=ivs, aad=abuf, aad_len=alen, aad_stride=astride, data=buf, len=length, stride=stride,
+             len_arr=lens.astype(np.uint32) if form == "slots" else None, tags=tags)
+    _, _, ok = emul_batch(emul, c, AG_DECRYPT_VERIFIED, G=2)
     assert (ok == want_ok).all()
-    out = np.full_like(buf, SENTINEL)
-    assert emul_v.emul_batch_ctr_gated(u8p(rk), nr, u8p(ivs), 0, u8p(buf), None, ctypes.c_uint64(length), ctypes.c_uint64(stride),
-                                       len_arr, u8p(out), u8p(ok), ctypes.c_uint64(n), ctypes.c_uint64(2)) == 0
     want = np.full_like(buf, SENTINEL)
     for m in range(n):
         if want_ok[m]:
             want[m * stride:m * stride + int(lens_cl[m])] = pt[int(in_off[m]):int(in_off[m + 1])]
-    assert (out == want).all(), (kb, form)
+    assert (emul_ctr_gated(emul, c, ok, 2) == want).all(), (kb, form)
 
 
-def test_emul_j0_forms(emul_v, oracle):
-    """J0 blocks of IVs that are not 96 bits: the counter starts at inc32(J0), E_K(J0) masks the tag."""
+def test_emul_j0_forms(emul, oracle):
+    """J0 blocks of IVs that are not 96 bits: the counter starts at inc32(J0), E_K(J0) masks the tag.  Through the
+    releasing decrypt and through both passes of the verify-then-release decrypt."""
     rng = np.random.default_rng(31)
-    kb, n = 16, 12
-    key = rng.integers(0, 256, kb, dtype=np.uint8)
-    rk, nr = _rk(oracle, key)
-    lens, alens = _ragged(rng, n, 100, 40)
-    in_off = np.concatenate([[0], np.cumsum(lens)]).astype(np.uint64)
-    aad_off = np.concatenate([[0], np.cumsum(alens)]).astype(np.uint64)
-    data = rng.integers(0, 256, int(in_off[-1]) + 1, dtype=np.uint8)
-    aad = rng.integers(0, 256, int(aad_off[-1]) + 1, dtype=np.uint8)
-    ivs = [rng.integers(0, 256, int(rng.integers(1, 40)), dtype=np.uint8).tobytes() for _ in range(n)]
-    j0 = np.zeros(16 * n, np.uint8)
-    pt = np.zeros_like(data)
-    tags = np.zeros(16 * n, np.uint8)
-    h, _ = oracle.h_ej0(rk.tobytes(), bytes(12))
-    for m in range(n):
-        iv = ivs[m]
+    n = 12
+    c = offsets_case(oracle, rng, n, 16, max_len=100, max_aad=40)
+    ivs = [rng.integers(0, 256, int(k), dtype=np.uint8).tobytes() for k in [1, 12, 16, 39] + list(rng.integers(1, 40, n - 4))]
+    h, _ = oracle.h_ej0(c["rk"].tobytes(), bytes(12))
+    c["ivs"], c["iv_is_j0"] = np.zeros(16 * n, np.uint8), 1
+    for m, iv in enumerate(ivs):
         if len(iv) == 12:
-            j0[16 * m:16 * m + 16] = np.frombuffer(iv + b"\0\0\0\1", np.uint8)
+            c["ivs"][16 * m:16 * m + 16] = np.frombuffer(iv + b"\0\0\0\1", np.uint8)
         else:
             blk = iv + bytes((-len(iv)) % 16) + bytes(8) + (8 * len(iv)).to_bytes(8, "big")
-            j0[16 * m:16 * m + 16] = np.frombuffer(oracle.ghash_absorb(h, blk), np.uint8)
-        a, b = int(in_off[m]), int(in_off[m + 1])
-        p_, t_ = oracle.gcm_crypt_any_iv(key.tobytes(), iv, aad[int(aad_off[m]):int(aad_off[m + 1])].tobytes(),
-                                         data[a:b].tobytes(), decrypt=True)
-        pt[a:b] = np.frombuffer(p_, np.uint8)
-        tags[16 * m:16 * m + 16] = np.frombuffer(t_, np.uint8)
-    tags[16 * 4] ^= 1
-    ok = np.zeros(n, np.uint8)
-    assert emul_v.emul_batch_verify(u8p(rk), nr, 4, 1, u8p(j0), 1, u8p(aad), u64p(aad_off), ctypes.c_uint64(0), ctypes.c_uint64(0),
-                                    u8p(data), u64p(in_off), ctypes.c_uint64(0), ctypes.c_uint64(0), None, u8p(tags), u8p(ok),
-                                    ctypes.c_uint64(n)) == 0
-    assert list(ok) == [1] * 4 + [0] + [1] * 7
-    out = np.full_like(data, SENTINEL)
-    emul_v.emul_batch_ctr_gated(u8p(rk), nr, u8p(j0), 1, u8p(data), u64p(in_off), ctypes.c_uint64(0), ctypes.c_uint64(0), None,
-                                u8p(out), u8p(ok), ctypes.c_uint64(n), ctypes.c_uint64(1))
-    for m in range(n):
-        a, b = int(in_off[m]), int(in_off[m + 1])
-        assert (out[a:b] == (pt[a:b] if ok[m] else SENTINEL)).all(), m
+            c["ivs"][16 * m:16 * m + 16] = np.frombuffer(oracle.ghash_absorb(h, blk), np.uint8)
+        a, b = int(c["in_off"][m]), int(c["in_off"][m + 1])
+        aad = c["aad"][int(c["aad_off"][m]):int(c["aad_off"][m + 1])].tobytes()
+        p_, t_ = oracle.gcm_crypt_any_iv(c["key"].tobytes(), iv, aad, c["data"][a:b].tobytes(), decrypt=True)
+        c["out"][a:b] = np.frombuffer(p_, np.uint8)
+        c["tags"][16 * m:16 * m + 16] = np.frombuffer(t_, np.uint8)
+    c["tags"][16 * 4] ^= 1
+    want_ok = [1] * 4 + [0] + [1] * 7
+    out, _, ok = emul_batch(emul, c, 1, G=4)
+    assert list(ok) == want_ok
+    assert (out == expect_offsets(c, np.ones(n))).all()
+    _, _, ok = emul_batch(emul, c, AG_DECRYPT_VERIFIED, G=4)
+    assert list(ok) == want_ok
+    assert (emul_ctr_gated(emul, c, ok, 1) == expect_offsets(c, ok)).all()
 
 
 @pytest.mark.parametrize("kb", [16, 24, 32])
-def test_emul_perkey_verified(emul_v, oracle, kb):
+def test_emul_perkey_verified(emul, oracle, kb):
     rng = np.random.default_rng(3000 + kb)
-    n = 30
-    lens, alens = _ragged(rng, n)
-    in_off = np.concatenate([[0], np.cumsum(lens)]).astype(np.uint64)
-    aad_off = np.concatenate([[0], np.cumsum(alens)]).astype(np.uint64)
-    data = rng.integers(0, 256, int(in_off[-1]) + 1, dtype=np.uint8)
-    aad = rng.integers(0, 256, int(aad_off[-1]) + 1, dtype=np.uint8)
-    ivs = rng.integers(0, 256, 12 * n, dtype=np.uint8)
-    keys = rng.integers(0, 256, kb * n, dtype=np.uint8)
-    pt, tags = oracle.gcm_batch(keys, kb, False, ivs, aad, aad_off, data[:int(in_off[-1])], in_off, decrypt=True)
-    want_ok = _corrupt(rng, n, lens, alens, tags, data, aad, in_off, aad_off)
-    out = np.full_like(data, SENTINEL)
-    ok = np.zeros(n, np.uint8)
-    assert emul_v.emul_batch_perkey_verified(u8p(keys), kb, u8p(ivs), u8p(aad), u64p(aad_off), u8p(data), u64p(in_off), u8p(out),
-                                             u8p(tags), u8p(ok), ctypes.c_uint64(n)) == 0
+    c = offsets_case(oracle, rng, 30, kb, perkey=True)
+    want_ok = corrupt(rng, c)
+    out, _, ok = emul_batch(emul, c, AG_DECRYPT_VERIFIED)
     assert (ok == want_ok).all()
-    for m in range(n):
-        a, b = int(in_off[m]), int(in_off[m + 1])
-        assert (out[a:b] == (pt[a:b] if want_ok[m] else SENTINEL)).all(), m
-    assert out[-1] == SENTINEL
+    assert (out == expect_offsets(c, want_ok)).all()
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -218,36 +110,14 @@ def _t(a):
     return torch.from_numpy(np.ascontiguousarray(a)).cuda()
 
 
-def _offsets_case(oracle, rng, n, kb, max_len=300, max_aad=300, long_lens=(), shift=0):
-    lens, alens = _ragged(rng, n, max_len, max_aad)
-    for i, L in enumerate(long_lens):
-        lens[6 + i] = L
-    in_off = (shift + np.concatenate([[0], np.cumsum(lens)])).astype(np.uint64)
-    aad_off = np.concatenate([[0], np.cumsum(alens)]).astype(np.uint64)
-    data = rng.integers(0, 256, int(in_off[-1]) + 9, dtype=np.uint8)
-    aad = rng.integers(0, 256, int(aad_off[-1]) + 1, dtype=np.uint8)
-    ivs = rng.integers(0, 256, 12 * n, dtype=np.uint8)
-    key = rng.integers(0, 256, kb, dtype=np.uint8)
-    pt, tags = oracle.gcm_batch(key, kb, True, ivs, aad, aad_off, data, in_off, decrypt=True, threads=8)
-    return dict(lens=lens, alens=alens, in_off=in_off, aad_off=aad_off, data=data, aad=aad, ivs=ivs, key=key, pt=pt, tags=tags)
-
-
-def _expect_offsets(c, ok):
-    want = np.full_like(c["data"], SENTINEL)
-    for m in np.nonzero(ok)[0]:
-        a, b = int(c["in_off"][m]), int(c["in_off"][m + 1])
-        want[a:b] = c["pt"][a:b]
-    return want
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("lanes", [0, 1, 2, 4, 8, 16, 32, 4097, 4100])
 def test_offsets_verified(engine, oracle, lanes):
     import torch
     rng = np.random.default_rng(4000 + lanes)
     for kb in (16, 24, 32):
-        c = _offsets_case(oracle, rng, 1500, kb, shift=int(rng.integers(0, 16)))
-        want_ok = _corrupt(rng, 1500, c["lens"], c["alens"], c["tags"], c["data"], c["aad"], c["in_off"], c["aad_off"])
+        c = offsets_case(oracle, rng, 1500, kb, shift=int(rng.integers(0, 16)))
+        want_ok = corrupt(rng, c)
         engine.set_key(c["key"])
         out = torch.full((c["data"].size,), SENTINEL, dtype=torch.uint8, device="cuda")
         ok = torch.full((1500,), 9, dtype=torch.uint8, device="cuda")
@@ -256,7 +126,7 @@ def test_offsets_verified(engine, oracle, lanes):
                                              avg_len_hint=150)
         torch.cuda.synchronize()
         assert (ok.cpu().numpy() == want_ok).all(), (kb, lanes)
-        assert (out.cpu().numpy() == _expect_offsets(c, want_ok)).all(), (kb, lanes)
+        assert (out.cpu().numpy() == expect_offsets(c, want_ok)).all(), (kb, lanes)
 
 
 @pytest.mark.gpu
@@ -267,15 +137,15 @@ def test_offsets_verified_layouts(engine, engine_small, oracle, shape):
     rng = np.random.default_rng(4100 + len(shape))
     eng = engine_small if shape == "small_grid" else engine
     if shape == "few_long":
-        c = _offsets_case(oracle, rng, 8, 32, long_lens=(3 << 20, (1 << 20) + 5))
+        c = offsets_case(oracle, rng, 8, 32, lens=(3 << 20, (1 << 20) + 5))
     elif shape == "warp_units":
-        c = _offsets_case(oracle, rng, 40, 16, max_len=200 << 10, max_aad=2000)
+        c = offsets_case(oracle, rng, 40, 16, max_len=200 << 10, max_aad=2000)
     elif shape == "classes":
-        c = _offsets_case(oracle, rng, 3000, 24, max_len=1600, long_lens=(40000, 70000, 20000))
+        c = offsets_case(oracle, rng, 3000, 24, max_len=1600, lens=(40000, 70000, 20000))
     else:
-        c = _offsets_case(oracle, rng, 1200, 16, max_len=5000)
+        c = offsets_case(oracle, rng, 1200, 16, max_len=5000)
     n = len(c["lens"])
-    want_ok = _corrupt(rng, n, c["lens"], c["alens"], c["tags"], c["data"], c["aad"], c["in_off"], c["aad_off"])
+    want_ok = corrupt(rng, c)
     eng.set_key(c["key"])
     out = torch.full((c["data"].size,), SENTINEL, dtype=torch.uint8, device="cuda")
     ok = torch.zeros(n, dtype=torch.uint8, device="cuda")
@@ -284,7 +154,7 @@ def test_offsets_verified_layouts(engine, engine_small, oracle, shape):
                                       avg_len_hint=int(np.mean(c["lens"])))
     torch.cuda.synchronize()
     assert (ok.cpu().numpy() == want_ok).all(), shape
-    assert (out.cpu().numpy() == _expect_offsets(c, want_ok)).all(), shape
+    assert (out.cpu().numpy() == expect_offsets(c, want_ok)).all(), shape
 
 
 @pytest.mark.gpu
@@ -293,7 +163,7 @@ def test_offsets_verified_matches_releasing_and_in_place(engine, oracle):
     their ciphertext."""
     import torch
     rng = np.random.default_rng(4200)
-    c = _offsets_case(oracle, rng, 2000, 32, max_len=2000)
+    c = offsets_case(oracle, rng, 2000, 32, max_len=2000)
     engine.set_key(c["key"])
     args = (_t(c["ivs"]), _t(c["aad"]), _t(c["aad_off"].astype(np.int64)))
     d_in, d_off, d_tags = _t(c["data"]), _t(c["in_off"].astype(np.int64)), _t(c["tags"])
@@ -305,7 +175,7 @@ def test_offsets_verified_matches_releasing_and_in_place(engine, oracle):
     engine.batch_decrypt_verified_device(*args, d_in, d_off, out_v, d_tags, ok_v)
     torch.cuda.synchronize()
     assert torch.equal(out_r, out_v) and torch.equal(ok_r, ok_v) and int(ok_v.min()) == 1
-    want_ok = _corrupt(rng, 2000, c["lens"], c["alens"], c["tags"], c["data"], c["aad"], c["in_off"], c["aad_off"])
+    want_ok = corrupt(rng, c)
     buf = _t(c["data"])
     ok = torch.zeros(2000, dtype=torch.uint8, device="cuda")
     engine.batch_decrypt_verified_device(_t(c["ivs"]), _t(c["aad"]), _t(c["aad_off"].astype(np.int64)), buf, d_off, buf,
@@ -315,7 +185,7 @@ def test_offsets_verified_matches_releasing_and_in_place(engine, oracle):
     want = c["data"].copy()
     for m in np.nonzero(want_ok)[0]:
         a, b = int(c["in_off"][m]), int(c["in_off"][m + 1])
-        want[a:b] = c["pt"][a:b]
+        want[a:b] = c["out"][a:b]
     assert (buf.cpu().numpy() == want).all()
 
 
@@ -458,23 +328,16 @@ def test_perkey_verified(engine, oracle, kb):
     import torch
     rng = np.random.default_rng(4600 + kb)
     n = 2500
-    lens, alens = _ragged(rng, n, 1600, 100)
-    in_off = (3 + np.concatenate([[0], np.cumsum(lens)])).astype(np.uint64)
-    aad_off = np.concatenate([[0], np.cumsum(alens)]).astype(np.uint64)
-    data = rng.integers(0, 256, int(in_off[-1]) + 5, dtype=np.uint8)
-    aad = rng.integers(0, 256, int(aad_off[-1]) + 1, dtype=np.uint8)
-    ivs = rng.integers(0, 256, 12 * n, dtype=np.uint8)
-    keys = rng.integers(0, 256, kb * n, dtype=np.uint8)
-    pt, tags = oracle.gcm_batch(keys, kb, False, ivs, aad, aad_off, data, in_off, decrypt=True, threads=8)
-    want_ok = _corrupt(rng, n, lens, alens, tags, data, aad, in_off, aad_off)
-    out = torch.full((data.size,), SENTINEL, dtype=torch.uint8, device="cuda")
+    c = offsets_case(oracle, rng, n, kb, max_len=1600, max_aad=100, shift=3, perkey=True)
+    want_ok = corrupt(rng, c)
+    out = torch.full((c["data"].size,), SENTINEL, dtype=torch.uint8, device="cuda")
     ok = torch.zeros(n, dtype=torch.uint8, device="cuda")
-    engine.batch_decrypt_verified_perkey_device(kb * 8, _t(keys), _t(ivs), _t(aad), _t(aad_off.astype(np.int64)), _t(data),
-                                                _t(in_off.astype(np.int64)), out, _t(tags), ok)
+    engine.batch_decrypt_verified_perkey_device(kb * 8, _t(c["key"]), _t(c["ivs"]), _t(c["aad"]),
+                                                _t(c["aad_off"].astype(np.int64)), _t(c["data"]),
+                                                _t(c["in_off"].astype(np.int64)), out, _t(c["tags"]), ok)
     torch.cuda.synchronize()
     assert (ok.cpu().numpy() == want_ok).all()
-    c = dict(data=data, in_off=in_off, pt=pt)
-    assert (out.cpu().numpy() == _expect_offsets(c, want_ok)).all()
+    assert (out.cpu().numpy() == expect_offsets(c, want_ok)).all()
     # uniform records, in place: failed records keep their ciphertext, padding untouched
     length, stride, alen = 1500, 1504, 16
     m_u = 3000

@@ -6,6 +6,7 @@ import ctypes
 import numpy as np
 import pytest
 
+from batch_cases import emul, emul_batch, expect_offsets, offsets_case  # noqa: F401 (emul: the fixture)
 from conftest import u8p, u64p
 
 
@@ -68,39 +69,27 @@ def test_stream_lanes(emul, oracle, kb):
                 assert part.tobytes() == oracle.ghash_absorb(h, ct), (kb, n, ncta, nt, mode)
 
 
+def _releasing(emul, c, dec, bad, G=1, S=1):
+    """Encrypt or releasing decrypt of case c: every message is written, and a decrypt rejects message `bad` only."""
+    if dec:
+        c["tags"][16 * bad + 5] ^= 0x10
+    out, tags, ok = emul_batch(emul, c, dec, G, S)
+    assert (out == expect_offsets(c, np.ones(c["n"]))).all()
+    if dec:
+        assert list(ok) == [int(m != bad) for m in range(c["n"])]
+    else:
+        assert (tags == c["tags"]).all()
+
+
 @pytest.mark.parametrize("G", [1, 2, 4, 8, 16, 32])
 def test_batch_lanes(emul, oracle, G):
+    """Lane groups of G lanes; the 16*600+3 B message carries the counter byte past 256 blocks."""
     rng = np.random.default_rng(17 + G)
     for kb in (16, 24, 32):
         for dec in (0, 1):
-            nm = 9
-            lens = rng.integers(0, 200, nm)
-            lens[0], lens[1], lens[2], lens[3] = 0, 16, 1500, 16 * 600 + 3   # > 256 blocks: counter byte carries
-            alens = rng.integers(0, 70, nm)
-            alens[2], alens[3] = 0, 16
-            in_off = np.concatenate([[0], np.cumsum(lens)]).astype(np.uint64)
-            aad_off = np.concatenate([[0], np.cumsum(alens)]).astype(np.uint64)
-            data = rng.integers(0, 256, int(in_off[-1]) + 1, dtype=np.uint8)
-            aad = rng.integers(0, 256, int(aad_off[-1]) + 1, dtype=np.uint8)
-            ivs = rng.integers(0, 256, 12 * nm, dtype=np.uint8)
-            key = rng.integers(0, 256, kb, dtype=np.uint8)
-            rk = np.frombuffer(oracle.key_expand(key.tobytes()), dtype=np.uint8).copy()
-            nr = len(rk) // 16 - 1
-            eo, et = oracle.gcm_batch(key, kb, True, ivs, aad, aad_off, data[:int(in_off[-1])], in_off, decrypt=bool(dec))
-            out = np.zeros_like(data)
-            tag = np.zeros(16 * nm, np.uint8)
-            ok = np.zeros(nm, np.uint8)
-            if dec:
-                tag[:] = et
-                tag[16 * 3 + 5] ^= 0x10  # corrupt one tag: must be rejected
-            rc = emul.emul_batch(u8p(rk), nr, dec, G, u8p(ivs), u8p(aad), u64p(aad_off), u8p(data), u64p(in_off), u8p(out),
-                                 u8p(tag), u8p(ok), ctypes.c_uint64(nm))
-            assert rc == 0
-            assert (out[:int(in_off[-1])] == eo).all(), (kb, G, dec)
-            if dec:
-                assert list(ok) == [1, 1, 1, 0, 1, 1, 1, 1, 1]
-            else:
-                assert (tag == et).all(), (kb, G)
+            c = offsets_case(oracle, rng, 9, kb, max_len=200, max_aad=70, lens=(1500, 16 * 600 + 3), aad_lens=(0, 16),
+                             decrypt=bool(dec))
+            _releasing(emul, c, dec, 7, G)
 
 
 @pytest.mark.parametrize("S", [2, 4, 16])
@@ -111,34 +100,9 @@ def test_batch_split_segments(emul, oracle, S):
     rng = np.random.default_rng(300 + S)
     for kb, G in ((16, 4), (32, 32), (24, 8)):
         for dec in (0, 1):
-            nm = 8
-            lens = rng.integers(0, 400, nm)
-            lens[0], lens[1], lens[2], lens[3], lens[4] = 0, 16, 16 * 300 + 5, 33, 16 * S * 7
-            alens = rng.integers(0, 70, nm)
-            alens[2], alens[3] = 0, 16
-            in_off = np.concatenate([[0], np.cumsum(lens)]).astype(np.uint64)
-            aad_off = np.concatenate([[0], np.cumsum(alens)]).astype(np.uint64)
-            data = rng.integers(0, 256, int(in_off[-1]) + 1, dtype=np.uint8)
-            aad = rng.integers(0, 256, int(aad_off[-1]) + 1, dtype=np.uint8)
-            ivs = rng.integers(0, 256, 12 * nm, dtype=np.uint8)
-            key = rng.integers(0, 256, kb, dtype=np.uint8)
-            rk = np.frombuffer(oracle.key_expand(key.tobytes()), dtype=np.uint8).copy()
-            nr = len(rk) // 16 - 1
-            eo, et = oracle.gcm_batch(key, kb, True, ivs, aad, aad_off, data[:int(in_off[-1])], in_off, decrypt=bool(dec))
-            out = np.zeros_like(data)
-            tag = np.zeros(16 * nm, np.uint8)
-            ok = np.zeros(nm, np.uint8)
-            if dec:
-                tag[:] = et
-                tag[16 * 2 + 9] ^= 0x01
-            rc = emul.emul_batch_split(u8p(rk), nr, dec, G, S, u8p(ivs), u8p(aad), u64p(aad_off), u8p(data), u64p(in_off),
-                                       u8p(out), u8p(tag), u8p(ok), ctypes.c_uint64(nm))
-            assert rc == 0
-            assert (out[:int(in_off[-1])] == eo).all(), (kb, G, dec)
-            if dec:
-                assert list(ok) == [1, 1, 0, 1, 1, 1, 1, 1]
-            else:
-                assert (tag == et).all(), (kb, G)
+            c = offsets_case(oracle, rng, 10, kb, max_len=400, max_aad=70, lens=(16 * 300 + 5, 33, 16 * S * 7),
+                             aad_lens=(0, 16), decrypt=bool(dec))
+            _releasing(emul, c, dec, 6, G, S)
 
 
 @pytest.mark.parametrize("n_warps", [1, 3, 7, 40])
@@ -186,32 +150,8 @@ def test_perkey_messages(emul, oracle, kb):
     """One distinct key per message: on-the-fly key schedule + private 4-bit GHASH table."""
     rng = np.random.default_rng(23 + kb)
     for dec in (0, 1):
-        nm = 12
-        lens = rng.integers(0, 300, nm)
-        lens[0], lens[1], lens[2] = 0, 16, 1500
-        alens = rng.integers(0, 80, nm)
-        alens[2], alens[3] = 64, 0
-        in_off = np.concatenate([[0], np.cumsum(lens)]).astype(np.uint64)
-        aad_off = np.concatenate([[0], np.cumsum(alens)]).astype(np.uint64)
-        data = rng.integers(0, 256, int(in_off[-1]) + 1, dtype=np.uint8)
-        aad = rng.integers(0, 256, int(aad_off[-1]) + 1, dtype=np.uint8)
-        ivs = rng.integers(0, 256, 12 * nm, dtype=np.uint8)
-        keys = rng.integers(0, 256, kb * nm, dtype=np.uint8)
-        eo, et = oracle.gcm_batch(keys, kb, False, ivs, aad, aad_off, data[:int(in_off[-1])], in_off, decrypt=bool(dec))
-        out = np.zeros_like(data)
-        tag = np.zeros(16 * nm, np.uint8)
-        ok = np.zeros(nm, np.uint8)
-        if dec:
-            tag[:] = et
-            tag[16 * 4 + 9] ^= 0x01
-        rc = emul.emul_batch_perkey(u8p(keys), kb, dec, u8p(ivs), u8p(aad), u64p(aad_off), u8p(data), u64p(in_off), u8p(out),
-                                    u8p(tag), u8p(ok), ctypes.c_uint64(nm))
-        assert rc == 0
-        assert (out[:int(in_off[-1])] == eo).all(), (kb, dec)
-        if dec:
-            assert list(ok) == [1, 1, 1, 1, 0] + [1] * 7
-        else:
-            assert (tag == et).all(), kb
+        c = offsets_case(oracle, rng, 12, kb, max_aad=80, lens=(1500,), aad_lens=(64, 0), perkey=True, decrypt=bool(dec))
+        _releasing(emul, c, dec, 4)
 
 
 def test_host_pipeline_granule_schedule(emul):
