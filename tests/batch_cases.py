@@ -44,10 +44,49 @@ def expand_key(oracle, key):
     return rk, len(rk) // 16 - 1
 
 
-def offsets_case(oracle, rng, n, kb, max_len=300, max_aad=300, lens=(), aad_lens=(), shift=0, perkey=False, decrypt=True):
+def gf_inv(oracle, h):
+    """h^(2^128 - 2) = h^-1 in GCM's field"""
+    r, e = bytes([0x80]) + bytes(15), (1 << 128) - 2
+    while e:
+        if e & 1:
+            r = oracle.gfmul(r, h)
+        h = oracle.gfmul(h, h)
+        e >>= 1
+    return r
+
+
+def iv_for_j0(oracle, h, h_inv, j0):
+    """The 16-byte IV whose J0 = GHASH_H(IV || 0^64 || [128]_64) = IV.H^2 ^ L.H is `j0`: IV = ((J0.H^-1) ^ L).H^-1."""
+    x = bytearray(oracle.gfmul(j0, h_inv))
+    x[15] ^= 128   # L = [0]_64 || [128]_64
+    iv = oracle.gfmul(bytes(x), h_inv)
+    assert oracle.ghash_absorb(h, iv + bytes(8) + (128).to_bytes(8, "big")) == j0
+    return iv
+
+
+def wrap_at(i):
+    """J0 counter field whose payload block i has counter 0 (inc32 wraps from 0xFFFFFFFF between blocks i-1 and i)"""
+    return (0xFFFFFFFF - i) & 0xFFFFFFFF
+
+
+def top_carry_at(i):
+    """J0 counter field whose payload block i has counter 0x01000000 (carry into the counter's top byte)"""
+    return 0x00FFFFFF - i
+
+
+def byte13_carry_at(i):
+    """J0 counter field whose payload block i has counter 0x00010000 (carry into byte 13 of the counter block)"""
+    return 0x0000FFFF - i
+
+
+def offsets_case(oracle, rng, n, kb, max_len=300, max_aad=300, lens=(), aad_lens=(), shift=0, perkey=False, decrypt=True,
+                 j0_ctrs=None):
     """n messages in the offsets form under one key (perkey: a key per message) with the oracle's output and tags.
     Payload lengths start 0, 1, 15, 16, 17, 16*7+3; messages 6, 7, ... take `lens` and `aad_lens`; the rest are drawn.
-    The batch starts `shift` bytes into `data`, which runs on past its end."""
+    The batch starts `shift` bytes into `data`, which runs on past its end.
+    j0_ctrs: message m gets a 16-byte IV whose J0 ends in the counter field j0_ctrs[m]; past its end, or where it holds
+    None, an IV of a drawn length (12 bytes for some).  c["ivs"] then holds the J0 blocks (iv_is_j0), c["iv_raw"] and
+    c["iv_off"] the IVs and their offsets, and the reference is the oracle's any-IV composition."""
     ln = rng.integers(0, max_len, n)
     ln[:6] = [0, 1, 15, 16, 17, 16 * 7 + 3][:min(6, n)]
     ln[6:6 + len(lens)] = lens
@@ -62,6 +101,29 @@ def offsets_case(oracle, rng, n, kb, max_len=300, max_aad=300, lens=(), aad_lens
     out, tags = oracle.gcm_batch(key, kb, not perkey, ivs, aad, aad_off, data, in_off, decrypt=decrypt, threads=8)
     c = dict(n=n, kb=kb, perkey=perkey, lens=ln, alens=alens, in_off=in_off, aad_off=aad_off, data=data, aad=aad, ivs=ivs,
              key=key, out=out, tags=tags)
+    if j0_ctrs is not None:
+        assert not perkey   # the per-key entry points take 96-bit IVs only
+        h = oracle.aes_encrypt_block(oracle.key_expand(key.tobytes()), bytes(16))
+        h_inv = gf_inv(oracle, h)
+        c["ivs"], c["iv_is_j0"], raw = np.zeros(16 * n, np.uint8), 1, []
+        for m in range(n):
+            c0 = j0_ctrs[m] if m < len(j0_ctrs) else None
+            if c0 is None:
+                iv = rng.integers(0, 256, int(rng.choice([1, 8, 12, 16, 20, 33])), dtype=np.uint8).tobytes()
+                j0 = iv + bytes([0, 0, 0, 1]) if len(iv) == 12 else oracle.ghash_absorb(
+                    h, iv + bytes(-len(iv) % 16) + bytes(8) + (8 * len(iv)).to_bytes(8, "big"))
+            else:
+                j0 = rng.integers(0, 256, 12, dtype=np.uint8).tobytes() + int(c0).to_bytes(4, "big")
+                iv = iv_for_j0(oracle, h, h_inv, j0)
+            c["ivs"][16 * m:16 * m + 16] = np.frombuffer(j0, np.uint8)
+            raw.append(iv)
+            a, b = int(in_off[m]), int(in_off[m + 1])
+            o_, t_ = oracle.gcm_crypt_any_iv(key.tobytes(), iv, aad[int(aad_off[m]):int(aad_off[m + 1])].tobytes(),
+                                             data[a:b].tobytes(), decrypt=decrypt)
+            out[a:b] = np.frombuffer(o_, np.uint8)
+            tags[16 * m:16 * m + 16] = np.frombuffer(t_, np.uint8)
+        c["iv_raw"] = np.frombuffer(b"".join(raw), np.uint8).copy()
+        c["iv_off"] = np.concatenate([[0], np.cumsum([len(iv) for iv in raw])]).astype(np.int64)
     if not perkey:
         c["rk"], c["nr"] = expand_key(oracle, key)
     return c

@@ -8,11 +8,17 @@ case; the reference MODEL calls pycryptodome (tb/gcm_model.py:18), which accepts
 and computes the function OpenSSL computes.  Expected CT/TAG here come from OpenSSL through
 `cryptography` (nonces of 8..128 bytes, its supported range); the published tags of the
 McGrew-Viega test cases 5, 6, 11, 12, 17, 18 (8- and 60-byte IVs) are asserted as anchors.
+
+The counter-edge section (appended after the random vectors, from its own RNG, so the earlier vectors stay as they
+were) chooses J0 and builds the 16-byte IV that GHASHes to it (iv_for_j0, plain Python, independent of the oracle):
+J0 counter fields at the 32-bit wrap, at the carries into the counter's top byte and into byte 13, and 0, with the
+carry or wrap on block 0, block 1, mid-message and in a ragged last block.  Each such vector also stores its `j0`.
 """
 import json
 import os
 import random
 
+from cryptography.hazmat.primitives.ciphers import Cipher, algorithms, modes
 from cryptography.hazmat.primitives.ciphers.aead import AESGCM
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -40,6 +46,73 @@ def case(name, key, iv, aad, pt):
             "ct": out[:-16].hex(), "tag": out[-16:].hex()}
 
 
+def aes_ecb(key, block):
+    e = Cipher(algorithms.AES(key), modes.ECB()).encryptor()
+    return e.update(block) + e.finalize()
+
+
+def gf_mul(x, y):
+    """Product in GCM's GF(2^128) (SP 800-38D 6.3) on blocks read as big-endian integers."""
+    z, v = 0, y
+    for i in range(128):
+        if (x >> (127 - i)) & 1:
+            z ^= v
+        v = (v >> 1) ^ (0xE1 << 120) if v & 1 else v >> 1
+    return z
+
+
+def gf_inv(h):
+    """h^(2^128 - 2) = h^-1"""
+    r, e = 1 << 127, (1 << 128) - 2   # 1 << 127 is the field's one
+    while e:
+        if e & 1:
+            r = gf_mul(r, h)
+        h = gf_mul(h, h)
+        e >>= 1
+    return r
+
+
+def iv_for_j0(key, j0):
+    """The 16-byte IV whose J0 = GHASH_H(IV || 0^64 || [128]_64) = IV.H^2 ^ L.H is `j0`: IV = ((J0.H^-1) ^ L).H^-1."""
+    h = int.from_bytes(aes_ecb(key, bytes(16)), "big")
+    hi, ln = gf_inv(h), 128
+    iv = gf_mul(gf_mul(int.from_bytes(j0, "big"), hi) ^ ln, hi)
+    assert gf_mul(gf_mul(iv, h) ^ ln, h) == int.from_bytes(j0, "big")
+    return iv.to_bytes(16, "big")
+
+
+def inc32(block, k=1):
+    return block[:12] + ((int.from_bytes(block[12:], "big") + k) & 0xFFFFFFFF).to_bytes(4, "big")
+
+
+# J0 counter fields: the 32-bit wrap on payload block 0, block 1 and block 15; the carry into the counter's top byte
+# (0x00FFFFFF -> 0x01000000) on block 0 and block 15; the carry into byte 13 on block 15; an ordinary start
+EDGE_CTRS = (0xFFFFFFFF, 0xFFFFFFFE, 0xFFFFFFF0, 0x00FFFFFF, 0x00FFFFF0, 0x0000FFF0, 0)
+EDGE_LENS = (1, 17, 33, 16 * 40 + 9)
+
+
+def counter_edge_vectors():
+    rnd = random.Random(20261020)
+    rb = lambda n: bytes(rnd.getrandbits(8) for _ in range(n))
+    vectors = []
+    for kb in (16, 24, 32):
+        for c0 in EDGE_CTRS:
+            key = rb(kb)
+            j0 = rb(12) + c0.to_bytes(4, "big")
+            iv = iv_for_j0(key, j0)
+            for n in EDGE_LENS:
+                for al in (0, 20):
+                    pt = rb(n)
+                    v = case("edge-k%d-c%08x-n%d-a%d" % (8 * kb, c0, n, al), key, iv, rb(al), pt)
+                    # the keystream of blocks 0 and 1 is E_K(inc32(J0)), E_K(inc32^2(J0)): the wrap really happens
+                    ks = bytes(a ^ b for a, b in zip(bytes.fromhex(v["ct"]), pt))[:32]
+                    want = aes_ecb(key, inc32(j0, 1)) + aes_ecb(key, inc32(j0, 2))
+                    assert ks == want[:len(ks)], v["name"]
+                    v["j0"] = j0.hex()
+                    vectors.append(v)
+    return vectors
+
+
 def main():
     vectors = []
     for (name, kb, iv), tag in PUBLISHED_TAGS.items():
@@ -53,6 +126,7 @@ def main():
             n = rnd.choice([0, 1, 15, 16, 17, 64, 333, 1500, 4096])
             al = rnd.choice([0, 1, 16, 20, 64, 100])
             vectors.append(case("rand-k%d-iv%d" % (8 * kb, ivl), rb(kb), rb(ivl), rb(al), rb(n)))
+    vectors += counter_edge_vectors()
     with open(os.path.join(HERE, "long_iv_vectors.json"), "w") as f:
         json.dump({"generator": "tests/golden/make_long_iv_golden.py (OpenSSL via cryptography; MV tags asserted)",
                    "vectors": vectors}, f, indent=1)

@@ -378,11 +378,12 @@ int emul_batch_ctr_gated(const uint8_t* rk_bytes, int nr, const uint8_t* iv, int
     });
 }
 
-int emul_batch_balanced(const uint8_t* rk_bytes, int nr, int decrypt, int n_warps, const uint8_t* iv, const uint8_t* aad,
-                        uint64_t aad_len, uint64_t aad_stride, const uint8_t* in, uint8_t* out, uint64_t len, uint64_t stride,
-                        uint8_t* tag, uint8_t* ok, uint64_t n_msgs)
+int emul_batch_balanced(const uint8_t* rk_bytes, int nr, int decrypt, int n_warps, const uint8_t* iv, int iv_is_j0,
+                        const uint8_t* aad, uint64_t aad_len, uint64_t aad_stride, const uint8_t* in, uint8_t* out, uint64_t len,
+                        uint64_t stride, uint8_t* tag, uint8_t* ok, uint64_t n_msgs)
 {
     BatchParams p = batch_params(rk_bytes, nr, iv, in, out, tag, ok, n_msgs);
+    p.iv_is_j0 = iv_is_j0 ? 1u : 0u;
     p.aad = aad_len ? aad : nullptr;
     p.aad_len = aad_len;
     p.aad_stride = aad_stride;
@@ -411,6 +412,56 @@ int emul_batch_perkey(const uint8_t* keys, int key_bytes, int decrypt, const uin
             perkey_nk<KB / 4, D != 0, D == AG_DECRYPT_VERIFIED>(p);
             return 0;
         });
+    });
+}
+
+// Keystream blocks of the counters ctr0, ctr0 + stride, ... (n_blocks of them, mod 2^32) under the 12 IV bytes, as one
+// lane makes them with one counter cache: which = 0 the sequential cache of the batch lanes (AesCtrSeqCache), 1 the
+// stream kernel's (AesCtrCache).  The kernels' strides never move the counter's top byte alone; a stride of 2^24 does.
+int emul_ctr_cached(const uint8_t* rk_bytes, int nr, const uint8_t iv12[12], uint32_t ctr0, uint32_t stride, uint64_t n_blocks,
+                    int which, uint8_t* out)
+{
+    uint32_t rk[60], iv[3];
+    memcpy(rk, rk_bytes, (size_t)16 * (nr + 1));
+    le_words(iv12, 3, iv);
+    const TeHost te{tables().te0};
+    const AesCtrConst cc = aes_ctr_precompute(rk, iv[0], iv[1], iv[2], te);
+    AesCtrSeqCache seq;
+    seq.key = 0xFFFFFFFFu;
+    AesCtrCache str;
+    str.key = 0x00FFFF00u;
+    return with<10, 12, 14>(nr, [&](auto NR) {
+        for (uint64_t b = 0; b < n_blocks; ++b) {
+            uint32_t ks[4];
+            const uint32_t ctr = ctr0 + (uint32_t)b * stride;
+            if (which) aes_ctr_block_cached<NR>(rk, cc, str, ctr, te, ks);
+            else aes_ctr_block_seq<NR>(rk, cc, seq, ctr, te, ks);
+            ag_store_block(out + 16 * b, 16, ks);
+        }
+        return 0;
+    });
+}
+
+// The per-key kernels' counter mode (perkey_ctr_init + perkey_ctr_block: the key schedule on the fly, their own copy of the
+// sequential cache) from the raw key, over the counters ctr0, ctr0 + stride, ... as in emul_ctr_cached
+int emul_perkey_ctr(const uint8_t* key, int key_bytes, const uint8_t iv12[12], uint32_t ctr0, uint32_t stride,
+                    uint64_t n_blocks, uint8_t* out)
+{
+    const TeHost te{tables().te0};
+    const SubWordHost sb{tables().sbox};
+    uint32_t kw[8], iv[3];
+    le_words(key, key_bytes / 4, kw);
+    le_words(iv12, 3, iv);
+    return with<16, 24, 32>(key_bytes, [&](auto KB) {
+        PerKeyCtr<KB / 4> st;
+        SubCacheHost subc;
+        perkey_ctr_init<KB / 4>(kw, iv[0], iv[1], iv[2], te, sb, subc, st);
+        for (uint64_t b = 0; b < n_blocks; ++b) {
+            uint32_t ks[4];
+            perkey_ctr_block(st, ctr0 + (uint32_t)b * stride, te, subc, ks);
+            ag_store_block(out + 16 * b, 16, ks);
+        }
+        return 0;
     });
 }
 

@@ -7,8 +7,8 @@ run on the host by tests/host_emul.cu, against the oracle.  GPU: all seven entry
 import numpy as np
 import pytest
 
-from batch_cases import (AG_DECRYPT_VERIFIED, SENTINEL, corrupt, emul, emul_batch, emul_ctr_gated,  # noqa: F401 (emul)
-                         expand_key, expect_offsets, offsets_case)
+from batch_cases import (AG_DECRYPT_VERIFIED, SENTINEL, byte13_carry_at, corrupt, emul, emul_batch,  # noqa: F401 (emul)
+                         emul_ctr_gated, expand_key, expect_offsets, offsets_case, top_carry_at, wrap_at)
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -17,14 +17,23 @@ from batch_cases import (AG_DECRYPT_VERIFIED, SENTINEL, corrupt, emul, emul_batc
 @pytest.mark.parametrize("kb", [16, 24, 32])
 @pytest.mark.parametrize("G,S", [(1, 1), (2, 1), (4, 1), (32, 1), (32, 4), (32, 16)])
 def test_emul_offsets_verify_then_gated(emul, oracle, kb, G, S):
-    """The batch starts at byte 5 of its buffer: bytes before in_off[0] stay untouched."""
+    """The batch starts at byte 5 of its buffer: bytes before in_off[0] stay untouched.  The second batch holds J0 blocks
+    whose counters wrap past 2^32 or carry into the counter's top byte or byte 13: on the first block of a segment of
+    the tag-only pass, inside a lane-group row and on a row boundary; the gated pass then decrypts the same messages."""
     rng = np.random.default_rng(1000 + kb + 7 * G + S)
     c = offsets_case(oracle, rng, 40, kb, lens=(16 * 40 + 9,), shift=5)
-    want_ok = corrupt(rng, c)
-    _, _, ok = emul_batch(emul, c, AG_DECRYPT_VERIFIED, G, S)
-    assert (ok == want_ok).all(), (kb, G, S)
-    for n_warps in (1, 3):
-        assert (emul_ctr_gated(emul, c, ok, n_warps) == expect_offsets(c, want_ok)).all(), (kb, G, S, n_warps)
+    n = 16 * 9 + 5                      # blocks of the J0 messages (no AAD)
+    seg1 = -(-n // S)                   # first block of segment 1 (ag_batch_segment, a payload block weighing 1)
+    c_j0 = offsets_case(oracle, rng, 40, kb, lens=(16 * n,) * 7, aad_lens=(0,) * 7, shift=5,
+                        j0_ctrs=[wrap_at(0), wrap_at(0), wrap_at(1), top_carry_at(0), wrap_at(1), byte13_carry_at(3),
+                                 wrap_at(seg1), top_carry_at(seg1), wrap_at(5 * G + 3), wrap_at(4 * G), top_carry_at(64),
+                                 byte13_carry_at(100), wrap_at(n - 1)])
+    for c in (c, c_j0):
+        want_ok = corrupt(rng, c)
+        _, _, ok = emul_batch(emul, c, AG_DECRYPT_VERIFIED, G, S)
+        assert (ok == want_ok).all(), (kb, G, S)
+        for n_warps in (1, 3):
+            assert (emul_ctr_gated(emul, c, ok, n_warps) == expect_offsets(c, want_ok)).all(), (kb, G, S, n_warps)
 
 
 @pytest.mark.parametrize("kb", [16, 24, 32])

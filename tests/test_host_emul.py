@@ -6,7 +6,8 @@ import ctypes
 import numpy as np
 import pytest
 
-from batch_cases import emul, emul_batch, expect_offsets, offsets_case  # noqa: F401 (emul: the fixture)
+from batch_cases import (byte13_carry_at, emul, emul_batch, expect_offsets, gf_inv, iv_for_j0, offsets_case,  # noqa: F401
+                         top_carry_at, wrap_at)
 from conftest import u8p, u64p
 
 
@@ -43,30 +44,35 @@ def test_gf_multiplies(emul, oracle):
 
 @pytest.mark.parametrize("kb", [16, 24, 32])
 def test_stream_lanes(emul, oracle, kb):
+    """Block i has counter ctr0 + i (mod 2^32): the pinned ctr0 put the 32-bit wrap on block 0, on the first block of
+    the second CTA and of the second grid row and on two blocks past a row's first, and the carries into the counter's
+    top byte and into byte 13 on block 8; two more are drawn."""
     rng = np.random.default_rng(13 + kb)
     for n in (0, 1, 15, 16, 17, 31, 32, 100, 1000, 4096 + 5):
         for (ncta, nt) in ((1, 1), (1, 4), (3, 8), (2, 32)):
-            for mode in (0, 1, 2):
-                key = rng.integers(0, 256, kb, dtype=np.uint8).tobytes()
-                iv = rng.integers(0, 256, 12, dtype=np.uint8)
-                data = rng.integers(0, 256, max(n, 1), dtype=np.uint8)[:n].copy()
-                rk = np.frombuffer(oracle.key_expand(key), dtype=np.uint8).copy()
-                nr = len(rk) // 16 - 1
-                out = np.zeros(max(n, 1), np.uint8)
-                part = np.zeros(16, np.uint8)
-                inp = data if n else np.zeros(1, np.uint8)
-                ctr0 = int(rng.integers(2, 2 ** 32))  # includes wrap-around of the 32-bit counter
-                rc = emul.emul_stream(u8p(rk), nr, u8p(iv), ctypes.c_uint32(ctr0), u8p(inp), u8p(out), ctypes.c_uint64(n),
-                                      mode, ncta, nt, u8p(part))
-                assert rc == 0
-                h, _ = oracle.h_ej0(rk.tobytes(), iv.tobytes())
-                if mode == 2:
-                    assert part.tobytes() == oracle.ghash_absorb(h, data.tobytes())
-                    continue
-                exp_out = oracle.gctr(rk.tobytes(), iv.tobytes(), ctr0, data.tobytes())
-                assert out[:n].tobytes() == exp_out, (kb, n, ncta, nt, mode)
-                ct = data.tobytes() if mode == 1 else exp_out
-                assert part.tobytes() == oracle.ghash_absorb(h, ct), (kb, n, ncta, nt, mode)
+            gt = ncta * nt
+            pinned = [wrap_at(0), wrap_at(nt), wrap_at(gt), wrap_at(gt // 2 + 1), wrap_at(2 * gt + 3), 0x00FFFFF8, 0x0000FFF8]
+            for ctr0 in pinned + [int(x) for x in rng.integers(2, 2 ** 32, 2)]:
+                for mode in (0, 1, 2):
+                    key = rng.integers(0, 256, kb, dtype=np.uint8).tobytes()
+                    iv = rng.integers(0, 256, 12, dtype=np.uint8)
+                    data = rng.integers(0, 256, max(n, 1), dtype=np.uint8)[:n].copy()
+                    rk = np.frombuffer(oracle.key_expand(key), dtype=np.uint8).copy()
+                    nr = len(rk) // 16 - 1
+                    out = np.zeros(max(n, 1), np.uint8)
+                    part = np.zeros(16, np.uint8)
+                    inp = data if n else np.zeros(1, np.uint8)
+                    rc = emul.emul_stream(u8p(rk), nr, u8p(iv), ctypes.c_uint32(ctr0), u8p(inp), u8p(out), ctypes.c_uint64(n),
+                                          mode, ncta, nt, u8p(part))
+                    assert rc == 0
+                    h, _ = oracle.h_ej0(rk.tobytes(), iv.tobytes())
+                    if mode == 2:
+                        assert part.tobytes() == oracle.ghash_absorb(h, data.tobytes())
+                        continue
+                    exp_out = oracle.gctr(rk.tobytes(), iv.tobytes(), ctr0, data.tobytes())
+                    assert out[:n].tobytes() == exp_out, (kb, n, ncta, nt, mode, hex(ctr0))
+                    ct = data.tobytes() if mode == 1 else exp_out
+                    assert part.tobytes() == oracle.ghash_absorb(h, ct), (kb, n, ncta, nt, mode, hex(ctr0))
 
 
 def _releasing(emul, c, dec, bad, G=1, S=1):
@@ -81,14 +87,27 @@ def _releasing(emul, c, dec, bad, G=1, S=1):
         assert (tags == c["tags"]).all()
 
 
+# J0 counter fields of the J0 cases below, one per message of offsets_case's fixed lengths 0, 1, 15, 16, 17, 16*7+3:
+# the 32-bit wrap on block 0, 0, 1 (past the ragged end), 0 (of a whole block) and 1 (ragged), and the top-byte carry
+# on block 3
+J0_FIRST6 = [wrap_at(0), wrap_at(0), wrap_at(1), wrap_at(0), wrap_at(1), top_carry_at(3)]
+
+
 @pytest.mark.parametrize("G", [1, 2, 4, 8, 16, 32])
 def test_batch_lanes(emul, oracle, G):
-    """Lane groups of G lanes; the 16*600+3 B message carries the counter byte past 256 blocks."""
+    """Lane groups of G lanes; the 16*600+3 B message carries the counter byte past 256 blocks.  J0 cases: the 32-bit
+    wrap and the carries into the counter's top byte and byte 13 on payload blocks 64 (a row boundary for every G) and
+    37 (inside a row for G > 1)."""
     rng = np.random.default_rng(17 + G)
     for kb in (16, 24, 32):
         for dec in (0, 1):
             c = offsets_case(oracle, rng, 9, kb, max_len=200, max_aad=70, lens=(1500, 16 * 600 + 3), aad_lens=(0, 16),
                              decrypt=bool(dec))
+            _releasing(emul, c, dec, 7, G)
+            c = offsets_case(oracle, rng, 12, kb, max_len=200, max_aad=70, lens=(16 * 100 + 3, 16 * 50, 16 * 70 + 9, 100, 16 * 40),
+                             aad_lens=(0, 16, 0, 33, 0), decrypt=bool(dec),
+                             j0_ctrs=J0_FIRST6 + [wrap_at(64), wrap_at(37), top_carry_at(64), byte13_carry_at(5),
+                                                  top_carry_at(37)])
             _releasing(emul, c, dec, 7, G)
 
 
@@ -98,10 +117,18 @@ def test_batch_split_segments(emul, oracle, S):
     segment 0, length block with segment S-1, partials scaled by H^after and XORed.  Includes
     messages shorter than S blocks (empty segments), ragged tails and empty payloads."""
     rng = np.random.default_rng(300 + S)
+    n_wrap = 16 * S * 7   # blocks of the J0 messages below, no AAD: S segments of 4 * n_wrap / S weight positions each
+    seg1 = -(-4 * n_wrap // S) // 4   # ag_batch_segment: first payload block of segment 1
     for kb, G in ((16, 4), (32, 32), (24, 8)):
         for dec in (0, 1):
             c = offsets_case(oracle, rng, 10, kb, max_len=400, max_aad=70, lens=(16 * 300 + 5, 33, 16 * S * 7),
                              aad_lens=(0, 16), decrypt=bool(dec))
+            _releasing(emul, c, dec, 6, G, S)
+            # J0 cases: the wrap and the top-byte carry on the first block of segment 1, on its last block before that
+            # and on a block inside it
+            c = offsets_case(oracle, rng, 10, kb, max_len=400, max_aad=70, lens=(16 * n_wrap,) * 4, aad_lens=(0,) * 4,
+                             decrypt=bool(dec), j0_ctrs=J0_FIRST6 + [wrap_at(seg1), top_carry_at(seg1), wrap_at(seg1 - 1),
+                                                                     top_carry_at(seg1 + 3)])
             _releasing(emul, c, dec, 6, G, S)
 
 
@@ -109,10 +136,16 @@ def test_batch_split_segments(emul, oracle, S):
 def test_batch_balanced_partition(emul, oracle, n_warps):
     """k_batch_warp's balanced partition of uniform records over a virtual grid: cuts inside the AAD,
     inside the payload, inside one payload block's weight, inside the finish positions; more warps
-    than messages and more messages than warps; ragged tails; every message closed exactly once."""
+    than messages and more messages than warps; ragged tails; every message closed exactly once.
+    The last three batches take J0 blocks (16-byte IVs) with the 32-bit wrap, the carry into the counter's top byte
+    and the carry into byte 13 on the first, a middle and the last payload block."""
     rng = np.random.default_rng(500 + n_warps)
-    for kb, nm, length, alen in ((16, 5, 16 * 37 + 5, 16 * 11 + 3), (32, 2, 16 * 200, 0), (24, 9, 100, 700), (16, 3, 0, 50),
-                                 (32, 6, 16, 16), (24, 1, 16 * 129 + 1, 16 * 5)):
+    edge = lambda nb: [wrap_at(0), wrap_at(nb // 2), top_carry_at(nb - 1), byte13_carry_at(1), top_carry_at(nb // 3),  # noqa: E731
+                       wrap_at(nb - 1)]
+    for kb, nm, length, alen, j0 in ((16, 5, 16 * 37 + 5, 16 * 11 + 3, False), (32, 2, 16 * 200, 0, False),
+                                     (24, 9, 100, 700, False), (16, 3, 0, 50, False), (32, 6, 16, 16, False),
+                                     (24, 1, 16 * 129 + 1, 16 * 5, False),
+                                     (16, 6, 16 * 37 + 5, 16 * 11 + 3, True), (32, 5, 16 * 200, 0, True), (24, 6, 100, 70, True)):
         for dec in (0, 1):
             stride, astride = length + 3, alen + 5
             buf = rng.integers(0, 256, nm * stride + 1, dtype=np.uint8)
@@ -125,24 +158,38 @@ def test_batch_balanced_partition(emul, oracle, n_warps):
             apacked = abuf[:nm * astride].reshape(nm, astride)[:, :alen].reshape(-1).copy()
             in_off = (np.arange(nm + 1) * length).astype(np.uint64)
             aad_off = (np.arange(nm + 1) * alen).astype(np.uint64)
-            eo, et = oracle.gcm_batch(key, kb, True, ivs, apacked if alen else None, aad_off if alen else None, packed, in_off,
-                                      decrypt=bool(dec))
+            if j0:
+                h = oracle.aes_encrypt_block(rk.tobytes(), bytes(16))
+                h_inv = gf_inv(oracle, h)
+                ivs = np.zeros(16 * nm, np.uint8)
+                eo, et = np.zeros(nm * length, np.uint8), np.zeros(16 * nm, np.uint8)
+                for m, c0 in enumerate(edge((length + 15) // 16)[:nm]):
+                    j0b = rng.integers(0, 256, 12, dtype=np.uint8).tobytes() + c0.to_bytes(4, "big")
+                    ivs[16 * m:16 * m + 16] = np.frombuffer(j0b, np.uint8)
+                    p_, t_ = oracle.gcm_crypt_any_iv(key.tobytes(), iv_for_j0(oracle, h, h_inv, j0b),
+                                                     apacked[m * alen:(m + 1) * alen].tobytes(),
+                                                     packed[m * length:(m + 1) * length].tobytes(), decrypt=bool(dec))
+                    eo[m * length:(m + 1) * length] = np.frombuffer(p_, np.uint8)
+                    et[16 * m:16 * m + 16] = np.frombuffer(t_, np.uint8)
+            else:
+                eo, et = oracle.gcm_batch(key, kb, True, ivs, apacked if alen else None, aad_off if alen else None, packed,
+                                          in_off, decrypt=bool(dec))
             out = np.zeros_like(buf)
             tag = np.zeros(16 * nm, np.uint8)
             ok = np.zeros(nm, np.uint8)
             if dec:
                 tag[:] = et
                 tag[16 * (nm - 1) + 2] ^= 0x40
-            rc = emul.emul_batch_balanced(u8p(rk), nr, dec, n_warps, u8p(ivs), u8p(abuf), ctypes.c_uint64(alen),
+            rc = emul.emul_batch_balanced(u8p(rk), nr, dec, n_warps, u8p(ivs), int(j0), u8p(abuf), ctypes.c_uint64(alen),
                                           ctypes.c_uint64(astride), u8p(buf), u8p(out), ctypes.c_uint64(length),
                                           ctypes.c_uint64(stride), u8p(tag), u8p(ok), ctypes.c_uint64(nm))
             assert rc == 0
             got = out[:nm * stride].reshape(nm, stride)[:, :length].reshape(-1)
-            assert (got == eo[:nm * length]).all(), (kb, nm, length, alen, dec)
+            assert (got == eo[:nm * length]).all(), (kb, nm, length, alen, dec, j0)
             if dec:
-                assert list(ok) == [1] * (nm - 1) + [0], (kb, nm, length, alen)
+                assert list(ok) == [1] * (nm - 1) + [0], (kb, nm, length, alen, j0)
             else:
-                assert (tag == et).all(), (kb, nm, length, alen)
+                assert (tag == et).all(), (kb, nm, length, alen, j0)
 
 
 @pytest.mark.parametrize("kb", [16, 24, 32])
@@ -152,6 +199,32 @@ def test_perkey_messages(emul, oracle, kb):
     for dec in (0, 1):
         c = offsets_case(oracle, rng, 12, kb, max_aad=80, lens=(1500,), aad_lens=(64, 0), perkey=True, decrypt=bool(dec))
         _releasing(emul, c, dec, 4)
+
+
+@pytest.mark.parametrize("kb", [16, 24, 32])
+def test_counter_caches(emul, oracle, kb):
+    """The per-lane counter caches against AES-ECB of the counter blocks: the batch lanes' sequential cache, the stream
+    kernel's cache and the per-key kernels' copy of the sequential refill (schedule on the fly).  32-block windows
+    across the carry into the counter's top byte, the carry into byte 13 and the wrap to 0; and steps that move one
+    counter byte alone (2^24: the top byte only), which consecutive counters never do."""
+    rng = np.random.default_rng(40 + kb)
+    key = rng.integers(0, 256, kb, dtype=np.uint8)
+    iv = rng.integers(0, 256, 12, dtype=np.uint8)
+    rk = np.frombuffer(oracle.key_expand(key.tobytes()), dtype=np.uint8).copy()
+    nr = len(rk) // 16 - 1
+    U32, U64 = ctypes.c_uint32, ctypes.c_uint64
+    for ctr0, stride, n in ((0x00FFFFF0, 1, 32), (0x0000FFF0, 1, 32), (0xFFFFFFF0, 1, 32), (0xFFFFFFF0, 3, 32),
+                            (0x00FFFFF0, 256, 32), (0x12345678, 1 << 24, 300), (0x12345678, 1 << 16, 300),
+                            (0x12345678, 1 << 8, 300), (0x12345678, 0x01010101, 300)):
+        want = b"".join(oracle.aes_encrypt_block(rk.tobytes(), iv.tobytes() + ((ctr0 + k * stride) & 0xFFFFFFFF).to_bytes(4, "big"))
+                        for k in range(n))
+        out = np.zeros(16 * n, np.uint8)
+        for which in (0, 1):
+            assert emul.emul_ctr_cached(u8p(rk), nr, u8p(iv), U32(ctr0), U32(stride), U64(n), which, u8p(out)) == 0
+            assert out.tobytes() == want, (kb, hex(ctr0), stride, which)
+        out[:] = 0
+        assert emul.emul_perkey_ctr(u8p(key), kb, u8p(iv), U32(ctr0), U32(stride), U64(n), u8p(out)) == 0
+        assert out.tobytes() == want, (kb, hex(ctr0), stride, "perkey")
 
 
 def test_host_pipeline_granule_schedule(emul):
