@@ -49,6 +49,10 @@ SIGNATURES = {
     "agcm_stream_decrypt_verified": (c_int, [c_vp, c_u8p, c_sz, c_u8p, c_u64, c_u8p, c_u8p, c_u64, c_u8p, c_u8p, c_vp]),
     "agcm_stream_decrypt_verified_host": (c_int, [c_vp, c_u8p, c_sz, c_u8p, c_u64, c_u8p, c_u8p, c_u64, c_u8p,
                                                   ctypes.POINTER(c_int)]),
+    "agcm_stream_decrypt_verified_peer": (c_int, [c_vp, c_u8p, c_sz, c_u64, c_u8p, c_u8p, c_u64, c_u64, c_u8p, c_u64, c_u64,
+                                                  c_u8p, c_u8p, c_vp]),
+    "agcm_stream_decrypt_verified_peer_host": (c_int, [c_vp, c_u8p, c_sz, c_u64, c_u8p, c_u8p, c_u64, c_u64, c_u8p, c_u64,
+                                                       c_u64, c_u8p, ctypes.POINTER(c_int)]),
     "agcm_derive_j0": (c_int, [c_vp, c_u8p, c_sz, c_u8p]),
     "agcm_gctr_j0": (c_int, [c_vp, c_u8p, c_u64, c_u8p, c_u8p, c_u64, c_vp]),
     "agcm_stream_part_j0": (c_int, [c_vp, c_int, c_u8p, c_u64, c_u8p, c_u8p, c_u64, c_u64, c_u8p, c_vp]),

@@ -914,6 +914,19 @@ static int peer_finish(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], const
     return AGCM_OK;
 }
 
+// This rank's bulk kernel of exchange `epoch` (ENC, DEC or GHASH_ONLY); its last CTA posts the scaled partial to every rank.
+static int peer_bulk(agcm_ctx* c, int mode, const uint8_t h_iv12[12], uint64_t first_block, const uint8_t* d_in, uint8_t* d_out,
+                     uint64_t n_bytes, uint64_t blocks_after, cudaStream_t st, uint32_t epoch)
+{
+    if (n_bytes)
+        return run_stream(c, mode, h_iv12, first_block, d_in, d_out, n_bytes, blocks_after, c->d_parts, nullptr, st, c->d_counters,
+                          nullptr, epoch);
+    // an empty counter range (fewer blocks than ranks) still posts its zero partial
+    AG_CUDA(c, ag_launch_peer_post(c->d_peer_bufs, (uint32_t)c->peer_rank, (uint32_t)c->peer_world, epoch, nullptr, st));
+    c->launches++;
+    return AGCM_OK;
+}
+
 static int stream_crypt_peer(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], uint64_t first_block, const uint8_t* d_in,
                              uint8_t* d_out, uint64_t n_bytes, uint64_t blocks_after, const uint8_t* d_aad, uint64_t aad_len,
                              uint64_t total_len, uint8_t* d_tag, uint8_t* d_ok, void* stream, bool deferred)
@@ -924,14 +937,8 @@ static int stream_crypt_peer(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12],
     uint32_t epoch = 0;
     int rc = peer_begin(c, first_block, n_bytes, blocks_after, aad_len, total_len, st, &epoch);
     if (rc) return rc;
-    if (n_bytes) {
-        rc = run_stream(c, decrypt ? AG_MODE_DEC : AG_MODE_ENC, h_iv12, first_block, d_in, d_out, n_bytes, blocks_after,
-                        c->d_parts, nullptr, st, c->d_counters, nullptr, epoch);
-        if (rc) return rc;
-    } else {   // an empty counter range (fewer blocks than ranks) still posts its zero partial
-        AG_CUDA(c, ag_launch_peer_post(c->d_peer_bufs, (uint32_t)c->peer_rank, (uint32_t)c->peer_world, epoch, nullptr, st));
-        c->launches++;
-    }
+    rc = peer_bulk(c, decrypt ? AG_MODE_DEC : AG_MODE_ENC, h_iv12, first_block, d_in, d_out, n_bytes, blocks_after, st, epoch);
+    if (rc) return rc;
     return peer_finish(c, decrypt, h_iv12, d_aad, aad_len, total_len, d_tag, d_ok, st, epoch, deferred);
 }
 
@@ -1016,6 +1023,30 @@ int agcm_stream_decrypt_verified(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len
     if (rc) return rc;
     // pass 2: GCTR, gated on the device by the flag pass 1 just wrote (no host round trip)
     return run_stream(c, AG_MODE_CTR_ONLY, j0, 0, d_ct, d_pt, n_bytes, 0, c->d_parts, nullptr, st, c->d_counters, nullptr, 0, d_ok);
+}
+
+int agcm_stream_decrypt_verified_peer(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len, uint64_t first_block,
+                                      const uint8_t* d_ct, uint8_t* d_pt, uint64_t n_bytes, uint64_t blocks_after,
+                                      const uint8_t* d_aad, uint64_t aad_len, uint64_t total_len, const uint8_t* d_tag,
+                                      uint8_t* d_ok, void* stream)
+{
+    if (!c || !h_iv || !d_tag || !d_ok || (n_bytes && (!d_ct || !d_pt)) || (aad_len && !d_aad)) return AGCM_E_BAD_ARG;
+    cudaStream_t st = (cudaStream_t)stream;
+    uint32_t epoch = 0;
+    int rc = peer_begin(c, first_block, n_bytes, blocks_after, aad_len, total_len, st, &epoch);
+    if (rc) return rc;
+    uint8_t j0[16];
+    rc = resolve_j0(c, h_iv, iv_len, j0, st);
+    if (rc) return rc;
+    J0Scope scope(c, j0);
+    // pass 1: GHASH over this rank's ciphertext, partial posted; the finish checks the WORLD's tag into d_ok
+    rc = peer_bulk(c, AG_MODE_GHASH_ONLY, j0, first_block, d_ct, nullptr, n_bytes, blocks_after, st, epoch);
+    if (rc) return rc;
+    rc = peer_finish(c, 1, j0, d_aad, aad_len, total_len, const_cast<uint8_t*>(d_tag), d_ok, st, epoch, false);
+    if (rc) return rc;
+    // pass 2: GCTR over this rank's shard, gated on the device by that flag
+    return run_stream(c, AG_MODE_CTR_ONLY, j0, first_block, d_ct, d_pt, n_bytes, 0, c->d_parts, nullptr, st, c->d_counters,
+                      nullptr, 0, d_ok);
 }
 
 int agcm_gctr(agcm_ctx* c, const uint8_t h_iv12[12], uint64_t first_block, const uint8_t* d_in, uint8_t* d_out,
@@ -1834,6 +1865,43 @@ int agcm_stream_crypt_host(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], c
     return host_end(c, decrypt, h_tag, h_ok, c->hs[0]);
 }
 
+// Pass 1 of a verify-then-release host decrypt: the ciphertext is copied into c->verify, where it stays for pass 2, and
+// absorbed chunk by chunk (the copy of chunk k+1 overlaps the GHASH of chunk k).  The chunk partials, each scaled for
+// every block after it (`blocks_after` more past the range), land in c->d_chunk_partials.  Waits for slots 1..kSlots-1.
+static int verify_absorb_host(agcm_ctx* c, const uint8_t j0[12], const uint8_t* h_ct, uint64_t n_bytes, uint64_t chunk,
+                              uint64_t blocks_after)
+{
+    const uint64_t nblocks = (n_bytes + 15) >> 4;
+    for (uint64_t k = 0, off = 0; off < n_bytes; ++k, off += chunk) {
+        const int s = (int)(k % kSlots);
+        const uint64_t nb = (n_bytes - off) < chunk ? (n_bytes - off) : chunk;
+        const uint64_t after = nblocks - (off >> 4) - ((nb + 15) >> 4) + blocks_after;
+        AG_CUDA(c, cudaMemcpyAsync(c->verify.p + off, h_ct + off, nb, cudaMemcpyHostToDevice, c->hs[s]));
+        int rc = run_stream(c, AG_MODE_GHASH_ONLY, j0, 0, c->verify.p + off, nullptr, nb, after, c->d_stage_parts[s],
+                            c->d_chunk_partials + 16 * k, c->hs[s], c->d_counters + 1 + s);
+        if (rc) return rc;
+    }
+    for (int s = 1; s < kSlots; ++s) AG_CUDA(c, cudaStreamSynchronize(c->hs[s]));
+    return AGCM_OK;
+}
+
+// Pass 2, run only once the tag matched: GCTR in place over c->verify from counter block `first_block`, chunk by chunk,
+// copied out to h_pt.  Waits for every slot.
+static int verify_release_host(agcm_ctx* c, const uint8_t j0[12], uint64_t first_block, uint8_t* h_pt, uint64_t n_bytes,
+                               uint64_t chunk)
+{
+    for (uint64_t k = 0, off = 0; off < n_bytes; ++k, off += chunk) {
+        const int s = (int)(k % kSlots);
+        const uint64_t nb = (n_bytes - off) < chunk ? (n_bytes - off) : chunk;
+        int rc = run_stream(c, AG_MODE_CTR_ONLY, j0, first_block + (off >> 4), c->verify.p + off, c->verify.p + off, nb, 0,
+                            c->d_stage_parts[s], nullptr, c->hs[s], c->d_counters + 1 + s);
+        if (rc) return rc;
+        AG_CUDA(c, cudaMemcpyAsync(h_pt + off, c->verify.p + off, nb, cudaMemcpyDeviceToHost, c->hs[s]));
+    }
+    for (int s = 0; s < kSlots; ++s) AG_CUDA(c, cudaStreamSynchronize(c->hs[s]));
+    return AGCM_OK;
+}
+
 int agcm_stream_decrypt_verified_host(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len, const uint8_t* h_aad, uint64_t aad_len,
                                       const uint8_t* h_ct, uint8_t* h_pt, uint64_t n_bytes, const uint8_t h_tag[16], int* h_ok)
 {
@@ -1848,21 +1916,12 @@ int agcm_stream_decrypt_verified_host(agcm_ctx* c, const uint8_t* h_iv, size_t i
     rc = resolve_j0(c, h_iv, iv_len, j0, c->hs[0]);
     if (rc) return rc;
     J0Scope scope(c, j0);
-    const uint64_t nblocks = (n_bytes + 15) >> 4, chunk = pick_chunk(c, n_bytes);
+    const uint64_t chunk = pick_chunk(c, n_bytes);
     const uint64_t n_chunks = (n_bytes + chunk - 1) / chunk;
     if (n_chunks > SC_PARTS_MAX) return AGCM_E_BAD_LEN;
-    // pass 1: copy in and absorb, chunk by chunk (the copy of chunk k+1 overlaps the GHASH of chunk k)
     if (aad_len) AG_CUDA(c, cudaMemcpyAsync(c->aad_stage.p, h_aad, aad_len, cudaMemcpyHostToDevice, c->hs[0]));
-    for (uint64_t k = 0; k < n_chunks; ++k) {
-        const int s = (int)(k % kSlots);
-        const uint64_t off = k * chunk, nb = (n_bytes - off) < chunk ? (n_bytes - off) : chunk;
-        const uint64_t after = nblocks - (off >> 4) - ((nb + 15) >> 4);
-        AG_CUDA(c, cudaMemcpyAsync(c->verify.p + off, h_ct + off, nb, cudaMemcpyHostToDevice, c->hs[s]));
-        rc = run_stream(c, AG_MODE_GHASH_ONLY, j0, 0, c->verify.p + off, nullptr, nb, after, c->d_stage_parts[s],
-                        c->d_chunk_partials + 16 * k, c->hs[s], c->d_counters + 1 + s);
-        if (rc) return rc;
-    }
-    for (int s = 1; s < kSlots; ++s) AG_CUDA(c, cudaStreamSynchronize(c->hs[s]));
+    rc = verify_absorb_host(c, j0, h_ct, n_bytes, chunk, 0);
+    if (rc) return rc;
     uint8_t* d_tag = c->d_scratch + SC_TAG;
     uint8_t* d_ok = c->d_scratch + SC_OK;
     AG_CUDA(c, cudaMemcpyAsync(d_tag, h_tag, 16, cudaMemcpyHostToDevice, c->hs[0]));
@@ -1870,17 +1929,52 @@ int agcm_stream_decrypt_verified_host(agcm_ctx* c, const uint8_t* h_iv, size_t i
     if (rc) return rc;
     rc = host_end(c, 1, nullptr, h_ok, c->hs[0]);
     if (rc || !*h_ok) return rc;   // not authentic: no plaintext byte leaves the device
-    // pass 2: GCTR in place, chunk by chunk, copy out
-    for (uint64_t k = 0; k < n_chunks; ++k) {
-        const int s = (int)(k % kSlots);
-        const uint64_t off = k * chunk, nb = (n_bytes - off) < chunk ? (n_bytes - off) : chunk;
-        rc = run_stream(c, AG_MODE_CTR_ONLY, j0, off >> 4, c->verify.p + off, c->verify.p + off, nb, 0, c->d_stage_parts[s], nullptr,
-                        c->hs[s], c->d_counters + 1 + s);
-        if (rc) return rc;
-        AG_CUDA(c, cudaMemcpyAsync(h_pt + off, c->verify.p + off, nb, cudaMemcpyDeviceToHost, c->hs[s]));
+    return verify_release_host(c, j0, 0, h_pt, n_bytes, chunk);
+}
+
+int agcm_stream_decrypt_verified_peer_host(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len, uint64_t first_block,
+                                           const uint8_t* h_ct, uint8_t* h_pt, uint64_t n_bytes, uint64_t blocks_after,
+                                           const uint8_t* h_aad, uint64_t aad_len, uint64_t total_len, const uint8_t h_tag[16],
+                                           int* h_ok)
+{
+    if (!c || !h_iv || !h_tag || !h_ok || (n_bytes && (!h_ct || !h_pt)) || (aad_len && !h_aad)) return AGCM_E_BAD_ARG;
+    if (c->peer_world < 1) return AGCM_E_BAD_ARG;
+    int rc = host_begin(c, aad_len);
+    if (rc) return rc;
+    const uint64_t chunk = pick_chunk(c, n_bytes);
+    const uint64_t n_chunks = (n_bytes + chunk - 1) / chunk;
+    if (n_chunks > SC_PARTS_MAX) return AGCM_E_BAD_LEN;
+    rc = grow(c, c->verify, n_bytes);   // this rank's ciphertext stays in HBM between the two passes
+    if (rc) return rc;
+    cudaStream_t st = c->hs[0];
+    uint32_t epoch = 0;
+    rc = peer_begin(c, first_block, n_bytes, blocks_after, aad_len, total_len, st, &epoch);
+    if (rc) return rc;
+    uint8_t j0[16];
+    rc = resolve_j0(c, h_iv, iv_len, j0, st);
+    if (rc) return rc;
+    J0Scope scope(c, j0);
+    if (aad_len) AG_CUDA(c, cudaMemcpyAsync(c->aad_stage.p, h_aad, aad_len, cudaMemcpyHostToDevice, st));
+    rc = verify_absorb_host(c, j0, h_ct, n_bytes, chunk, blocks_after);
+    if (rc) return rc;
+    uint8_t* d_tag = c->d_scratch + SC_TAG;
+    uint8_t* d_ok = c->d_scratch + SC_OK;
+    AG_CUDA(c, cudaMemcpyAsync(d_tag, h_tag, 16, cudaMemcpyHostToDevice, st));
+    const uint8_t* d_p = nullptr;   // null = the zero partial of an empty range
+    if (n_chunks) {
+        AG_CUDA(c, ag_launch_xor_parts(c->d_chunk_partials, (uint32_t)n_chunks, c->d_scratch + SC_PART_CT, st));
+        c->launches++;
+        d_p = c->d_scratch + SC_PART_CT;
     }
-    for (int s = 0; s < kSlots; ++s) AG_CUDA(c, cudaStreamSynchronize(c->hs[s]));
-    return AGCM_OK;
+    AG_CUDA(c, ag_launch_peer_post(c->d_peer_bufs, (uint32_t)c->peer_rank, (uint32_t)c->peer_world, epoch, d_p, st));
+    c->launches++;
+    rc = peer_finish(c, 1, j0, c->aad_stage.p, aad_len, total_len, d_tag, d_ok, st, epoch, false);
+    if (rc) return rc;
+    rc = host_end(c, 1, nullptr, h_ok, st);
+    if (rc) return rc;
+    if (*(volatile uint32_t*)c->h_peer_status) return AGCM_E_PEER_TIMEOUT;   // failed closed: ok = 0, nothing released
+    if (!*h_ok) return AGCM_OK;   // the world's tag did not match: no plaintext byte leaves the device
+    return verify_release_host(c, j0, first_block, h_pt, n_bytes, chunk);
 }
 
 int agcm_stream_crypt_iv_host(agcm_ctx* c, int decrypt, const uint8_t* h_iv, size_t iv_len, const uint8_t* h_aad,

@@ -256,6 +256,20 @@ class GcmEngine:
                                                      ctypes.byref(ok)))
         return bool(ok.value) if decrypt else t.tobytes()
 
+    def stream_decrypt_verified_peer_host(self, iv, first_block, ct, pt, blocks_after, aad, total_len, tag):
+        """Verify-then-release form of stream_crypt_peer_host(1, ...): `pt` is written only if the whole message's tag
+        matches on every rank.  IV of any length.  -> ok."""
+        ivb, d, o, a, tb = _np_u8(iv), _np_u8(ct), _np_u8(pt), _np_u8(aad), _np_u8(tag)
+        if tb.size != 16:
+            raise _lib.AgcmError(_lib.E_BAD_LEN, "tag must be 16 bytes")
+        if o.size < d.size:
+            raise _lib.AgcmError(_lib.E_BAD_LEN, "output buffer too small")
+        ok = ctypes.c_int(0)
+        self._ck(self._L.agcm_stream_decrypt_verified_peer_host(self._ctx, _addr(ivb), ivb.size, int(first_block), _addr(d),
+                                                                _addr(o), d.size, int(blocks_after), _addr(a), a.size,
+                                                                int(total_len), _addr(tb), ctypes.byref(ok)))
+        return bool(ok.value)
+
     def timing_enable(self, on=True):
         self._ck(self._L.agcm_timing_enable(self._ctx, int(bool(on))))
 
@@ -327,6 +341,17 @@ class GcmEngine:
             self._ck(self._L.agcm_stream_crypt_peer_j0(*args, int(bool(defer))))
         else:
             self._ck((self._L.agcm_stream_crypt_peer_async if defer else self._L.agcm_stream_crypt_peer)(*args))
+
+    def stream_decrypt_verified_peer_device(self, iv, first_block, ct, pt, blocks_after, aad, total_len, tag, ok, n_bytes=None,
+                                            stream=None):
+        """Verify-then-release form of stream_crypt_peer_device(1, ...): ok[0] = 1 on every rank if and only if the whole
+        message's tag matches, and only then is this rank's `pt` written.  IV of any length; no deferred form."""
+        ivb = _np_u8(iv)
+        n = (0 if ct is None else ct.numel()) if n_bytes is None else int(n_bytes)
+        self._ck(self._L.agcm_stream_decrypt_verified_peer(self._ctx, _addr(ivb), ivb.size, int(first_block), _dptr(ct),
+                                                           _dptr(pt), n, int(blocks_after), _dptr(aad),
+                                                           0 if aad is None else aad.numel(), int(total_len), _dptr(tag),
+                                                           _dptr(ok), _stream(stream)))
 
     def peer_join(self, stream=None):
         """`stream` waits for every deferred peer finish issued so far (no host synchronisation)."""

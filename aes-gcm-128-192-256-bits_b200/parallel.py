@@ -116,6 +116,18 @@ class PeerExchange:
         return self.engine.stream_crypt_peer_host(decrypt, iv, shard.first_block, h_in[:shard.n_bytes], h_out[:shard.n_bytes],
                                                   shard.blocks_after, aad, total_bytes, tag)
 
+    def decrypt_verified(self, iv, aad, shard, ct, pt, total_bytes, tag, ok, stream=None):
+        """Verify-then-release decrypt of this rank's shard: ok[0] = 1 on every rank if and only if the whole message's
+        tag matches, and no rank writes any plaintext otherwise.  `ok` and `pt` are valid in stream order (no join)."""
+        self.engine.stream_decrypt_verified_peer_device(iv, shard.first_block, ct if shard.n_bytes else None,
+                                                        pt if shard.n_bytes else None, shard.blocks_after, aad, total_bytes,
+                                                        tag, ok, n_bytes=shard.n_bytes, stream=stream)
+
+    def decrypt_verified_host(self, iv, aad, shard, h_ct, h_pt, total_bytes, tag):
+        """The same for a shard in (pinned) HOST memory.  -> ok; on False h_pt is untouched."""
+        return self.engine.stream_decrypt_verified_peer_host(iv, shard.first_block, h_ct[:shard.n_bytes], h_pt[:shard.n_bytes],
+                                                             shard.blocks_after, aad, total_bytes, tag)
+
     def join(self, stream=None):
         self.engine.peer_join(stream)
 

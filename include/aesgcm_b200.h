@@ -125,7 +125,8 @@ int agcm_stream_crypt(agcm_ctx* ctx, int decrypt, const uint8_t h_iv12[12], cons
  * block at load_cipher_text time, the tag is only checked at get_tag), every decrypt call above and
  * below writes the plaintext BEFORE the tag is known to match -- on the host-buffer paths each chunk
  * is copied back while later chunks are still in flight.  Callers that must not see unauthenticated
- * plaintext use the two-pass form:
+ * plaintext use the two-pass forms: this one for a message on one GPU, agcm_batch_decrypt_verified* for
+ * batches, agcm_stream_decrypt_verified_peer(_host) for a message sharded over GPUs (below).
  * agcm_stream_decrypt_verified: pass 1 = GHASH over the ciphertext + tag check (about 4x the rate of
  * the fused pass), pass 2 = GCTR gated ON THE DEVICE by the flag pass 1 wrote: when the tag does
  * not match, *d_ok = 0 and d_pt is not written at all.  IV of any length (host pointer). */
@@ -243,6 +244,34 @@ int agcm_stream_crypt_peer_async(agcm_ctx* ctx, int decrypt, const uint8_t h_iv1
                                  const uint8_t* d_in, uint8_t* d_out, uint64_t n_bytes, uint64_t blocks_after,
                                  const uint8_t* d_aad, uint64_t aad_len, uint64_t total_len, uint8_t* d_tag, uint8_t* d_ok,
                                  void* stream);
+
+/* VERIFY-THEN-RELEASE SHARDED DECRYPT: agcm_stream_decrypt_verified_peer decrypts this rank's shard of a message sharded as
+ * for agcm_stream_crypt_peer.  Pass 1 = GHASH over this rank's ciphertext, the scaled partial posted to every rank; the
+ * one-warp finish compares the WORLD's tag with d_tag; pass 2 = GCTR over this rank's shard, gated on the device by that
+ * flag.  IV of any length (host pointer, as agcm_stream_decrypt_verified).  Guarantees:
+ *   - on every rank, *d_ok = 1 if and only if the tag of the whole message matches the d_tag that rank was given;
+ *   - a rank writes its plaintext bytes if and only if its *d_ok == 1; no other byte of d_pt is ever written, so one
+ *     flipped bit in any rank's ciphertext, in the AAD or in the tag makes every rank release nothing;
+ *   - d_ct == d_pt (exactly aliased) is allowed: a failed shard then still holds its ciphertext;
+ *   - FAILS CLOSED as the releasing calls: if a rank never posts, *d_ok = 0, nothing is released, and every later peer
+ *     call returns AGCM_E_PEER_TIMEOUT until agcm_peer_setup runs again.
+ * d_ok and d_pt are valid in stream order on `stream`.  There is no deferred form: release needs the world's tag, so every
+ * message is a rank-wide wait.  Argument checks, error codes and limits are those of agcm_stream_crypt_peer (aad_len <= 4096,
+ * the same first_block / blocks_after / total_len consistency, an empty counter range still posts, total_len == 0 = GMAC
+ * only); d_tag and d_ok are required (AGCM_E_BAD_ARG).  The call takes one epoch of the exchange ring like every other peer
+ * call, so it interleaves with the releasing calls as long as every rank makes the same sequence of calls.
+ * agcm_stream_decrypt_verified_peer_host: the same from host buffers, as agcm_stream_decrypt_verified_host -- the shard is
+ * copied into HBM once (n_bytes of device memory, kept by the context) and absorbed chunk by chunk; only when the world's
+ * tag matches does the GCTR pass run and the plaintext travel back.  On a mismatch *h_ok = 0 and h_pt is untouched; if a
+ * rank never posts, the call returns AGCM_E_PEER_TIMEOUT at once (h_pt untouched).  Synchronous. */
+int agcm_stream_decrypt_verified_peer(agcm_ctx* ctx, const uint8_t* h_iv, size_t iv_len, uint64_t first_block,
+                                      const uint8_t* d_ct, uint8_t* d_pt, uint64_t n_bytes, uint64_t blocks_after,
+                                      const uint8_t* d_aad, uint64_t aad_len, uint64_t total_len,
+                                      const uint8_t* d_tag, uint8_t* d_ok, void* stream);
+int agcm_stream_decrypt_verified_peer_host(agcm_ctx* ctx, const uint8_t* h_iv, size_t iv_len, uint64_t first_block,
+                                           const uint8_t* h_ct, uint8_t* h_pt, uint64_t n_bytes, uint64_t blocks_after,
+                                           const uint8_t* h_aad, uint64_t aad_len, uint64_t total_len,
+                                           const uint8_t h_tag[16], int* h_ok);
 
 /* ---- many independent messages under the shared key ---------------------------
  * Message i: IV d_iv12[12i..], AAD d_aad[aad_off[i]..aad_off[i+1]), payload
