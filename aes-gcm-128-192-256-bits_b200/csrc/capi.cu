@@ -22,6 +22,8 @@ constexpr size_t kChunkBytesMax = 64u << 20;  // host pipeline granule (upper bo
 constexpr size_t kMaxChunks = 8192;
 constexpr uint64_t kAadInlineMax = 4096;   // bytes of AAD folded inside k_stream_finish
 constexpr uint64_t kMaxBlocks = 0xFFFFFFFEull;
+// J0 of the all-zero 96-bit IV, for the GHASH-only launches that belong to no message (derive_j0, agcm_ghash)
+constexpr uint8_t kJ0ZeroIv[16] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 1};
 
 // scratch layout (bytes) inside ctx->d_scratch
 constexpr size_t SC_PART_CT = 0;     // 16
@@ -63,7 +65,6 @@ struct agcm_ctx {
     uint32_t* d_counters = nullptr;  // last-CTA tickets: [0] context scratch, [1+s] pipeline slot s
     PowCache pow_n;                  // H^n for the tag finish
     PowCache pow_scale;              // H^blocks_after of the last shard call
-    uint32_t j0ctr = 1;              // counter field of J0 for the call in progress (1 for a 96-bit IV)
     GrownBuf<uint8_t> iv_stage;      // padded long IV for the J0 derivation
     // peer-memory exchange (multi-GPU)
     uint8_t** d_peer_bufs = nullptr; // device array of world pointers
@@ -99,7 +100,6 @@ struct agcm_ctx {
     uint8_t* d_chunk_partials = nullptr;
     GrownBuf<uint8_t> aad_stage;         // host-supplied AAD
     uint32_t* d_tile_ticket = nullptr;   // k_batch_tile / _warp / _cta: next unit (zeroed before each launch)
-    bool no_ticket = false;              // set while the host batch pipeline runs chunks on several streams at once
     GrownBuf<uint32_t> sort;             // length sort of an offset batch: 4096 bucket counters, then perm[n_msgs]
     void* tmap_encode = nullptr;         // cuTensorMapEncodeTiled, resolved through the runtime (no link-time libcuda)
     GrownBuf<uint8_t> verify;            // whole ciphertext of a verify-then-release host decrypt
@@ -132,11 +132,25 @@ int mode_to_nr(int mode)
     return 0;
 }
 
-void iv_words(const uint8_t iv[12], uint32_t w[3])
+// J0 as the kernels take it: its first 12 bytes as little-endian words in w, and its counter field (the last 32 bits,
+// big-endian; 1 for a 96-bit IV) returned
+uint32_t j0_words(const uint8_t j0[16], uint32_t w[3])
 {
     for (int i = 0; i < 3; ++i)
-        w[i] = (uint32_t)iv[4 * i] | ((uint32_t)iv[4 * i + 1] << 8) | ((uint32_t)iv[4 * i + 2] << 16) |
-               ((uint32_t)iv[4 * i + 3] << 24);
+        w[i] = (uint32_t)j0[4 * i] | ((uint32_t)j0[4 * i + 1] << 8) | ((uint32_t)j0[4 * i + 2] << 16) |
+               ((uint32_t)j0[4 * i + 3] << 24);
+    return ((uint32_t)j0[12] << 24) | ((uint32_t)j0[13] << 16) | ((uint32_t)j0[14] << 8) | (uint32_t)j0[15];
+}
+
+// J0 of a 96-bit IV (SP 800-38D 7.1 step 2), IV || 0^31 || 1, written to j0 and returned; null for a null IV, which
+// every function that takes J0 refuses with AGCM_E_BAD_ARG
+const uint8_t* j0_of_iv12(const uint8_t* iv, uint8_t j0[16])
+{
+    if (!iv) return nullptr;
+    memcpy(j0, iv, 12);
+    j0[12] = j0[13] = j0[14] = 0;
+    j0[15] = 1;
+    return j0;
 }
 
 // fold finished (event pair) timings of the stream kernel into the running total
@@ -206,15 +220,14 @@ int ensure_pow(agcm_ctx* c, uint64_t n_blocks, cudaStream_t st)
 }
 
 // Fields all three forms of the tag finish share.  On decrypt the computed tag goes to scratch, never to the caller.
-FinishParams finish_params(const agcm_ctx* c, int decrypt, const uint8_t iv[12], const uint8_t* d_aad, uint64_t aad_len,
+FinishParams finish_params(const agcm_ctx* c, int decrypt, const uint8_t j0[16], const uint8_t* d_aad, uint64_t aad_len,
                            uint64_t ct_len, uint8_t* d_tag, uint8_t* d_ok, const uint32_t* hn)
 {
     FinishParams f;
     memset(&f, 0, sizeof(f));
     memcpy(f.rk, c->h_rk, sizeof(f.rk));
     f.nr = (uint32_t)c->nr;
-    iv_words(iv, f.iv);
-    f.j0w = __builtin_bswap32(c->j0ctr);
+    f.j0w = __builtin_bswap32(j0_words(j0, f.iv));
     f.key = c->d_key;
     f.te0 = c->d_te0;
     f.aad = d_aad;
@@ -231,7 +244,7 @@ FinishParams finish_params(const agcm_ctx* c, int decrypt, const uint8_t iv[12],
 // scaled by H^blocks_after; the fold of the per-CTA partials runs in the last CTA of
 // the same launch.  parts_raw: per-CTA scratch (AG_MAX_CTA x 4 words); counter: its ticket.
 // ff: the tag finish fused into the same launch (single-shard message, short AAD).
-int run_stream(agcm_ctx* c, int mode, const uint8_t iv[12], uint64_t first_block, const uint8_t* d_in, uint8_t* d_out,
+int run_stream(agcm_ctx* c, int mode, const uint8_t j0[16], uint64_t first_block, const uint8_t* d_in, uint8_t* d_out,
                uint64_t n_bytes, uint64_t blocks_after, uint32_t* parts_raw, uint8_t* d_partial16, cudaStream_t st,
                uint32_t* counter, const FinishParams* ff = nullptr, uint32_t peer_epoch = 0, const uint8_t* gate = nullptr)
 {
@@ -242,9 +255,9 @@ int run_stream(agcm_ctx* c, int mode, const uint8_t iv[12], uint64_t first_block
     StreamParams p;
     memset(&p, 0, sizeof(p));
     memcpy(p.rk, c->h_rk, sizeof(p.rk));
-    iv_words(iv, p.iv);
-    p.ctr0 = (uint32_t)(c->j0ctr + 1 + first_block);   // inc32 from J0 (2 + first_block for a 96-bit IV)
-    p.j0w = __builtin_bswap32(c->j0ctr);
+    const uint32_t ctr = j0_words(j0, p.iv);
+    p.ctr0 = (uint32_t)(ctr + 1 + first_block);   // inc32 from J0 (2 + first_block for a 96-bit IV)
+    p.j0w = __builtin_bswap32(ctr);
     p.n_bytes = n_bytes;
     p.in = d_in;
     p.out = d_out;
@@ -309,7 +322,7 @@ int run_stream(agcm_ctx* c, int mode, const uint8_t iv[12], uint64_t first_block
 }
 
 // parts16: device list of n_parts partials (natural byte order), may live anywhere.
-int run_finish(agcm_ctx* c, int decrypt, const uint8_t iv[12], const uint8_t* d_parts16, int n_parts, const uint8_t* d_aad,
+int run_finish(agcm_ctx* c, int decrypt, const uint8_t j0[16], const uint8_t* d_parts16, int n_parts, const uint8_t* d_aad,
                uint64_t aad_len, uint64_t ct_len, uint8_t* d_tag, uint8_t* d_ok, cudaStream_t st)
 {
     if (n_parts < 0 || (size_t)n_parts > SC_PARTS_MAX) return AGCM_E_BAD_ARG;
@@ -325,7 +338,7 @@ int run_finish(agcm_ctx* c, int decrypt, const uint8_t iv[12], const uint8_t* d_
         // bulk AAD: same grid-wide Horner in GHASH-only mode, weighted by H^(n_ct_blocks)
         uint8_t* list = c->d_scratch + SC_PARTS;
         if (n_parts) AG_CUDA(c, cudaMemcpyAsync(list, d_parts16, 16 * (size_t)n_parts, cudaMemcpyDeviceToDevice, st));
-        int rc = run_stream(c, AG_MODE_GHASH_ONLY, iv, 0, d_aad, nullptr, aad_len, n_ct_blocks,
+        int rc = run_stream(c, AG_MODE_GHASH_ONLY, j0, 0, d_aad, nullptr, aad_len, n_ct_blocks,
                             c->d_parts + 4 * AG_MAX_CTA, list + 16 * (size_t)n_parts, st, c->d_counters);
         if (rc) return rc;
         parts = list;
@@ -336,7 +349,7 @@ int run_finish(agcm_ctx* c, int decrypt, const uint8_t iv[12], const uint8_t* d_
         int rc = ensure_pow(c, n_ct_blocks, st);
         if (rc) return rc;
     }
-    FinishParams f = finish_params(c, decrypt, iv, aad_inline, aad_len, ct_len, d_tag, d_ok, aad_inline ? c->pow_n.d : nullptr);
+    FinishParams f = finish_params(c, decrypt, j0, aad_inline, aad_len, ct_len, d_tag, d_ok, aad_inline ? c->pow_n.d : nullptr);
     f.parts = parts;
     f.n_parts = (uint32_t)np;
     AG_CUDA(c, ag_launch_finish(f, st));
@@ -345,8 +358,7 @@ int run_finish(agcm_ctx* c, int decrypt, const uint8_t iv[12], const uint8_t* d_
 }
 
 // J0 of an IV that is not 96 bits long (SP 800-38D 7.1 step 2): GHASH_H(IV || 0^(s+64) || [len(IV)]_64),
-// computed by the device (k_stream<GHASH_ONLY>) and read back; the message then runs with the
-// first 96 bits of J0 as its "IV" and J0's last 32 bits as the counter field.  Synchronises `st`.
+// computed by the device (k_stream<GHASH_ONLY>) and read back.  Synchronises `st`.
 int derive_j0(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len, uint8_t j0[16], cudaStream_t st)
 {
     if (!h_iv || iv_len == 0 || iv_len > (1ull << 32)) return AGCM_E_BAD_LEN;
@@ -359,8 +371,7 @@ int derive_j0(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len, uint8_t j0[16], c
     int rc = grow(c, c->iv_stage, padded < 4096 ? 4096 : padded);
     if (rc) return rc;
     AG_CUDA(c, cudaMemcpyAsync(c->iv_stage.p, buf.data(), padded, cudaMemcpyHostToDevice, st));
-    const uint8_t iv0[12] = {0};
-    rc = run_stream(c, AG_MODE_GHASH_ONLY, iv0, 0, c->iv_stage.p, nullptr, padded, 0, c->d_parts, c->d_scratch + SC_J0, st,
+    rc = run_stream(c, AG_MODE_GHASH_ONLY, kJ0ZeroIv, 0, c->iv_stage.p, nullptr, padded, 0, c->d_parts, c->d_scratch + SC_J0, st,
                     c->d_counters);
     if (rc) return rc;
     AG_CUDA(c, cudaMemcpyAsync(j0, c->d_scratch + SC_J0, 16, cudaMemcpyDeviceToHost, st));
@@ -372,21 +383,9 @@ int derive_j0(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len, uint8_t j0[16], c
 int resolve_j0(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len, uint8_t j0[16], cudaStream_t st)
 {
     if (iv_len != 12) return derive_j0(c, h_iv, iv_len, j0, st);
-    memcpy(j0, h_iv, 12);
-    j0[12] = j0[13] = j0[14] = 0;
-    j0[15] = 1;
+    j0_of_iv12(h_iv, j0);
     return AGCM_OK;
 }
-
-// The counter field of J0 replaces the constant 1 of the 96-bit case for the duration of a call.
-struct J0Scope {
-    agcm_ctx* c;
-    J0Scope(agcm_ctx* ctx, const uint8_t j0[16]) : c(ctx)
-    {
-        if (c && j0) c->j0ctr = ((uint32_t)j0[12] << 24) | ((uint32_t)j0[13] << 16) | ((uint32_t)j0[14] << 8) | (uint32_t)j0[15];
-    }
-    ~J0Scope() { if (c) c->j0ctr = 1; }
-};
 
 // First steps of a host-buffer call (they may allocate, so before anything is enqueued): the device, the pipeline
 // (created on first use) and room for `aad_len` bytes of AAD
@@ -748,33 +747,35 @@ int agcm_get_h(const agcm_ctx* c, uint8_t h_h16[16])
     return AGCM_OK;
 }
 
-int agcm_stream_part(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], uint64_t first_block, const uint8_t* d_in,
-                     uint8_t* d_out, uint64_t n_bytes, uint64_t blocks_after, uint8_t* d_partial16, void* stream)
+// ---- stream calls: one form per call takes J0 (agcm_*_j0, or file-local where the ABI has no _j0 form); the 96-bit IV
+// form passes it IV || 0^31 || 1, and an IV of any length goes through resolve_j0
+int agcm_stream_part_j0(agcm_ctx* c, int decrypt, const uint8_t h_j0[16], uint64_t first_block, const uint8_t* d_in,
+                        uint8_t* d_out, uint64_t n_bytes, uint64_t blocks_after, uint8_t* d_partial16, void* stream)
 {
-    if (!c || !h_iv12 || !d_partial16 || (n_bytes && (!d_in || !d_out))) return AGCM_E_BAD_ARG;
+    if (!c || !h_j0 || !d_partial16 || (n_bytes && (!d_in || !d_out))) return AGCM_E_BAD_ARG;
     if (!c->key_set) return AGCM_E_NO_KEY;
     const uint64_t nb = (n_bytes + 15) >> 4;
     if (first_block > kMaxBlocks || nb > kMaxBlocks - first_block || blocks_after > kMaxBlocks - first_block - nb)
         return AGCM_E_COUNTER_OVERFLOW;
     if (blocks_after && (n_bytes & 15)) return AGCM_E_BAD_LEN;  // only the last shard may be ragged
     AG_CUDA(c, cudaSetDevice(c->device));
-    return run_stream(c, decrypt ? AG_MODE_DEC : AG_MODE_ENC, h_iv12, first_block, d_in, d_out, n_bytes, blocks_after,
+    return run_stream(c, decrypt ? AG_MODE_DEC : AG_MODE_ENC, h_j0, first_block, d_in, d_out, n_bytes, blocks_after,
                       c->d_parts, d_partial16, (cudaStream_t)stream, c->d_counters);
 }
 
-int agcm_stream_finish(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], const uint8_t* d_partials16, int n_parts,
-                       const uint8_t* d_aad, uint64_t aad_len, uint64_t ct_len, uint8_t* d_tag, uint8_t* d_ok, void* stream)
+int agcm_stream_finish_j0(agcm_ctx* c, int decrypt, const uint8_t h_j0[16], const uint8_t* d_partials16, int n_parts,
+                          const uint8_t* d_aad, uint64_t aad_len, uint64_t ct_len, uint8_t* d_tag, uint8_t* d_ok, void* stream)
 {
-    if (!c || !h_iv12 || (n_parts && !d_partials16)) return AGCM_E_BAD_ARG;
+    if (!c || !h_j0 || (n_parts && !d_partials16)) return AGCM_E_BAD_ARG;
     if (!c->key_set) return AGCM_E_NO_KEY;
     AG_CUDA(c, cudaSetDevice(c->device));
-    return run_finish(c, decrypt, h_iv12, d_partials16, n_parts, d_aad, aad_len, ct_len, d_tag, d_ok, (cudaStream_t)stream);
+    return run_finish(c, decrypt, h_j0, d_partials16, n_parts, d_aad, aad_len, ct_len, d_tag, d_ok, (cudaStream_t)stream);
 }
 
-int agcm_stream_crypt(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], const uint8_t* d_aad, uint64_t aad_len,
-                      const uint8_t* d_in, uint8_t* d_out, uint64_t n_bytes, uint8_t* d_tag, uint8_t* d_ok, void* stream)
+static int stream_crypt(agcm_ctx* c, int decrypt, const uint8_t j0[16], const uint8_t* d_aad, uint64_t aad_len,
+                        const uint8_t* d_in, uint8_t* d_out, uint64_t n_bytes, uint8_t* d_tag, uint8_t* d_ok, void* stream)
 {
-    if (!c || !h_iv12) return AGCM_E_BAD_ARG;
+    if (!c || !j0) return AGCM_E_BAD_ARG;
     uint8_t* part = c->d_scratch + SC_PART_CT;
     if (n_bytes && aad_len <= kAadInlineMax) {
         // whole message in ONE launch: the last CTA folds the partials and finishes the tag
@@ -782,30 +783,51 @@ int agcm_stream_crypt(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], const 
         if (!d_in || !d_out || (aad_len && !d_aad) || !d_tag || (decrypt && !d_ok)) return AGCM_E_BAD_ARG;
         if (((n_bytes + 15) >> 4) > kMaxBlocks) return AGCM_E_COUNTER_OVERFLOW;
         AG_CUDA(c, cudaSetDevice(c->device));
-        const FinishParams ff = finish_params(c, decrypt, h_iv12, aad_len ? d_aad : nullptr, aad_len, n_bytes, d_tag, d_ok, c->pow_n.d);
+        const FinishParams ff = finish_params(c, decrypt, j0, aad_len ? d_aad : nullptr, aad_len, n_bytes, d_tag, d_ok, c->pow_n.d);
         if (aad_len) {
             int rc = ensure_pow(c, (n_bytes + 15) >> 4, (cudaStream_t)stream);
             if (rc) return rc;
         }
-        return run_stream(c, decrypt ? AG_MODE_DEC : AG_MODE_ENC, h_iv12, 0, d_in, d_out, n_bytes, 0, c->d_parts, nullptr,
+        return run_stream(c, decrypt ? AG_MODE_DEC : AG_MODE_ENC, j0, 0, d_in, d_out, n_bytes, 0, c->d_parts, nullptr,
                           (cudaStream_t)stream, c->d_counters, &ff);
     }
-    int rc = agcm_stream_part(c, decrypt, h_iv12, 0, d_in, d_out, n_bytes, 0, part, stream);
+    int rc = agcm_stream_part_j0(c, decrypt, j0, 0, d_in, d_out, n_bytes, 0, part, stream);
     if (rc) return rc;
-    return agcm_stream_finish(c, decrypt, h_iv12, part, 1, d_aad, aad_len, n_bytes, d_tag, d_ok, stream);
+    return agcm_stream_finish_j0(c, decrypt, j0, part, 1, d_aad, aad_len, n_bytes, d_tag, d_ok, stream);
+}
+
+int agcm_stream_part(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], uint64_t first_block, const uint8_t* d_in,
+                     uint8_t* d_out, uint64_t n_bytes, uint64_t blocks_after, uint8_t* d_partial16, void* stream)
+{
+    uint8_t j0[16];
+    return agcm_stream_part_j0(c, decrypt, j0_of_iv12(h_iv12, j0), first_block, d_in, d_out, n_bytes, blocks_after, d_partial16,
+                               stream);
+}
+
+int agcm_stream_finish(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], const uint8_t* d_partials16, int n_parts,
+                       const uint8_t* d_aad, uint64_t aad_len, uint64_t ct_len, uint8_t* d_tag, uint8_t* d_ok, void* stream)
+{
+    uint8_t j0[16];
+    return agcm_stream_finish_j0(c, decrypt, j0_of_iv12(h_iv12, j0), d_partials16, n_parts, d_aad, aad_len, ct_len, d_tag, d_ok,
+                                 stream);
+}
+
+int agcm_stream_crypt(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], const uint8_t* d_aad, uint64_t aad_len,
+                      const uint8_t* d_in, uint8_t* d_out, uint64_t n_bytes, uint8_t* d_tag, uint8_t* d_ok, void* stream)
+{
+    uint8_t j0[16];
+    return stream_crypt(c, decrypt, j0_of_iv12(h_iv12, j0), d_aad, aad_len, d_in, d_out, n_bytes, d_tag, d_ok, stream);
 }
 
 int agcm_stream_crypt_iv(agcm_ctx* c, int decrypt, const uint8_t* h_iv, size_t iv_len, const uint8_t* d_aad, uint64_t aad_len,
                          const uint8_t* d_in, uint8_t* d_out, uint64_t n_bytes, uint8_t* d_tag, uint8_t* d_ok, void* stream)
 {
     if (!c || !h_iv) return AGCM_E_BAD_ARG;
-    if (iv_len == 12) return agcm_stream_crypt(c, decrypt, h_iv, d_aad, aad_len, d_in, d_out, n_bytes, d_tag, d_ok, stream);
-    AG_CUDA(c, cudaSetDevice(c->device));
+    if (iv_len != 12) AG_CUDA(c, cudaSetDevice(c->device));
     uint8_t j0[16];
     int rc = resolve_j0(c, h_iv, iv_len, j0, (cudaStream_t)stream);
     if (rc) return rc;
-    J0Scope scope(c, j0);
-    return agcm_stream_crypt(c, decrypt, j0, d_aad, aad_len, d_in, d_out, n_bytes, d_tag, d_ok, stream);
+    return stream_crypt(c, decrypt, j0, d_aad, aad_len, d_in, d_out, n_bytes, d_tag, d_ok, stream);
 }
 
 int agcm_peer_setup(agcm_ctx* c, int rank, int world, const uint64_t* h_peer_ptrs)
@@ -886,14 +908,14 @@ static int peer_begin(agcm_ctx* c, uint64_t first_block, uint64_t n_bytes, uint6
 }
 
 // The one-warp finish of `epoch` on the side stream, ordered after everything queued on `st`.
-static int peer_finish(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], const uint8_t* d_aad, uint64_t aad_len,
+static int peer_finish(agcm_ctx* c, int decrypt, const uint8_t j0[16], const uint8_t* d_aad, uint64_t aad_len,
                        uint64_t total_len, uint8_t* d_tag, uint8_t* d_ok, cudaStream_t st, uint32_t epoch, bool deferred)
 {
     const uint32_t slot = epoch % AG_PEER_RING;
     c->peer_epoch = epoch;
     PeerFinishParams pf;
     memset(&pf, 0, sizeof(pf));
-    pf.f = finish_params(c, decrypt, h_iv12, aad_len ? d_aad : nullptr, aad_len, total_len, d_tag, d_ok,
+    pf.f = finish_params(c, decrypt, j0, aad_len ? d_aad : nullptr, aad_len, total_len, d_tag, d_ok,
                          aad_len ? c->pow_n.d : nullptr);
     pf.peer_bufs = c->d_peer_bufs;
     pf.rank = (uint32_t)c->peer_rank;
@@ -914,40 +936,53 @@ static int peer_finish(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], const
     return AGCM_OK;
 }
 
-// This rank's bulk kernel of exchange `epoch` (ENC, DEC or GHASH_ONLY); its last CTA posts the scaled partial to every rank.
-static int peer_bulk(agcm_ctx* c, int mode, const uint8_t h_iv12[12], uint64_t first_block, const uint8_t* d_in, uint8_t* d_out,
-                     uint64_t n_bytes, uint64_t blocks_after, cudaStream_t st, uint32_t epoch)
+// Post this rank's partial of exchange `epoch` to every rank: the xor of the first n_chunks chunk partials of a host
+// pipeline (each already scaled), or the zero partial of an empty counter range (fewer blocks than ranks) when n_chunks = 0.
+static int peer_post(agcm_ctx* c, uint64_t n_chunks, uint32_t epoch, cudaStream_t st)
 {
-    if (n_bytes)
-        return run_stream(c, mode, h_iv12, first_block, d_in, d_out, n_bytes, blocks_after, c->d_parts, nullptr, st, c->d_counters,
-                          nullptr, epoch);
-    // an empty counter range (fewer blocks than ranks) still posts its zero partial
-    AG_CUDA(c, ag_launch_peer_post(c->d_peer_bufs, (uint32_t)c->peer_rank, (uint32_t)c->peer_world, epoch, nullptr, st));
+    const uint8_t* d_p = nullptr;   // null = the zero partial
+    if (n_chunks) {
+        AG_CUDA(c, ag_launch_xor_parts(c->d_chunk_partials, (uint32_t)n_chunks, c->d_scratch + SC_PART_CT, st));
+        c->launches++;
+        d_p = c->d_scratch + SC_PART_CT;
+    }
+    AG_CUDA(c, ag_launch_peer_post(c->d_peer_bufs, (uint32_t)c->peer_rank, (uint32_t)c->peer_world, epoch, d_p, st));
     c->launches++;
     return AGCM_OK;
 }
 
-static int stream_crypt_peer(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], uint64_t first_block, const uint8_t* d_in,
-                             uint8_t* d_out, uint64_t n_bytes, uint64_t blocks_after, const uint8_t* d_aad, uint64_t aad_len,
-                             uint64_t total_len, uint8_t* d_tag, uint8_t* d_ok, void* stream, bool deferred)
+// This rank's bulk kernel of exchange `epoch` (ENC, DEC or GHASH_ONLY); its last CTA posts the scaled partial to every rank.
+static int peer_bulk(agcm_ctx* c, int mode, const uint8_t j0[16], uint64_t first_block, const uint8_t* d_in, uint8_t* d_out,
+                     uint64_t n_bytes, uint64_t blocks_after, cudaStream_t st, uint32_t epoch)
 {
-    if (!c || !h_iv12 || (n_bytes && (!d_in || !d_out)) || !d_tag || (decrypt && !d_ok) || (aad_len && !d_aad))
+    if (n_bytes)
+        return run_stream(c, mode, j0, first_block, d_in, d_out, n_bytes, blocks_after, c->d_parts, nullptr, st, c->d_counters,
+                          nullptr, epoch);
+    return peer_post(c, 0, epoch, st);
+}
+
+int agcm_stream_crypt_peer_j0(agcm_ctx* c, int decrypt, const uint8_t h_j0[16], uint64_t first_block, const uint8_t* d_in,
+                              uint8_t* d_out, uint64_t n_bytes, uint64_t blocks_after, const uint8_t* d_aad, uint64_t aad_len,
+                              uint64_t total_len, uint8_t* d_tag, uint8_t* d_ok, void* stream, int deferred)
+{
+    if (!c || !h_j0 || (n_bytes && (!d_in || !d_out)) || !d_tag || (decrypt && !d_ok) || (aad_len && !d_aad))
         return AGCM_E_BAD_ARG;
     cudaStream_t st = (cudaStream_t)stream;
     uint32_t epoch = 0;
     int rc = peer_begin(c, first_block, n_bytes, blocks_after, aad_len, total_len, st, &epoch);
     if (rc) return rc;
-    rc = peer_bulk(c, decrypt ? AG_MODE_DEC : AG_MODE_ENC, h_iv12, first_block, d_in, d_out, n_bytes, blocks_after, st, epoch);
+    rc = peer_bulk(c, decrypt ? AG_MODE_DEC : AG_MODE_ENC, h_j0, first_block, d_in, d_out, n_bytes, blocks_after, st, epoch);
     if (rc) return rc;
-    return peer_finish(c, decrypt, h_iv12, d_aad, aad_len, total_len, d_tag, d_ok, st, epoch, deferred);
+    return peer_finish(c, decrypt, h_j0, d_aad, aad_len, total_len, d_tag, d_ok, st, epoch, deferred != 0);
 }
 
 int agcm_stream_crypt_peer(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], uint64_t first_block, const uint8_t* d_in,
                            uint8_t* d_out, uint64_t n_bytes, uint64_t blocks_after, const uint8_t* d_aad, uint64_t aad_len,
                            uint64_t total_len, uint8_t* d_tag, uint8_t* d_ok, void* stream)
 {
-    return stream_crypt_peer(c, decrypt, h_iv12, first_block, d_in, d_out, n_bytes, blocks_after, d_aad, aad_len, total_len,
-                             d_tag, d_ok, stream, false);
+    uint8_t j0[16];
+    return agcm_stream_crypt_peer_j0(c, decrypt, j0_of_iv12(h_iv12, j0), first_block, d_in, d_out, n_bytes, blocks_after, d_aad,
+                                     aad_len, total_len, d_tag, d_ok, stream, 0);
 }
 
 int agcm_stream_crypt_peer_async(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], uint64_t first_block,
@@ -955,51 +990,18 @@ int agcm_stream_crypt_peer_async(agcm_ctx* c, int decrypt, const uint8_t h_iv12[
                                  const uint8_t* d_aad, uint64_t aad_len, uint64_t total_len, uint8_t* d_tag, uint8_t* d_ok,
                                  void* stream)
 {
-    return stream_crypt_peer(c, decrypt, h_iv12, first_block, d_in, d_out, n_bytes, blocks_after, d_aad, aad_len, total_len,
-                             d_tag, d_ok, stream, true);
+    uint8_t j0[16];
+    return agcm_stream_crypt_peer_j0(c, decrypt, j0_of_iv12(h_iv12, j0), first_block, d_in, d_out, n_bytes, blocks_after, d_aad,
+                                     aad_len, total_len, d_tag, d_ok, stream, 1);
 }
 
 // ---- IVs of any length on the shard / peer / gctr entry points: the caller derives J0 once
-// (agcm_derive_j0) and passes it instead of the 12 IV bytes (J0Scope).
+// (agcm_derive_j0) and passes it instead of the 12 IV bytes.
 int agcm_derive_j0(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len, uint8_t h_j0[16])
 {
     if (!c || !h_iv || !h_j0) return AGCM_E_BAD_ARG;
     if (iv_len != 12) AG_CUDA(c, cudaSetDevice(c->device));
     return resolve_j0(c, h_iv, iv_len, h_j0, nullptr);   // the legacy stream: this call takes none
-}
-
-int agcm_gctr_j0(agcm_ctx* c, const uint8_t h_j0[16], uint64_t first_block, const uint8_t* d_in, uint8_t* d_out,
-                 uint64_t n_bytes, void* stream)
-{
-    if (!c || !h_j0) return AGCM_E_BAD_ARG;
-    J0Scope scope(c, h_j0);
-    return agcm_gctr(c, h_j0, first_block, d_in, d_out, n_bytes, stream);
-}
-
-int agcm_stream_part_j0(agcm_ctx* c, int decrypt, const uint8_t h_j0[16], uint64_t first_block, const uint8_t* d_in,
-                        uint8_t* d_out, uint64_t n_bytes, uint64_t blocks_after, uint8_t* d_partial16, void* stream)
-{
-    if (!c || !h_j0) return AGCM_E_BAD_ARG;
-    J0Scope scope(c, h_j0);
-    return agcm_stream_part(c, decrypt, h_j0, first_block, d_in, d_out, n_bytes, blocks_after, d_partial16, stream);
-}
-
-int agcm_stream_finish_j0(agcm_ctx* c, int decrypt, const uint8_t h_j0[16], const uint8_t* d_partials16, int n_parts,
-                          const uint8_t* d_aad, uint64_t aad_len, uint64_t ct_len, uint8_t* d_tag, uint8_t* d_ok, void* stream)
-{
-    if (!c || !h_j0) return AGCM_E_BAD_ARG;
-    J0Scope scope(c, h_j0);
-    return agcm_stream_finish(c, decrypt, h_j0, d_partials16, n_parts, d_aad, aad_len, ct_len, d_tag, d_ok, stream);
-}
-
-int agcm_stream_crypt_peer_j0(agcm_ctx* c, int decrypt, const uint8_t h_j0[16], uint64_t first_block, const uint8_t* d_in,
-                              uint8_t* d_out, uint64_t n_bytes, uint64_t blocks_after, const uint8_t* d_aad, uint64_t aad_len,
-                              uint64_t total_len, uint8_t* d_tag, uint8_t* d_ok, void* stream, int deferred)
-{
-    if (!c || !h_j0) return AGCM_E_BAD_ARG;
-    J0Scope scope(c, h_j0);
-    return stream_crypt_peer(c, decrypt, h_j0, first_block, d_in, d_out, n_bytes, blocks_after, d_aad, aad_len, total_len, d_tag,
-                             d_ok, stream, deferred != 0);
 }
 
 int agcm_stream_decrypt_verified(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len, const uint8_t* d_aad, uint64_t aad_len,
@@ -1014,7 +1016,6 @@ int agcm_stream_decrypt_verified(agcm_ctx* c, const uint8_t* h_iv, size_t iv_len
     uint8_t j0[16];
     int rc = resolve_j0(c, h_iv, iv_len, j0, st);   // on `st`: the caller's earlier work there may use the same scratch
     if (rc) return rc;
-    J0Scope scope(c, j0);
     // pass 1: GHASH over the ciphertext only (about 4x the rate of the fused pass), then the tag check
     uint8_t* part = c->d_scratch + SC_PART_CT;
     rc = run_stream(c, AG_MODE_GHASH_ONLY, j0, 0, d_ct, nullptr, n_bytes, 0, c->d_parts, part, st, c->d_counters);
@@ -1038,7 +1039,6 @@ int agcm_stream_decrypt_verified_peer(agcm_ctx* c, const uint8_t* h_iv, size_t i
     uint8_t j0[16];
     rc = resolve_j0(c, h_iv, iv_len, j0, st);
     if (rc) return rc;
-    J0Scope scope(c, j0);
     // pass 1: GHASH over this rank's ciphertext, partial posted; the finish checks the WORLD's tag into d_ok
     rc = peer_bulk(c, AG_MODE_GHASH_ONLY, j0, first_block, d_ct, nullptr, n_bytes, blocks_after, st, epoch);
     if (rc) return rc;
@@ -1049,16 +1049,23 @@ int agcm_stream_decrypt_verified_peer(agcm_ctx* c, const uint8_t* h_iv, size_t i
                       nullptr, 0, d_ok);
 }
 
-int agcm_gctr(agcm_ctx* c, const uint8_t h_iv12[12], uint64_t first_block, const uint8_t* d_in, uint8_t* d_out,
-              uint64_t n_bytes, void* stream)
+int agcm_gctr_j0(agcm_ctx* c, const uint8_t h_j0[16], uint64_t first_block, const uint8_t* d_in, uint8_t* d_out,
+                 uint64_t n_bytes, void* stream)
 {
-    if (!c || !h_iv12 || (n_bytes && (!d_in || !d_out))) return AGCM_E_BAD_ARG;
+    if (!c || !h_j0 || (n_bytes && (!d_in || !d_out))) return AGCM_E_BAD_ARG;
     if (!c->key_set) return AGCM_E_NO_KEY;
     const uint64_t nb = (n_bytes + 15) >> 4;
     if (first_block > kMaxBlocks || nb > kMaxBlocks - first_block) return AGCM_E_COUNTER_OVERFLOW;
     AG_CUDA(c, cudaSetDevice(c->device));
-    return run_stream(c, AG_MODE_CTR_ONLY, h_iv12, first_block, d_in, d_out, n_bytes, 0, c->d_parts, nullptr,
+    return run_stream(c, AG_MODE_CTR_ONLY, h_j0, first_block, d_in, d_out, n_bytes, 0, c->d_parts, nullptr,
                       (cudaStream_t)stream, c->d_counters);
+}
+
+int agcm_gctr(agcm_ctx* c, const uint8_t h_iv12[12], uint64_t first_block, const uint8_t* d_in, uint8_t* d_out,
+              uint64_t n_bytes, void* stream)
+{
+    uint8_t j0[16];
+    return agcm_gctr_j0(c, j0_of_iv12(h_iv12, j0), first_block, d_in, d_out, n_bytes, stream);
 }
 
 int agcm_ghash(agcm_ctx* c, const uint8_t* d_in, uint64_t n_bytes, uint8_t* d_y16, void* stream)
@@ -1066,8 +1073,7 @@ int agcm_ghash(agcm_ctx* c, const uint8_t* d_in, uint64_t n_bytes, uint8_t* d_y1
     if (!c || !d_y16 || (n_bytes && !d_in)) return AGCM_E_BAD_ARG;
     if (!c->key_set) return AGCM_E_NO_KEY;
     AG_CUDA(c, cudaSetDevice(c->device));
-    const uint8_t iv0[12] = {0};
-    return run_stream(c, AG_MODE_GHASH_ONLY, iv0, 0, d_in, nullptr, n_bytes, 0, c->d_parts, d_y16, (cudaStream_t)stream,
+    return run_stream(c, AG_MODE_GHASH_ONLY, kJ0ZeroIv, 0, d_in, nullptr, n_bytes, 0, c->d_parts, d_y16, (cudaStream_t)stream,
                       c->d_counters);
 }
 
@@ -1096,9 +1102,10 @@ static int batch_bind_key(agcm_ctx* c, int decrypt, BatchParams& p, size_t n_msg
 }
 
 // decrypt == AG_DECRYPT_VERIFIED: pass 1 of the verify-then-release decrypt -- the tag-only flavour of the lane-group /
-// warp-unit kernels
+// warp-unit kernels.  own_ticket: false when other calls on this context may run at the same time on other streams (the
+// context has one ticket word); the CTA layout then assigns its units statically.
 static int batch_common(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len, BatchParams& p, size_t n_msgs, void* stream,
-                        bool aligned16 = true)
+                        bool aligned16 = true, bool own_ticket = true)
 {
     if (!c->key_set) return AGCM_E_NO_KEY;
     if (n_msgs == 0) return AGCM_OK;
@@ -1161,7 +1168,7 @@ static int batch_common(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len, B
             p.seg_parts = c->seg_parts.p;
         }
         const int ncta_m = (int)(n_units < (uint64_t)c->ncta ? n_units : (uint64_t)c->ncta);
-        if (n_units > (uint64_t)ncta_m && n_units < 0xFFFFFFFFull && !c->no_ticket) {   // more units than CTAs: hand them out dynamically
+        if (n_units > (uint64_t)ncta_m && n_units < 0xFFFFFFFFull && own_ticket) {   // more units than CTAs: hand them out dynamically
             rc = zeroed_ticket(c, 1, (cudaStream_t)stream, p.ticket);
             if (rc) return rc;
         }
@@ -1173,7 +1180,7 @@ static int batch_common(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len, B
     const uint64_t groups_per_cta = (uint64_t)c->nt / g;
     uint64_t need = (n_msgs + groups_per_cta - 1) / groups_per_cta;
     int ncta = (int)(need < (uint64_t)c->ncta ? need : (uint64_t)c->ncta);
-    if (ragged && n_msgs >= 1024 && n_msgs < 0xFFFFFF00ull && !c->no_ticket && !getenv("AGCM_NO_LEN_SORT")) {
+    if (ragged && n_msgs >= 1024 && n_msgs < 0xFFFFFF00ull && !getenv("AGCM_NO_LEN_SORT")) {
         // Messages of different lengths: take them longest first, so that the 32/G messages a warp works on in
         // lock step are equally long (3 small launches; the kernels then follow perm[]), warp by warp by ticket.
         // With lanes = 0 the order is cut into three length classes, one launch each: 32 lanes per message from
@@ -1341,7 +1348,7 @@ static int batch_tile(agcm_ctx* c, int decrypt, BatchParams& p, size_t n_msgs, c
 static bool tile_slots_eligible(const agcm_ctx* c, int lanes, const BatchParams& p, size_t n_msgs)
 {
     if (lanes != 0 && lanes != 2048) return false;
-    if (!p.len_arr || p.stride == 0 || p.stride >= (1ull << 31) || n_msgs >= (1ull << 30) || c->no_ticket) return false;
+    if (!p.len_arr || p.stride == 0 || p.stride >= (1ull << 31) || n_msgs >= (1ull << 30)) return false;
     if ((((uintptr_t)p.in | (uintptr_t)p.out) & 15) || (p.stride & 15)) return false;
     if (lanes == 2048) return true;   // asked for by name
     // Not a default: measured against the lane-group classes on 2^20 messages (profiles/r2_ragged.md) it is within
@@ -1440,7 +1447,7 @@ static int batch_offsets(agcm_ctx* c, bool decrypt, int lanes, uint64_t avg_len_
 
 static int batch_uniform(agcm_ctx* c, bool decrypt, int lanes, const uint8_t* d_iv, int iv_is_j0, const uint8_t* d_aad,
                          uint64_t aad_len, uint64_t aad_stride, const uint8_t* d_in, uint8_t* d_out, uint64_t len,
-                         uint64_t stride, uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
+                         uint64_t stride, uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream, bool own_ticket)
 {
     if (!c) return AGCM_E_BAD_ARG;
     BatchParams p;
@@ -1450,7 +1457,7 @@ static int batch_uniform(agcm_ctx* c, bool decrypt, int lanes, const uint8_t* d_
     if (lanes == 2048 && !tile_eligible(c, lanes, p, n_msgs)) return AGCM_E_BAD_ARG;
     if (n_msgs && tile_eligible(c, lanes, p, n_msgs)) return batch_tile(c, decrypt, p, n_msgs, (cudaStream_t)stream);
     // work estimate for the layout choice: an AAD block costs about a quarter of a payload block (no AES)
-    return batch_common(c, decrypt, lanes, len + (d_aad ? aad_len / 4 : 0), p, n_msgs, stream, aligned16);
+    return batch_common(c, decrypt, lanes, len + (d_aad ? aad_len / 4 : 0), p, n_msgs, stream, aligned16, own_ticket);
 }
 
 int agcm_batch_crypt(agcm_ctx* c, int decrypt, int lanes, uint64_t avg_len_hint, const uint8_t* d_iv12,
@@ -1474,7 +1481,7 @@ int agcm_batch_crypt_uniform(agcm_ctx* c, int decrypt, int lanes, const uint8_t*
                              uint64_t stride, uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
 {
     return batch_uniform(c, decrypt, lanes, d_iv12, 0, d_aad, aad_len, aad_stride, d_in, d_out, len, stride, d_tag, d_ok, n_msgs,
-                         stream);
+                         stream, true);
 }
 
 int agcm_batch_crypt_uniform_j0(agcm_ctx* c, int decrypt, int lanes, const uint8_t* d_j0, const uint8_t* d_aad,
@@ -1482,7 +1489,7 @@ int agcm_batch_crypt_uniform_j0(agcm_ctx* c, int decrypt, int lanes, const uint8
                                 uint64_t stride, uint8_t* d_tag, uint8_t* d_ok, size_t n_msgs, void* stream)
 {
     return batch_uniform(c, decrypt, lanes, d_j0, 1, d_aad, aad_len, aad_stride, d_in, d_out, len, stride, d_tag, d_ok, n_msgs,
-                         stream);
+                         stream, true);
 }
 
 // Checks and BatchParams of a slots batch (message i: d_len[i] bytes at i * stride)
@@ -1628,7 +1635,7 @@ static int perkey_common(agcm_ctx* c, int mode, int decrypt, BatchParams& p, siz
         if (rc) return rc;
         return tile_launch(c, t, nr, decrypt, 0, st);
     }
-    if ((p.in_off || p.aad_off) && n_msgs >= 1024 && n_msgs < 0xFFFFFF00ull && !c->no_ticket && !getenv("AGCM_NO_LEN_SORT")) {
+    if ((p.in_off || p.aad_off) && n_msgs >= 1024 && n_msgs < 0xFFFFFF00ull && !getenv("AGCM_NO_LEN_SORT")) {
         // messages of different lengths, a message per lane: take them in length order (as batch_common does), so that
         // the 32 messages of a warp are equally long; thread g then works on perm[g], perm[g + grid], ...
         int rc = len_sort(c, p, n_msgs, st);
@@ -1717,7 +1724,7 @@ static uint64_t pick_chunk(const agcm_ctx* c, uint64_t n_bytes)
 // chunked H2D -> fused kernel -> D2H of one counter range; the per-chunk partials
 // (each scaled for everything after it, including `blocks_after0`) land in
 // c->d_chunk_partials[0..n_chunks).  Waits for slots 1..kSlots-1 and leaves hs[0] running.
-static int host_pipeline(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], uint64_t first_block0, const uint8_t* h_in,
+static int host_pipeline(agcm_ctx* c, int decrypt, const uint8_t j0[16], uint64_t first_block0, const uint8_t* h_in,
                          uint8_t* h_out, uint64_t n_bytes, uint64_t blocks_after0, uint64_t* n_chunks_out)
 {
     const uint64_t nblocks = (n_bytes + 15) >> 4;
@@ -1736,7 +1743,7 @@ static int host_pipeline(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], uin
         const uint64_t fb = off >> 4;
         const uint64_t after = nblocks - fb - ((nb + 15) >> 4) + blocks_after0;
         AG_CUDA(c, cudaMemcpyAsync(c->d_stage[s], h_in + off, nb, cudaMemcpyHostToDevice, st));
-        int rc = run_stream(c, mode, h_iv12, first_block0 + fb, c->d_stage[s], c->d_stage[s], nb,
+        int rc = run_stream(c, mode, j0, first_block0 + fb, c->d_stage[s], c->d_stage[s], nb,
                             after, c->d_stage_parts[s], c->d_chunk_partials + 16 * k, st, c->d_counters + 1 + s);
         if (rc) return rc;
         AG_CUDA(c, cudaMemcpyAsync(h_out + off, c->d_stage[s], nb, cudaMemcpyDeviceToHost, st));
@@ -1758,8 +1765,9 @@ int agcm_stream_part_host(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], ui
     if (blocks_after && (n_bytes & 15)) return AGCM_E_BAD_LEN;
     int rc = host_begin(c, 0);
     if (rc) return rc;
+    uint8_t j0[16];
     uint64_t n_chunks = 0;
-    rc = host_pipeline(c, decrypt, h_iv12, first_block, h_in, h_out, n_bytes, blocks_after, &n_chunks);
+    rc = host_pipeline(c, decrypt, j0_of_iv12(h_iv12, j0), first_block, h_in, h_out, n_bytes, blocks_after, &n_chunks);
     if (rc) return rc;
     // xor of the chunk partials = this range's partial (exponent 0: already scaled)
     uint8_t* d_p = c->d_scratch + SC_PART_CT;
@@ -1789,7 +1797,9 @@ int agcm_stream_finish_host(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], 
     uint8_t* d_tag = c->d_scratch + SC_TAG;
     uint8_t* d_ok = c->d_scratch + SC_OK;
     if (decrypt) AG_CUDA(c, cudaMemcpyAsync(d_tag, h_tag, 16, cudaMemcpyHostToDevice, st));
-    rc = run_finish(c, decrypt, h_iv12, c->d_chunk_partials, n_parts, c->aad_stage.p, aad_len, ct_len, d_tag, d_ok, st);
+    uint8_t j0[16];
+    rc = run_finish(c, decrypt, j0_of_iv12(h_iv12, j0), c->d_chunk_partials, n_parts, c->aad_stage.p, aad_len, ct_len, d_tag,
+                    d_ok, st);
     if (rc) return rc;
     return host_end(c, decrypt, h_tag, h_ok, st);
 }
@@ -1811,18 +1821,14 @@ int agcm_stream_crypt_peer_host(agcm_ctx* c, int decrypt, const uint8_t h_iv12[1
     uint8_t* d_tag = c->d_scratch + SC_TAG;
     uint8_t* d_ok = c->d_scratch + SC_OK;
     if (decrypt) AG_CUDA(c, cudaMemcpyAsync(d_tag, h_tag, 16, cudaMemcpyHostToDevice, st));
+    uint8_t j0[16];
+    j0_of_iv12(h_iv12, j0);
     uint64_t n_chunks = 0;
-    rc = host_pipeline(c, decrypt, h_iv12, first_block, h_in, h_out, n_bytes, blocks_after, &n_chunks);
+    rc = host_pipeline(c, decrypt, j0, first_block, h_in, h_out, n_bytes, blocks_after, &n_chunks);
     if (rc) return rc;
-    const uint8_t* d_p = nullptr;   // null = the zero partial of an empty range
-    if (n_chunks) {
-        AG_CUDA(c, ag_launch_xor_parts(c->d_chunk_partials, (uint32_t)n_chunks, c->d_scratch + SC_PART_CT, st));
-        c->launches++;
-        d_p = c->d_scratch + SC_PART_CT;
-    }
-    AG_CUDA(c, ag_launch_peer_post(c->d_peer_bufs, (uint32_t)c->peer_rank, (uint32_t)c->peer_world, epoch, d_p, st));
-    c->launches++;
-    rc = peer_finish(c, decrypt, h_iv12, c->aad_stage.p, aad_len, total_len, d_tag, d_ok, st, epoch, false);
+    rc = peer_post(c, n_chunks, epoch, st);
+    if (rc) return rc;
+    rc = peer_finish(c, decrypt, j0, c->aad_stage.p, aad_len, total_len, d_tag, d_ok, st, epoch, false);
     if (rc) return rc;
     rc = host_end(c, decrypt, h_tag, h_ok, st);
     if (rc) return rc;
@@ -1830,10 +1836,10 @@ int agcm_stream_crypt_peer_host(agcm_ctx* c, int decrypt, const uint8_t h_iv12[1
     return AGCM_OK;
 }
 
-int agcm_stream_crypt_host(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], const uint8_t* h_aad, uint64_t aad_len,
-                           const uint8_t* h_in, uint8_t* h_out, uint64_t n_bytes, uint8_t h_tag[16], int* h_ok)
+static int stream_crypt_host(agcm_ctx* c, int decrypt, const uint8_t j0[16], const uint8_t* h_aad, uint64_t aad_len,
+                             const uint8_t* h_in, uint8_t* h_out, uint64_t n_bytes, uint8_t h_tag[16], int* h_ok)
 {
-    if (!c || !h_iv12 || !h_tag || (n_bytes && (!h_in || !h_out)) || (aad_len && !h_aad) || (decrypt && !h_ok))
+    if (!c || !j0 || !h_tag || (n_bytes && (!h_in || !h_out)) || (aad_len && !h_aad) || (decrypt && !h_ok))
         return AGCM_E_BAD_ARG;
     if (!c->key_set) return AGCM_E_NO_KEY;
     if (((n_bytes + 15) >> 4) > kMaxBlocks) return AGCM_E_COUNTER_OVERFLOW;
@@ -1849,26 +1855,32 @@ int agcm_stream_crypt_host(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], c
         cudaStream_t st = c->hs[0];
         AG_CUDA(c, cudaMemcpyAsync(c->d_stage[0], h_in, n_bytes, cudaMemcpyHostToDevice, st));
         if (decrypt) AG_CUDA(c, cudaMemcpyAsync(d_tag, h_tag, 16, cudaMemcpyHostToDevice, st));
-        rc = agcm_stream_crypt(c, decrypt, h_iv12, c->aad_stage.p, aad_len, c->d_stage[0], c->d_stage[0], n_bytes, d_tag, d_ok,
-                               st);
+        rc = stream_crypt(c, decrypt, j0, c->aad_stage.p, aad_len, c->d_stage[0], c->d_stage[0], n_bytes, d_tag, d_ok, st);
         if (rc) return rc;
         AG_CUDA(c, cudaMemcpyAsync(h_out, c->d_stage[0], n_bytes, cudaMemcpyDeviceToHost, st));
     } else {
         uint64_t n_chunks = 0;
-        rc = host_pipeline(c, decrypt, h_iv12, 0, h_in, h_out, n_bytes, 0, &n_chunks);
+        rc = host_pipeline(c, decrypt, j0, 0, h_in, h_out, n_bytes, 0, &n_chunks);
         if (rc) return rc;
         if (decrypt) AG_CUDA(c, cudaMemcpyAsync(d_tag, h_tag, 16, cudaMemcpyHostToDevice, c->hs[0]));
-        rc = run_finish(c, decrypt, h_iv12, c->d_chunk_partials, (int)n_chunks, c->aad_stage.p, aad_len, n_bytes, d_tag, d_ok,
+        rc = run_finish(c, decrypt, j0, c->d_chunk_partials, (int)n_chunks, c->aad_stage.p, aad_len, n_bytes, d_tag, d_ok,
                         c->hs[0]);
         if (rc) return rc;
     }
     return host_end(c, decrypt, h_tag, h_ok, c->hs[0]);
 }
 
+int agcm_stream_crypt_host(agcm_ctx* c, int decrypt, const uint8_t h_iv12[12], const uint8_t* h_aad, uint64_t aad_len,
+                           const uint8_t* h_in, uint8_t* h_out, uint64_t n_bytes, uint8_t h_tag[16], int* h_ok)
+{
+    uint8_t j0[16];
+    return stream_crypt_host(c, decrypt, j0_of_iv12(h_iv12, j0), h_aad, aad_len, h_in, h_out, n_bytes, h_tag, h_ok);
+}
+
 // Pass 1 of a verify-then-release host decrypt: the ciphertext is copied into c->verify, where it stays for pass 2, and
 // absorbed chunk by chunk (the copy of chunk k+1 overlaps the GHASH of chunk k).  The chunk partials, each scaled for
 // every block after it (`blocks_after` more past the range), land in c->d_chunk_partials.  Waits for slots 1..kSlots-1.
-static int verify_absorb_host(agcm_ctx* c, const uint8_t j0[12], const uint8_t* h_ct, uint64_t n_bytes, uint64_t chunk,
+static int verify_absorb_host(agcm_ctx* c, const uint8_t j0[16], const uint8_t* h_ct, uint64_t n_bytes, uint64_t chunk,
                               uint64_t blocks_after)
 {
     const uint64_t nblocks = (n_bytes + 15) >> 4;
@@ -1887,7 +1899,7 @@ static int verify_absorb_host(agcm_ctx* c, const uint8_t j0[12], const uint8_t* 
 
 // Pass 2, run only once the tag matched: GCTR in place over c->verify from counter block `first_block`, chunk by chunk,
 // copied out to h_pt.  Waits for every slot.
-static int verify_release_host(agcm_ctx* c, const uint8_t j0[12], uint64_t first_block, uint8_t* h_pt, uint64_t n_bytes,
+static int verify_release_host(agcm_ctx* c, const uint8_t j0[16], uint64_t first_block, uint8_t* h_pt, uint64_t n_bytes,
                                uint64_t chunk)
 {
     for (uint64_t k = 0, off = 0; off < n_bytes; ++k, off += chunk) {
@@ -1915,7 +1927,6 @@ int agcm_stream_decrypt_verified_host(agcm_ctx* c, const uint8_t* h_iv, size_t i
     uint8_t j0[16];
     rc = resolve_j0(c, h_iv, iv_len, j0, c->hs[0]);
     if (rc) return rc;
-    J0Scope scope(c, j0);
     const uint64_t chunk = pick_chunk(c, n_bytes);
     const uint64_t n_chunks = (n_bytes + chunk - 1) / chunk;
     if (n_chunks > SC_PARTS_MAX) return AGCM_E_BAD_LEN;
@@ -1953,21 +1964,14 @@ int agcm_stream_decrypt_verified_peer_host(agcm_ctx* c, const uint8_t* h_iv, siz
     uint8_t j0[16];
     rc = resolve_j0(c, h_iv, iv_len, j0, st);
     if (rc) return rc;
-    J0Scope scope(c, j0);
     if (aad_len) AG_CUDA(c, cudaMemcpyAsync(c->aad_stage.p, h_aad, aad_len, cudaMemcpyHostToDevice, st));
     rc = verify_absorb_host(c, j0, h_ct, n_bytes, chunk, blocks_after);
     if (rc) return rc;
     uint8_t* d_tag = c->d_scratch + SC_TAG;
     uint8_t* d_ok = c->d_scratch + SC_OK;
     AG_CUDA(c, cudaMemcpyAsync(d_tag, h_tag, 16, cudaMemcpyHostToDevice, st));
-    const uint8_t* d_p = nullptr;   // null = the zero partial of an empty range
-    if (n_chunks) {
-        AG_CUDA(c, ag_launch_xor_parts(c->d_chunk_partials, (uint32_t)n_chunks, c->d_scratch + SC_PART_CT, st));
-        c->launches++;
-        d_p = c->d_scratch + SC_PART_CT;
-    }
-    AG_CUDA(c, ag_launch_peer_post(c->d_peer_bufs, (uint32_t)c->peer_rank, (uint32_t)c->peer_world, epoch, d_p, st));
-    c->launches++;
+    rc = peer_post(c, n_chunks, epoch, st);
+    if (rc) return rc;
     rc = peer_finish(c, 1, j0, c->aad_stage.p, aad_len, total_len, d_tag, d_ok, st, epoch, false);
     if (rc) return rc;
     rc = host_end(c, 1, nullptr, h_ok, st);
@@ -1982,14 +1986,12 @@ int agcm_stream_crypt_iv_host(agcm_ctx* c, int decrypt, const uint8_t* h_iv, siz
                               int* h_ok)
 {
     if (!c || !h_iv) return AGCM_E_BAD_ARG;
-    if (iv_len == 12) return agcm_stream_crypt_host(c, decrypt, h_iv, h_aad, aad_len, h_in, h_out, n_bytes, h_tag, h_ok);
-    int rc = host_begin(c, 0);
+    int rc = iv_len == 12 ? AGCM_OK : host_begin(c, 0);   // derive_j0 runs on the pipeline's first stream
     if (rc) return rc;
     uint8_t j0[16];
     rc = resolve_j0(c, h_iv, iv_len, j0, c->hs[0]);
     if (rc) return rc;
-    J0Scope scope(c, j0);
-    return agcm_stream_crypt_host(c, decrypt, j0, h_aad, aad_len, h_in, h_out, n_bytes, h_tag, h_ok);
+    return stream_crypt_host(c, decrypt, j0, h_aad, aad_len, h_in, h_out, n_bytes, h_tag, h_ok);
 }
 
 int agcm_batch_crypt_uniform_host(agcm_ctx* c, int decrypt, int lanes, const uint8_t* h_iv12, const uint8_t* h_aad,
@@ -2017,12 +2019,6 @@ int agcm_batch_crypt_uniform_host(agcm_ctx* c, int decrypt, int lanes, const uin
     // partials in one scratch buffer per context: whole-message layouts only on this path
     if (g > 4096) g = 32;     // (the warp-unit layout as well)
     if (g > 1024) g = 1024;
-    // (and no ticket-driven distribution: the context has ONE ticket word)
-    struct NoTicket {
-        agcm_ctx* c;
-        explicit NoTicket(agcm_ctx* ctx) : c(ctx) { c->no_ticket = true; }
-        ~NoTicket() { c->no_ticket = false; }
-    } no_ticket_scope(c);
     uint64_t k = 0;
     for (uint64_t m0 = 0; m0 < n_msgs; m0 += m_chunk, ++k) {
         const int s = (int)(k % kSlots);
@@ -2040,8 +2036,9 @@ int agcm_batch_crypt_uniform_host(agcm_ctx* c, int decrypt, int lanes, const uin
         if (aad_len)
             AG_CUDA(c, cudaMemcpyAsync(d_aad, h_aad + m0 * aad_stride, (nm - 1) * aad_stride + aad_len, cudaMemcpyHostToDevice, st));
         if (decrypt) AG_CUDA(c, cudaMemcpyAsync(d_tag, h_tag + 16 * m0, 16 * nm, cudaMemcpyHostToDevice, st));
-        rc = agcm_batch_crypt_uniform(c, decrypt, g, d_iv, d_aad, aad_len, aad_stride, d_data, d_data, len, stride, d_tag,
-                                      d_ok, nm, st);
+        // no ticket-driven distribution: the context has ONE ticket word
+        rc = batch_uniform(c, decrypt, g, d_iv, 0, d_aad, aad_len, aad_stride, d_data, d_data, len, stride, d_tag, d_ok, nm, st,
+                           false);
         if (rc) return rc;
         if (len) {
             if (stride == len) {
