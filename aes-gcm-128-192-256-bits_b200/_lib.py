@@ -14,6 +14,7 @@ CSRC = os.path.join(_HERE, "csrc")
 
 OK = 0
 E_BAD_MODE, E_BAD_LEN, E_COUNTER_OVERFLOW, E_CUDA, E_NO_KEY, E_BAD_ARG, E_NO_DEVICE, E_PEER_TIMEOUT = -1, -2, -3, -4, -5, -6, -7, -8
+PEER_HANDLE_BYTES = 128   # AGCM_PEER_HANDLE_BYTES
 
 c_u8p = ctypes.c_void_p  # raw addresses (host or device) are passed as integers
 c_u64 = ctypes.c_uint64
@@ -42,6 +43,9 @@ SIGNATURES = {
     "agcm_stream_crypt_iv": (c_int, [c_vp, c_int, c_u8p, c_sz, c_u8p, c_u64, c_u8p, c_u8p, c_u64, c_u8p, c_u8p, c_vp]),
     "agcm_stream_part": (c_int, [c_vp, c_int, c_u8p, c_u64, c_u8p, c_u8p, c_u64, c_u64, c_u8p, c_vp]),
     "agcm_stream_finish": (c_int, [c_vp, c_int, c_u8p, c_u8p, c_int, c_u8p, c_u64, c_u64, c_u8p, c_u8p, c_vp]),
+    "agcm_peer_export": (c_int, [c_vp, c_u8p]),
+    "agcm_peer_import": (c_int, [c_vp, c_int, c_int, c_u8p]),
+    "agcm_peer_close": (c_int, [c_vp]),
     "agcm_peer_setup": (c_int, [c_vp, c_int, c_int, ctypes.POINTER(c_u64)]),
     "agcm_peer_status": (c_int, [c_vp, ctypes.POINTER(c_int)]),
     "agcm_stream_crypt_peer": (c_int, [c_vp, c_int, c_u8p, c_u64, c_u8p, c_u8p, c_u64, c_u64, c_u8p, c_u64, c_u64, c_u8p,

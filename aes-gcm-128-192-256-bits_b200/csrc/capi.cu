@@ -8,6 +8,7 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <unistd.h>
 #include <new>
 #include <vector>
 
@@ -53,6 +54,21 @@ struct PowCache {
     cudaStream_t st = nullptr;   // the producer's stream
 };
 
+// What agcm_peer_export writes into the AGCM_PEER_HANDLE_BYTES of a handle (the rest is zero).  The address and the pid
+// let a context of the exporting process itself use the buffer directly: CUDA refuses to open a handle there.
+struct PeerHandle {
+    uint32_t magic;            // kPeerMagic
+    uint32_t version;          // kPeerVersion
+    int32_t pid;               // exporting process
+    uint32_t reserved;
+    uint64_t addr;             // the buffer's device address in the exporting process
+    uint64_t size;             // bytes
+    cudaIpcMemHandle_t ipc;    // cudaIpcGetMemHandle of the buffer
+};
+static_assert(sizeof(PeerHandle) <= AGCM_PEER_HANDLE_BYTES, "the handle does not fit AGCM_PEER_HANDLE_BYTES");
+constexpr uint32_t kPeerMagic = 0x4d434741u;   // "AGCM" in memory order
+constexpr uint32_t kPeerVersion = 1;
+
 }  // namespace
 
 struct agcm_ctx {
@@ -76,6 +92,9 @@ struct agcm_ctx {
     cudaStream_t peer_side = nullptr;    // the finishes wait for the world's flags here, off the caller's stream
     cudaEvent_t peer_bulk_ev[AG_PEER_RING] = {};
     cudaEvent_t peer_fin_ev[AG_PEER_RING] = {};
+    uint8_t* peer_own = nullptr;         // this context's exchange buffer once agcm_peer_export made it
+    uint8_t peer_handle[AGCM_PEER_HANDLE_BYTES] = {};   // ... and its handle
+    void* peer_opened[AG_PEER_MAX] = {}; // other processes' buffers the last agcm_peer_import mapped
     uint32_t h_rk[60];
     uint8_t h_H[16];
     uint8_t h_key_in[240];           // the key as it was loaded, to recognise a reload of the same key
@@ -606,6 +625,9 @@ void agcm_ctx_destroy(agcm_ctx* c)
     cudaFree(c->d_counters);
     cudaFree(c->pow_n.d);
     cudaFree(c->pow_scale.d);
+    for (void* p : c->peer_opened)
+        if (p) cudaIpcCloseMemHandle(p);
+    cudaFree(c->peer_own);
     cudaFree(c->d_peer_bufs);
     cudaFree(c->d_peer_status);
     if (c->h_peer_status) cudaFreeHost(c->h_peer_status);
@@ -830,11 +852,26 @@ int agcm_stream_crypt_iv(agcm_ctx* c, int decrypt, const uint8_t* h_iv, size_t i
     return stream_crypt(c, decrypt, j0, d_aad, aad_len, d_in, d_out, n_bytes, d_tag, d_ok, stream);
 }
 
-int agcm_peer_setup(agcm_ctx* c, int rank, int world, const uint64_t* h_peer_ptrs)
+// Leaves the world: waits for the device (no finish of an earlier session may still be waiting, no kernel may still use a
+// mapping) and closes what the last agcm_peer_import mapped.  Peer calls return AGCM_E_BAD_ARG until the next set-up.
+static int peer_leave(agcm_ctx* c)
 {
-    if (!c || !h_peer_ptrs || world < 1 || world > (int)AG_PEER_MAX || rank < 0 || rank >= world) return AGCM_E_BAD_ARG;
     AG_CUDA(c, cudaSetDevice(c->device));
-    AG_CUDA(c, cudaDeviceSynchronize());   // no finish of an earlier session may still be waiting
+    AG_CUDA(c, cudaDeviceSynchronize());
+    c->peer_world = 0;
+    for (void*& p : c->peer_opened) {
+        if (!p) continue;
+        const cudaError_t e = cudaIpcCloseMemHandle(p);
+        p = nullptr;
+        AG_CUDA(c, e);
+    }
+    return AGCM_OK;
+}
+
+// Joins a world whose exchange buffers are mapped at h_peer_ptrs (the caller left the previous one): zeroes this rank's
+// buffer, resets epoch and status, preloads the peer kernels.
+static int peer_attach(agcm_ctx* c, int rank, int world, const uint64_t* h_peer_ptrs)
+{
     if (!c->d_peer_bufs) AG_CUDA(c, cudaMalloc(&c->d_peer_bufs, sizeof(uint8_t*) * AG_PEER_MAX));
     if (!c->d_peer_status) AG_CUDA(c, cudaMalloc(&c->d_peer_status, sizeof(uint32_t)));
     if (!c->h_peer_status) AG_CUDA(c, cudaHostAlloc(reinterpret_cast<void**>(&c->h_peer_status), sizeof(uint32_t), cudaHostAllocMapped));
@@ -860,6 +897,89 @@ int agcm_peer_setup(agcm_ctx* c, int rank, int world, const uint64_t* h_peer_ptr
     c->peer_world = world;
     c->peer_epoch = 0;
     return AGCM_OK;
+}
+
+static bool peer_world_ok(int rank, int world) { return world >= 1 && world <= (int)AG_PEER_MAX && rank >= 0 && rank < world; }
+
+int agcm_peer_setup(agcm_ctx* c, int rank, int world, const uint64_t* h_peer_ptrs)
+{
+    if (!c || !h_peer_ptrs || !peer_world_ok(rank, world)) return AGCM_E_BAD_ARG;
+    int rc = peer_leave(c);
+    if (rc) return rc;
+    return peer_attach(c, rank, world, h_peer_ptrs);
+}
+
+int agcm_peer_export(agcm_ctx* c, uint8_t h_handle[AGCM_PEER_HANDLE_BYTES])
+{
+    if (!c || !h_handle) return AGCM_E_BAD_ARG;
+    if (!c->peer_own) {
+        AG_CUDA(c, cudaSetDevice(c->device));
+        uint8_t* p = nullptr;
+        AG_CUDA(c, cudaMalloc(&p, AG_PEER_BYTES));   // a dedicated allocation: the exported base is the buffer itself
+        PeerHandle h;
+        memset(&h, 0, sizeof(h));
+        h.magic = kPeerMagic;
+        h.version = kPeerVersion;
+        h.pid = (int32_t)getpid();
+        h.addr = (uint64_t)(uintptr_t)p;
+        h.size = AG_PEER_BYTES;
+        const cudaError_t e = cudaIpcGetMemHandle(&h.ipc, p);
+        if (e != cudaSuccess) {
+            cudaFree(p);
+            return cuda_fail(c, e);
+        }
+        memcpy(c->peer_handle, &h, sizeof(h));
+        c->peer_own = p;
+    }
+    memcpy(h_handle, c->peer_handle, AGCM_PEER_HANDLE_BYTES);
+    return AGCM_OK;
+}
+
+int agcm_peer_import(agcm_ctx* c, int rank, int world, const uint8_t* h_handles)
+{
+    if (!c || !h_handles || !peer_world_ok(rank, world)) return AGCM_E_BAD_ARG;
+    // entry `rank` must be this context's own export
+    if (!c->peer_own || memcmp(h_handles + (size_t)rank * AGCM_PEER_HANDLE_BYTES, c->peer_handle, AGCM_PEER_HANDLE_BYTES))
+        return AGCM_E_BAD_ARG;
+    PeerHandle h[AG_PEER_MAX];
+    for (int w = 0; w < world; ++w) {
+        memcpy(&h[w], h_handles + (size_t)w * AGCM_PEER_HANDLE_BYTES, sizeof(PeerHandle));
+        if (h[w].magic != kPeerMagic || h[w].version != kPeerVersion || h[w].pid <= 0 || !h[w].addr ||
+            h[w].size < AG_PEER_BYTES)
+            return AGCM_E_BAD_ARG;
+        for (int v = 0; v < w; ++v)
+            if (h[v].pid == h[w].pid && h[v].addr == h[w].addr) return AGCM_E_BAD_ARG;   // two ranks, one buffer
+    }
+    int rc = peer_leave(c);
+    if (rc) return rc;
+    const int32_t me = (int32_t)getpid();
+    uint64_t ptrs[AG_PEER_MAX];
+    for (int w = 0; w < world; ++w) {
+        if (h[w].pid != me) {   // peer access to the exporter's device is enabled by the open
+            void* p = nullptr;
+            AG_CUDA(c, cudaIpcOpenMemHandle(&p, h[w].ipc, cudaIpcMemLazyEnablePeerAccess));
+            c->peer_opened[w] = p;
+            ptrs[w] = (uint64_t)(uintptr_t)p;
+            continue;
+        }
+        // a buffer of this process (CUDA refuses to open a handle where it was exported): its address is valid here
+        cudaPointerAttributes a;
+        AG_CUDA(c, cudaPointerGetAttributes(&a, reinterpret_cast<const void*>(h[w].addr)));
+        if (a.type != cudaMemoryTypeDevice) return AGCM_E_BAD_ARG;
+        if (a.device != c->device) {
+            const cudaError_t e = cudaDeviceEnablePeerAccess(a.device, 0);
+            if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();   // not an error: clear it
+            else AG_CUDA(c, e);
+        }
+        ptrs[w] = h[w].addr;
+    }
+    return peer_attach(c, rank, world, ptrs);
+}
+
+int agcm_peer_close(agcm_ctx* c)
+{
+    if (!c) return AGCM_E_BAD_ARG;
+    return peer_leave(c);
 }
 
 int agcm_peer_status(agcm_ctx* c, int* h_timed_out)

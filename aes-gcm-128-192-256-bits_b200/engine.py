@@ -324,6 +324,25 @@ class GcmEngine:
         arr = (ctypes.c_uint64 * world)(*[int(p) for p in peer_ptrs])
         self._ck(self._L.agcm_peer_setup(self._ctx, int(rank), int(world), arr))
 
+    def peer_export(self):
+        """-> the handle (bytes) of this context's exchange buffer, allocated on the first call; every rank hands its
+        handle to every other rank (any transport) for peer_import."""
+        out = np.zeros(_lib.PEER_HANDLE_BYTES, dtype=np.uint8)
+        self._ck(self._L.agcm_peer_export(self._ctx, _addr(out)))
+        return out.tobytes()
+
+    def peer_import(self, rank, world, handles):
+        """handles: the world's peer_export() results in rank order (entry `rank` is this engine's own).  Maps the
+        other ranks' buffers and sets up the exchange; barrier the ranks before the first peer call."""
+        if len(handles) != int(world) or any(len(h) != _lib.PEER_HANDLE_BYTES for h in handles):
+            raise _lib.AgcmError(_lib.E_BAD_ARG, "expected %d handles of %d bytes" % (int(world), _lib.PEER_HANDLE_BYTES))
+        arr = np.frombuffer(b"".join(bytes(h) for h in handles), dtype=np.uint8)
+        self._ck(self._L.agcm_peer_import(self._ctx, int(rank), int(world), _addr(arr)))
+
+    def peer_close(self):
+        """Unmap the other ranks' buffers and leave the world (every rank, then a barrier, then close())."""
+        self._ck(self._L.agcm_peer_close(self._ctx))
+
     def peer_timed_out(self):
         v = ctypes.c_int()
         self._ck(self._L.agcm_peer_status(self._ctx, ctypes.byref(v)))

@@ -79,27 +79,32 @@ def stream_crypt_sharded(engine, decrypt, iv, aad, shard, data_in, data_out, tot
 class PeerExchange:
     """Peer-memory (NVLink) exchange buffers for `GcmEngine.stream_crypt_peer_device`.
 
-    Allocates one small symmetric-memory buffer per rank (torch.distributed._symmetric_memory:
-    CUDA VMM allocations mapped into every process of the node), hands the peer addresses to the
-    engine, and barriers once.  After that a sharded message costs one bulk kernel per rank plus a
-    one-warp finish on the engine's side stream, and no collective call: the 16-byte partials cross
-    NVLink as plain stores from the bulk kernel's tail (src/gcm_ghash.vhd:317-344 linearity).
+    Each rank's engine exports its own small exchange buffer as a CUDA IPC handle (`peer_export`); the
+    handles go round the group once (`all_gather_object`), every engine maps the others' buffers
+    (`peer_import`), and the ranks barrier once.  After that a sharded message costs one bulk kernel per
+    rank plus a one-warp finish on the engine's side stream, and no collective call: the 16-byte partials
+    cross NVLink as plain stores from the bulk kernel's tail (src/gcm_ghash.vhd:317-344 linearity).
+    `close()` unmaps the peers' buffers on every rank before any engine is closed.
     """
 
     def __init__(self, engine, group=None):
         import torch
         import torch.distributed as dist
-        import torch.distributed._symmetric_memory as symm_mem
         self.group = group if group is not None else dist.group.WORLD
         self.rank, self.world = dist.get_rank(self.group), dist.get_world_size(self.group)
-        dev = torch.device("cuda", engine.device)
-        self.buf = symm_mem.empty(4096, dtype=torch.uint8, device=dev)
-        self.handle = symm_mem.rendezvous(self.buf, self.group)
-        ptrs = list(self.handle.buffer_ptrs)
-        engine.peer_setup(self.rank, self.world, ptrs)
+        handles = [None] * self.world
+        dist.all_gather_object(handles, engine.peer_export(), group=self.group)
+        engine.peer_import(self.rank, self.world, handles)
         dist.barrier(self.group)   # every buffer is zeroed before anyone stores into it
-        torch.cuda.synchronize(dev)
+        torch.cuda.synchronize(torch.device("cuda", engine.device))
         self.engine = engine
+
+    def close(self):
+        """Leave the exchange: unmap the peers' buffers, then barrier, so that no rank frees its buffer (by closing its
+        engine) while another still maps it."""
+        import torch.distributed as dist
+        self.engine.peer_close()
+        dist.barrier(self.group)
 
     def crypt(self, decrypt, iv, aad, shard, data_in, data_out, total_bytes, tag, ok=None, stream=None, defer=False):
         """This rank's shard of one message.  defer=True keeps the ranks free-running (the finish of

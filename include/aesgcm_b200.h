@@ -33,7 +33,7 @@
  *     message holds fewer than 2^32 blocks of AAD + payload + 1 (checked for the uniform forms; for the
  *     offset forms the offsets live in device memory and the limit is the caller's to keep: UNCHECKED);
  *     agcm_stream_finish takes up to
- *     1024 shard partials; agcm_peer_setup up to 16 ranks; the host-buffer stream call up to
+ *     1024 shard partials; agcm_peer_setup / agcm_peer_import up to 16 ranks; the host-buffer stream call up to
  *     1024 x 64 MiB per call.  AAD of any length (bytes 4097.. run through the grid-wide GHASH).
  *   - Device buffers may have any byte alignment; 16-byte alignment selects the 128-bit
  *     load/store path (4-byte alignment a 32-bit path, anything else bytes; batched messages that a single
@@ -215,9 +215,31 @@ int agcm_stream_crypt_peer_j0(agcm_ctx* ctx, int decrypt, const uint8_t h_j0[16]
                               uint64_t total_len, uint8_t* d_tag, uint8_t* d_ok, void* stream, int deferred);
 
 /* ---- sharded message, partials exchanged over peer memory (NVLink) ---------------------------
- * agcm_peer_setup: h_peer_ptrs[w] = device address, valid in THIS process, of rank w's exchange
- * buffer (>= 2560 bytes, e.g. torch symmetric memory); zeroes this rank's buffer -- barrier before
- * the first exchange.  world <= 16.  AGCM_PEER_TIMEOUT_MS (environment, default 10000) bounds the wait.
+ * Every rank needs every rank's exchange buffer mapped in its own process.  Two ways to set that up:
+ *   - agcm_peer_export / agcm_peer_import (any client, one process per GPU or several contexts in one process):
+ *     the library owns the buffers and moves them between processes as CUDA IPC handles.
+ *       agcm_peer_export: on the first call allocates this context's exchange buffer (cudaMalloc, 2560 bytes, on the
+ *         context's device) and writes an opaque AGCM_PEER_HANDLE_BYTES handle to it; later calls write the same
+ *         handle.  The caller moves the handles between the ranks by any means (a file, a socket, MPI).  The buffer
+ *         lives until agcm_ctx_destroy.
+ *       agcm_peer_import: h_handles = world handles, rank w's at h_handles + w * AGCM_PEER_HANDLE_BYTES; entry `rank`
+ *         must be this context's own export.  Maps every other rank's buffer (cudaIpcOpenMemHandle; a buffer of this
+ *         same process is used at its own address, with peer access enabled when it lives on another device), then
+ *         sets up as agcm_peer_setup does.  AGCM_E_BAD_ARG for a handle that is not one (wrong magic or version), a
+ *         buffer under 2560 bytes, two entries naming the same buffer, an entry `rank` that is not this context's
+ *         export, and the argument checks of agcm_peer_setup.  Barrier after the import, before the first exchange.
+ *         A process may import a given device's handles into one CUDA context per device (the CUDA rule); the
+ *         library uses the device's primary context, so several contexts on one device may import the same handles.
+ *       agcm_peer_close: unmaps what the last import mapped and leaves the world: peer calls return AGCM_E_BAD_ARG
+ *         until the next set-up.  Teardown: every rank calls agcm_peer_close, the ranks barrier, then each rank
+ *         calls agcm_ctx_destroy (an exported buffer must not be freed while another process still maps it).
+ *         agcm_ctx_destroy also closes any mappings still open.
+ *     A second import, or an agcm_peer_setup after an import, first closes the previous import's mappings.
+ *   - agcm_peer_setup (callers that map the buffers themselves): h_peer_ptrs[w] = device address, valid in THIS
+ *     process, of rank w's exchange buffer (>= 2560 bytes); the caller keeps the buffers mapped while the world is in
+ *     use.
+ * Both zero this rank's buffer -- barrier before the first exchange.  world <= 16.  AGCM_PEER_TIMEOUT_MS
+ * (environment, default 10000) bounds the wait.
  * agcm_stream_crypt_peer: agcm_stream_part + the 16-byte all-to-all + agcm_stream_finish without a
  * collective library call.  The last CTA of the bulk kernel stores the scaled partial into every
  * peer's buffer (plain stores over NVLink) and raises an epoch flag; it does NOT wait.  A one-warp
@@ -232,8 +254,12 @@ int agcm_stream_crypt_peer_j0(agcm_ctx* ctx, int decrypt, const uint8_t h_j0[16]
  * All ranks must make the same sequence of peer calls; n_bytes == 0 is allowed (a rank whose
  * counter range is empty still posts); aad_len <= 4096 (else use part + gather + finish).
  * FAILS CLOSED: if a rank never posts, the finish zeroes the tag, clears ok, and every later peer
- * call on the context returns AGCM_E_PEER_TIMEOUT until agcm_peer_setup is called again;
+ * call on the context returns AGCM_E_PEER_TIMEOUT until the exchange is set up again;
  * agcm_peer_status (synchronises the side stream) reports it too. */
+#define AGCM_PEER_HANDLE_BYTES 128
+int agcm_peer_export(agcm_ctx* ctx, uint8_t h_handle[AGCM_PEER_HANDLE_BYTES]);
+int agcm_peer_import(agcm_ctx* ctx, int rank, int world, const uint8_t* h_handles);
+int agcm_peer_close(agcm_ctx* ctx);
 int agcm_peer_setup(agcm_ctx* ctx, int rank, int world, const uint64_t* h_peer_ptrs);
 int agcm_peer_status(agcm_ctx* ctx, int* h_timed_out);
 int agcm_peer_join(agcm_ctx* ctx, void* stream);
@@ -254,7 +280,7 @@ int agcm_stream_crypt_peer_async(agcm_ctx* ctx, int decrypt, const uint8_t h_iv1
  *     flipped bit in any rank's ciphertext, in the AAD or in the tag makes every rank release nothing;
  *   - d_ct == d_pt (exactly aliased) is allowed: a failed shard then still holds its ciphertext;
  *   - FAILS CLOSED as the releasing calls: if a rank never posts, *d_ok = 0, nothing is released, and every later peer
- *     call returns AGCM_E_PEER_TIMEOUT until agcm_peer_setup runs again.
+ *     call returns AGCM_E_PEER_TIMEOUT until the exchange is set up again.
  * d_ok and d_pt are valid in stream order on `stream`.  There is no deferred form: release needs the world's tag, so every
  * message is a rank-wide wait.  Argument checks, error codes and limits are those of agcm_stream_crypt_peer (aad_len <= 4096,
  * the same first_block / blocks_after / total_len consistency, an empty counter range still posts, total_len == 0 = GMAC
